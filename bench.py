@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] ...     # CPU reference arm (oracle port)
+    python bench.py ... --dump-outputs DIR                          # also save a sample of the last step's scores
 
 Workloads (`--workload`, named in `config.workload`): default "plaid" = BASELINE.json configs[3] — plaid() on a 1M-cell x 20k-gene
 sparse single-cell matrix with 30k gene sets, sample-sharded over 8 B200 — run as its per-GPU
@@ -16,6 +17,10 @@ normalisation) over the rank's shard.
   roofline   dominant kernel (k_score): algorithmic bytes of SURVEY.md §8(d) per launch / CUDA-event
              duration of that launch (events on the library's own stream), vs MEASURED_PEAKS.json;
   cpu_baseline  the oracle (numpy/scipy restatement of the R path) on 1 host core, bounded sample.
+
+Every timed leg (value, e2e and its pinned / pageable / fused-test legs) times exactly --steps steps.
+--dump-outputs saves rank 0's shard only (ranks hold disjoint cells) and applies to --impl ours: the reference arm
+keeps no scores.
 
 Other workloads (same JSON line, same keys): "ssgsea" / "ucell" = replaid.ssgsea(alpha=0) / replaid.ucell on the
 same sparse shard (BASELINE.json configs[2] / configs[4], the north star's second target), "sing" / "aucell" = the
@@ -39,6 +44,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 P_GENES, S_SETS, CELLS_PER_GPU = 20000, 30000, 125000
+DUMP_CELLS = 256  # 256 cells x 30,000 sets in fp64 = 61 MB: a dump stays under 64 MB
 METRIC = "plaid() cells x genesets scored/sec"
 UNIT = "cells*genesets/s"
 
@@ -54,7 +60,15 @@ def parse():
     ap.add_argument("--e2e-cells", type=int, default=-1,
                     help="cells per GPU of the host-buffer e2e legs (-1 = the full shard when host memory allows, 0 = skip)")
     ap.add_argument("--cpu-cells", type=int, default=3000, help="cells of the 1-core CPU baseline sample (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help=f"after the timed steps, write the scores of the last one as DIR/scores.npy: float64, all sets x "
+                         f"{DUMP_CELLS} cells of rank 0's shard, the same cells every run (fixed seed, ascending)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
 
 
 def peaks():
@@ -195,6 +209,14 @@ def bind_to_gpu_node(torch, local):
         return f"unbound ({type(ex).__name__})"
 
 
+def dump_scores(torch, path, out, n_cells):
+    """Write DIR/scores.npy: the S x n_cells result (column-major on the device) at a fixed, seeded sample of cells."""
+    cols = np.sort(np.random.default_rng(0).choice(n_cells, min(DUMP_CELLS, n_cells), replace=False))
+    sample = out.view(n_cells, S_SETS).index_select(0, torch.from_numpy(cols).to(out.device))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "scores.npy"), np.ascontiguousarray(sample.T.cpu().numpy()))
+
+
 # ---------------------------------------------------------------------------------------------
 def run_ours(a):
     import torch
@@ -287,6 +309,8 @@ def run_ours(a):
         barrier()
         dt = time.perf_counter() - t0
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        dump_scores(torch, a.dump_outputs, out, Nc)
     launches = ctx.launch_count()
     tt = torch.tensor([dt, float(launches), k_ms[0], float(nnz), k_ms[3]], dtype=torch.float64, device=dev)
     if dist is not None:
@@ -368,7 +392,7 @@ def run_ours(a):
                 return sharded.score_shard(ctx, comm, Mh, rowmap, oh, out_ptr, Ne)
             estep(); estep()  # the second call sizes its early-shipped part from the first one's measured rates
             barrier()
-            ke = max(1, min(a.steps, 3 if Ne * per_cell > (8 << 30) else 5))
+            ke = a.steps
             t0 = time.perf_counter()
             for _ in range(ke):
                 estep()
@@ -403,7 +427,7 @@ def run_ours(a):
                                                                mo.ctypes.data))
                 fstep()
                 torch.cuda.synchronize()
-                kf = max(1, min(a.steps, 5))
+                kf = a.steps
                 t0 = time.perf_counter()
                 for _ in range(kf):
                     fstep()

@@ -289,8 +289,8 @@ def _w_dgc(out, m, rownames, colnames, symtab):
 
 
 def write_rda(path: str, objects: dict, version: int = 3, compress: bool = True, rds: bool = False):
-    """objects: {name: (scipy csc_matrix, rownames | None, colnames | None)}.  `rds=True` writes the first
-    object the way saveRDS() does (no RDX header, no name)."""
+    """objects: {name: (scipy csc_matrix, rownames | None, colnames | None) or a list of str (a character
+    vector)}.  `rds=True` writes the first object, a matrix, the way saveRDS() does (no RDX header, no name)."""
     out: list = []
     if not rds:
         out.append(b"RDX3\n" if version == 3 else b"RDX2\n")
@@ -308,11 +308,15 @@ def write_rda(path: str, objects: dict, version: int = 3, compress: bool = True,
         m.sort_indices()
         _w_dgc(out, m, rn, cn, symtab)
     else:
-        for name, (m, rn, cn) in objects.items():
-            m = m.tocsc()
-            m.sort_indices()
+        for name, obj in objects.items():
             _w_int(out, 2 | 0x400)
             _w_sym(out, name, symtab)
+            if isinstance(obj, list):
+                _w_strsxp(out, obj)
+                continue
+            m, rn, cn = obj
+            m = m.tocsc()
+            m.sort_indices()
             _w_dgc(out, m, rn, cn, symtab)
         _w_int(out, _NILVALUE)
     raw = b"".join(out)

@@ -1,6 +1,6 @@
 """Expression-matrix ingestion (scope row f4): the product's C++ readers (plaid_b200/csrc/matio.cu, host
 code, no GPU needed) against independent decoders — the oracle's RDX reader, scipy.io.mmread — on generated
-files and, where the reference tree is present, on the reference's own fixture."""
+files, among them one holding the contents of the reference's bundled fixture (tests/golden)."""
 import gzip
 import os
 
@@ -12,8 +12,6 @@ import scipy.sparse as sp
 import plaid_b200 as pb
 from plaid_b200 import _lib as L
 from oracle import rdata
-
-REF_FIXTURE = "/root/reference/inst/extdata/pbmc3k-50cells.rda"
 
 
 def _rand_csc(P, N, density, seed, integer=False):
@@ -34,15 +32,20 @@ def _same(a: pb.NamedMatrix, m, rn, cn):
     assert a.colnames == (list(cn) if cn is not None else None)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_FIXTURE), reason="reference tree not present")
-def test_reference_fixture_matches_oracle_reader():
-    m, rn, cn = rdata.dgc_to_scipy(rdata.read_rda(REF_FIXTURE)["X"])
-    X = pb.read_rda(REF_FIXTURE)
-    _same(X, m, rn, cn)
-    _same(pb.read_rda(REF_FIXTURE, "X"), m, rn, cn)
-    assert X.mat.shape == (7728, 50)
+def test_pbmc3k_fixture_contents_round_trip(tmp_path, fixture_mats, golden):
+    """The contents of the reference's inst/extdata/pbmc3k-50cells.rda (dgCMatrix X, 7728 x 50, with its gene and
+    barcode names, plus the character vector celltype), as decoded into tests/golden/pbmc3k50_hallmarks.npz, written
+    by oracle.rdata.write_rda.  The R-written file itself is not part of the repository: this pins the reader on the
+    reference's values and names, not on the exact bytes R's save() emits."""
+    m, rn, cn = fixture_mats[:3]
+    celltype = [str(s) for s in golden["celltype"]]
+    path = str(tmp_path / "pbmc3k-50cells.rda")
+    rdata.write_rda(path, {"X": (m, rn, cn), "celltype": celltype})
+    assert rdata.read_rda(path)["celltype"] == celltype  # the writer's character vector, by the independent reader
+    _same(pb.read_rda(path), m, rn, cn)
+    _same(pb.read_rda(path, "X"), m, rn, cn)
     with pytest.raises(L.PlaidGpuError, match="celltype"):
-        pb.read_rda(REF_FIXTURE, "celltype")  # a character vector, not a dgCMatrix
+        pb.read_rda(path, "celltype")  # a character vector, not a dgCMatrix
 
 
 @pytest.mark.parametrize("version,compress,rds", [(3, True, False), (2, False, False), (3, True, True)])
