@@ -275,6 +275,30 @@ int plaidgpu_group_moments(plaidgpu_ctx* ctx, const double* x, int32_t S, int64_
 int plaidgpu_score_group_moments(plaidgpu_ctx* ctx, const plaidgpu_matrix* X, const int32_t* rowmap,
                                  const plaidgpu_opts* opts, const int32_t* y, double* out);
 
+/* Per gene set the sums and sums of squares over the samples of each of K groups: the reductions behind
+ * plaid.test(tests = "lm") when every cluster is compared with the rest (one pass over the scores, whatever K is).
+ * x: S x N column-major doubles at `location`; labels: host int32[N], labels[j] in [0, K) is the group of sample j and
+ * -1 leaves it out; out: host double[K * 2 * S] = {sum_k[S], sumsq_k[S]} for k = 0 .. K-1 (an empty group gives
+ * zeros).  Columns are added in a fixed order, so results are bit-reproducible; with K = 2 and labels y != 0 they
+ * equal plaidgpu_group_moments bit for bit.  K < 1 or a label outside [-1, K) is PLAIDGPU_ERR_ARG. */
+int plaidgpu_group_stats(plaidgpu_ctx* ctx, const double* x, int32_t S, int64_t N, const int32_t* labels, int K,
+                         int location, double* out);
+
+/* The same reductions fused onto the scoring call, for any scorer and option plaidgpu_score accepts: the scores stay
+ * on the device as raw scores and are normalised in registers while reducing; K * 2 * S doubles come back (layout as
+ * above).  Equal, bit for bit, to plaidgpu_score followed by plaidgpu_group_stats.  When X is in host memory and the
+ * S x N scores exceed the device, the columns are scored in tiles (a normalised call makes two passes over X like
+ * plaidgpu_score: medians first, then scores reduced tile by tile) and the tiles' moments are added in tile order.
+ * plaidgpu_score_group_moments is this call with K = 2. */
+int plaidgpu_score_group_stats(plaidgpu_ctx* ctx, const plaidgpu_matrix* X, const int32_t* rowmap,
+                               const plaidgpu_opts* opts, const int32_t* labels, int K, double* out);
+
+/* plaidgpu_score_group_stats over n devices from ONE host process, split like plaidgpu_score_multi (X in host memory,
+ * one host thread per context, scalars and medians combined on the host in column order); every shard reduces its
+ * own scores and the shards' moments are added in shard order.  Each shard's scores must fit its device. */
+int plaidgpu_score_group_stats_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
+                                     const plaidgpu_opts* opts, const int32_t* labels, int K, double* out);
+
 /* ---- gene-set ingestion ("next" row f2): host-side, no GPU needed -------------------------- */
 
 /* read.gmt() + gmt2mat() with default arguments (reference R/gmt-utils.R:99-125, 19-66): a GMT text

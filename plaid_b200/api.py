@@ -122,6 +122,7 @@ class Context:
                                                   gi.ctypes.data, gx.ctypes.data))
         self._gkey = key
         self._glast = G0  # only after the C call succeeded: a failed registration is retried
+        self.n_sets = int(G.shape[1])
 
     def launch_count(self) -> int:
         return int(self.lib.plaidgpu_launch_count(self.h))
@@ -482,17 +483,69 @@ def score_group_moments(X: NamedMatrix, matG: NamedMatrix, y, *, ctx=None, **opt
     return out
 
 
-def plaid_test(X: NamedMatrix, y, G: NamedMatrix, gsetX: Optional[NamedMatrix] = None, tests=("one", "two", "lm"),
-               metap_method: str = "fisher", sort_by: str = "p.meta", *, ctx=None):
-    """`plaid.test(X, y, G, gsetX, tests=c("one","two","lm"), metap.method="fisher", sort.by="p.meta")`
-    (R/plaid.R:392-474).  GPU: the score matrix (plaid), the crossprods of the one/two-sample tests
-    (chunked_crossprod on G != 0) and the per-set group moments of the "lm" test; host: pt / pchisq / p.adjust.
-    Returns (table, column names, row names) like the oracle."""
-    from scipy import stats
+def group_stats(gsetX, labels, K=None, *, ctx=None):
+    """Per row of a dense S x N matrix: (sum, sum of squares) over the columns of each group k = labels[j] in [0, K)
+    (`plaidgpu_group_stats`); a label of -1 leaves the column out.  K defaults to max(labels) + 1.  Returns an
+    array of shape (K, 2, S); empty groups give zeros."""
     ctx = ctx or default_context()
-    y = np.asarray(y)
-    if not np.all(np.isin(np.unique(y), [0, 1])):
-        raise ValueError("elements of y must be 0 or 1")  # R/plaid.R:394
+    if _is_torch(gsetX):
+        raise TypeError("pass device matrices through the C ABI directly")
+    a = np.asfortranarray(np.asarray(gsetX, dtype=np.float64))
+    lab, K = _labels(labels, a.shape[1], K)
+    out = np.empty((K, 2, a.shape[0]), dtype=np.float64)
+    ctx.check(ctx.lib.plaidgpu_group_stats(ctx.h, a.ctypes.data, a.shape[0], a.shape[1], lab.ctypes.data, K, L.HOST,
+                                           out.ctypes.data))
+    return out
+
+
+def _labels(labels, n, K):
+    lab = np.ascontiguousarray(np.asarray(labels), dtype=np.int32)
+    if lab.ndim != 1 or lab.size != n:
+        raise ValueError("length(labels) must equal ncol(X)")
+    if K is None:
+        K = int(lab.max()) + 1 if lab.size else 1
+    return lab, int(K)
+
+
+def score_group_stats(X: NamedMatrix, matG: NamedMatrix, labels, K=None, *, ctx=None, **opts_kw):
+    """plaid() (or another scorer through `opts_kw`) fused with the per-group reductions of group_stats
+    (`plaidgpu_score_group_stats`): the S x N scores stay on the device, K x 2 x S doubles come back.  `ctx` may be a
+    list of Contexts on different devices: the columns are then split over them
+    (`plaidgpu_score_group_stats_multi`).  Returns an array of shape (K, 2, S), or None on no overlap."""
+    ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else None
+    ctx = (ctxs[0] if ctxs else ctx) or default_context()
+    if X.rownames is None or matG.rownames is None:
+        _message("[plaid] ERROR. No overlapping features.")
+        return None
+    rowmap = make_rowmap(X.rownames, matG.rownames)
+    if not (rowmap >= 0).any():
+        _message("[plaid] ERROR. No overlapping features.")
+        return None
+    for cx in (ctxs or [ctx]):
+        cx.set_genesets(matG.mat)
+    keep: list = []
+    M = _matrix_struct(X.mat, keep)
+    lab, K = _labels(labels, M.N, K)
+    kw = dict(scorer=L.PLAID, stats_mean=1, normalize=1)
+    kw.update(opts_kw)
+    o = _opts(ctx.lib, **kw)
+    out = np.empty((K, 2, int(matG.mat.shape[1])), dtype=np.float64)
+    if ctxs and len(ctxs) > 1:
+        hs = (C.c_void_p * len(ctxs))(*[cx.h for cx in ctxs])
+        rc = ctx.lib.plaidgpu_score_group_stats_multi(hs, len(ctxs), C.byref(M), rowmap.ctypes.data, C.byref(o),
+                                                      lab.ctypes.data, K, out.ctypes.data)
+    else:
+        rc = ctx.lib.plaidgpu_score_group_stats(ctx.h, C.byref(M), rowmap.ctypes.data, C.byref(o), lab.ctypes.data, K,
+                                                out.ctypes.data)
+    if rc == L.ERR_NOOVERLAP:
+        _message("[plaid] ERROR. No overlapping features.")
+        return None
+    ctx.check(rc)
+    return out
+
+
+def _align(X: NamedMatrix, G: NamedMatrix):
+    """intersect(rownames(G), rownames(X)) and X[gg, ], G[gg, ] (R/plaid.R:402-404)"""
     xset = set(X.rownames)
     gg = [g for g in dict.fromkeys(G.rownames) if g in xset]
     xpos, gpos = {}, {}
@@ -504,19 +557,15 @@ def plaid_test(X: NamedMatrix, y, G: NamedMatrix, gsetX: Optional[NamedMatrix] =
     gi = np.array([gpos[g] for g in gg])
     Xs = sp.csc_matrix(X.mat).tocsr()[xi].tocsc() if sp.issparse(X.mat) else np.asarray(X.mat, dtype=np.float64)[xi]
     Gs = sp.csc_matrix(G.mat).tocsr()[gi].tocsc()
-    n1, n0 = int((y == 1).sum()), int((y == 0).sum())
-    if sp.issparse(Xs):
-        fc = np.asarray(Xs[:, y == 1].sum(axis=1)).ravel() / n1 - np.asarray(Xs[:, y == 0].sum(axis=1)).ravel() / n0
-    else:
-        fc = Xs[:, y == 1].mean(axis=1) - Xs[:, y == 0].mean(axis=1)
     Gb = Gs.copy()
     Gb.data = (Gb.data != 0).astype(np.float64)
     Gb.eliminate_zeros()
-    sumG = np.asarray(Gb.sum(axis=0)).ravel()
-    P, Fs = {}, {}
-    if "one" in tests or "two" in tests:
-        cp = chunked_crossprod(Gb, np.column_stack([fc, fc ** 2]), ctx=ctx)  # crossprod(G != 0, [F, F^2]) on the GPU
-        s1, q1 = cp[:, 0], cp[:, 1]
+    return gg, Xs, Gs, Gb
+
+
+def _set_tests(tests, s1, q1, sumG, ngenes, fc, P, Fs):
+    """the "one" and "two" tests of plaid.test from crossprod(G != 0, [fc, fc^2]) = [s1, q1] (R/plaid.R:476-520)"""
+    from scipy import stats
     with np.errstate(invalid="ignore", divide="ignore"):
         if "one" in tests:  # R/plaid.R:476-486
             meanx = s1 / (1e-8 + sumG)
@@ -524,7 +573,7 @@ def plaid_test(X: NamedMatrix, y, G: NamedMatrix, gsetX: Optional[NamedMatrix] =
             t = meanx / (1e-8 + sdx) * np.sqrt(sumG)
             P["one"], Fs["one"] = 2.0 * stats.t.sf(np.abs(t), np.maximum(sumG - 1, 1)), meanx
         if "two" in tests:  # R/plaid.R:488-520
-            sum1, sum0 = sumG, Gb.shape[0] - sumG
+            sum1, sum0 = sumG, ngenes - sumG
             ssq0, m0 = -q1 + (fc ** 2).sum(), -s1 + fc.sum()
             mean1, mean0 = s1 / (1e-8 + sum1), m0 / (1e-8 + sum0)
             var0 = (ssq0 - mean0 ** 2 * sum0) / (sum0 - 1)
@@ -533,19 +582,25 @@ def plaid_test(X: NamedMatrix, y, G: NamedMatrix, gsetX: Optional[NamedMatrix] =
             dof = varsum ** 2 / (var0 / sum0 * (sum0 - 1) + var1 / sum1 * (sum1 - 1))
             f = mean1 - mean0
             P["two"], Fs["two"] = 2.0 * stats.t.sf(np.abs(f / np.sqrt(varsum)), np.maximum(dof, 1)), f
-        if "lm" in tests:  # R/plaid.R:423-433
-            if gsetX is None:  # scores never leave the device: reductions fused onto the scoring call
-                _message("[plaid.test] computing plaid scores...")
-                gm = score_group_moments(NamedMatrix(Xs, gg, X.colnames), NamedMatrix(Gs, gg, G.colnames), y, ctx=ctx)
-            else:
-                gm = group_moments(gsetX.mat, y, ctx=ctx)
-            m1, m2 = gm[0] / n0, gm[2] / n1  # ina 1 = (y == 0), ina 2 = (y == 1)
-            v1 = (gm[1] - n0 * m1 ** 2) / (n0 - 1)
-            v2 = (gm[3] - n1 * m2 ** 2) / (n1 - 1)
-            fac = v1 / n0 + v2 / n1
-            stat = (m1 - m2) / np.sqrt(fac)
-            dof = fac ** 2 / ((v1 / n0) ** 2 / (n0 - 1) + (v2 / n1) ** 2 / (n1 - 1))
-            P["lm"], Fs["lm"] = 2.0 * stats.t.sf(np.abs(stat), dof), m2 - m1
+
+
+def _lm_test(s0, q0, n0, s1, q1, n1, P, Fs):
+    """Rfast::ttests(t(gsetX), ina = y + 1) (R/plaid.R:429-431) from the group sums / sums of squares: Welch's test
+    of group 1 against group 0"""
+    from scipy import stats
+    with np.errstate(invalid="ignore", divide="ignore"):
+        m1, m2 = s0 / n0, s1 / n1  # ina 1 = (y == 0), ina 2 = (y == 1)
+        v1 = (q0 - n0 * m1 ** 2) / (n0 - 1)
+        v2 = (q1 - n1 * m2 ** 2) / (n1 - 1)
+        fac = v1 / n0 + v2 / n1
+        stat = (m1 - m2) / np.sqrt(fac)
+        dof = fac ** 2 / ((v1 / n0) ** 2 / (n0 - 1) + (v2 / n1) ** 2 / (n1 - 1))
+        P["lm"], Fs["lm"] = 2.0 * stats.t.sf(np.abs(stat), dof), m2 - m1
+
+
+def _test_table(P, Fs, G: NamedMatrix, metap_method, sort_by):
+    """p-value clamp, meta p-value, FDR and the sorted result table of plaid.test (R/plaid.R:440-474)"""
+    from scipy import stats
     for k in P:
         p1 = np.where(np.isnan(P[k]), 1.0, P[k])
         P[k] = np.minimum(np.maximum(p1, 1e-99), 1 - 1e-99)
@@ -570,6 +625,93 @@ def plaid_test(X: NamedMatrix, y, G: NamedMatrix, gsetX: Optional[NamedMatrix] =
         oo = np.argsort(tab[:, cols.index(sort_by)], kind="stable")
         tab, rows = tab[oo], [rows[k] for k in oo]
     return tab, cols, rows
+
+
+def plaid_test(X: NamedMatrix, y, G: NamedMatrix, gsetX: Optional[NamedMatrix] = None, tests=("one", "two", "lm"),
+               metap_method: str = "fisher", sort_by: str = "p.meta", *, ctx=None):
+    """`plaid.test(X, y, G, gsetX, tests=c("one","two","lm"), metap.method="fisher", sort.by="p.meta")`
+    (R/plaid.R:392-474).  GPU: the score matrix (plaid), the crossprods of the one/two-sample tests
+    (chunked_crossprod on G != 0) and the per-set group moments of the "lm" test; host: pt / pchisq / p.adjust.
+    Returns (table, column names, row names) like the oracle."""
+    ctx = ctx or default_context()
+    y = np.asarray(y)
+    if not np.all(np.isin(np.unique(y), [0, 1])):
+        raise ValueError("elements of y must be 0 or 1")  # R/plaid.R:394
+    gg, Xs, Gs, Gb = _align(X, G)
+    n1, n0 = int((y == 1).sum()), int((y == 0).sum())
+    if sp.issparse(Xs):
+        fc = np.asarray(Xs[:, y == 1].sum(axis=1)).ravel() / n1 - np.asarray(Xs[:, y == 0].sum(axis=1)).ravel() / n0
+    else:
+        fc = Xs[:, y == 1].mean(axis=1) - Xs[:, y == 0].mean(axis=1)
+    sumG = np.asarray(Gb.sum(axis=0)).ravel()
+    P, Fs = {}, {}
+    if "one" in tests or "two" in tests:
+        cp = chunked_crossprod(Gb, np.column_stack([fc, fc ** 2]), ctx=ctx)  # crossprod(G != 0, [F, F^2]) on the GPU
+        _set_tests(tests, cp[:, 0], cp[:, 1], sumG, Gb.shape[0], fc, P, Fs)
+    if "lm" in tests:  # R/plaid.R:423-433
+        if gsetX is None:  # scores never leave the device: reductions fused onto the scoring call
+            _message("[plaid.test] computing plaid scores...")
+            gm = score_group_moments(NamedMatrix(Xs, gg, X.colnames), NamedMatrix(Gs, gg, G.colnames), y, ctx=ctx)
+        else:
+            gm = group_moments(gsetX.mat, y, ctx=ctx)
+        _lm_test(gm[0], gm[1], n0, gm[2], gm[3], n1, P, Fs)
+    return _test_table(P, Fs, G, metap_method, sort_by)
+
+
+def _missing(v) -> bool:
+    return v is None or v != v  # None or NaN
+
+
+def plaid_test_groups(X: NamedMatrix, groups, G: NamedMatrix, gsetX: Optional[NamedMatrix] = None,
+                      tests=("one", "two", "lm"), metap_method: str = "fisher", sort_by: str = "p.meta", *, ctx=None):
+    """plaid_test of every group against all other labelled cells, in one scoring pass.  `groups` holds one label per
+    cell of X; None / NaN leaves the cell out.  Returns {label: (table, column names, row names)} over the sorted
+    unique labels, each entry what `plaid_test(X[:, keep], groups[keep] == label, G, gsetX[:, keep])` returns with
+    keep = the labelled cells.  GPU: the scores and their per-group moments (score_group_stats, or group_stats on
+    gsetX) and one crossprod(G != 0, [F_1..F_K, F_1^2..F_K^2]); host: the per-group gene means (one sparse product)
+    and the distribution functions.  `ctx` may be a list of Contexts (the scores are then split over them)."""
+    ctx0 = (ctx[0] if isinstance(ctx, (list, tuple)) else ctx) or default_context()
+    groups = list(groups)
+    if len(groups) != X.shape[1]:
+        raise ValueError("length(groups) must equal ncol(X)")
+    keep = np.array([not _missing(v) for v in groups], dtype=bool)
+    levels = sorted(set(v for v, k in zip(groups, keep) if k))
+    if not levels:
+        raise ValueError("no cell has a group label")
+    index = {v: k for k, v in enumerate(levels)}
+    labels = np.array([index[v] if k else -1 for v, k in zip(groups, keep)], dtype=np.int32)
+    K = len(levels)
+    lab = labels[keep]
+    n = int(lab.size)
+    nk = np.bincount(lab, minlength=K).astype(np.float64)
+    gg, Xs, Gs, Gb = _align(X, G)
+    Xs = Xs[:, np.flatnonzero(keep)]
+    colnames = [X.colnames[j] for j in np.flatnonzero(keep)] if X.colnames is not None else None
+    P = [dict() for _ in range(K)]
+    Fs = [dict() for _ in range(K)]
+    with np.errstate(invalid="ignore", divide="ignore"):
+        if "one" in tests or "two" in tests:
+            onehot = sp.csc_matrix((np.ones(n), (np.arange(n), lab)), shape=(n, K))
+            gsum = np.asarray((Xs @ onehot).todense() if sp.issparse(Xs) else Xs @ onehot.toarray())  # genes x K
+            total = np.asarray(Xs.sum(axis=1)).ravel()
+            F = gsum / nk - (total[:, None] - gsum) / (n - nk)  # mean(group) - mean(other labelled cells)
+            alone = nk == n  # no other cell: F is NaN, and so is every statistic built on it
+            Fz = np.where(alone, 0.0, F)
+            cp = chunked_crossprod(Gb, np.column_stack([Fz, Fz ** 2]), ctx=ctx0)  # crossprod(G != 0, [F_k, F_k^2])
+            cp[:, np.concatenate([alone, alone])] = np.nan
+            sumG = np.asarray(Gb.sum(axis=0)).ravel()
+            for k in range(K):
+                _set_tests(tests, cp[:, k], cp[:, K + k], sumG, Gb.shape[0], F[:, k], P[k], Fs[k])
+        if "lm" in tests:
+            if gsetX is None:
+                _message("[plaid.test] computing plaid scores...")
+                gm = score_group_stats(NamedMatrix(Xs, gg, colnames), NamedMatrix(Gs, gg, G.colnames), lab, K, ctx=ctx)
+            else:
+                gm = group_stats(gsetX.mat, labels, K, ctx=ctx0)
+            tot = gm.sum(axis=0)  # all labelled cells: (2, S)
+            for k in range(K):
+                _lm_test(tot[0] - gm[k, 0], tot[1] - gm[k, 1], n - nk[k], gm[k, 0], gm[k, 1], nk[k], P[k], Fs[k])
+    return {levels[k]: _test_table(P[k], Fs[k], G, metap_method, sort_by) for k in range(K)}
 
 
 # ---------------------------------------------------------------------------------------

@@ -206,8 +206,9 @@ struct plaidgpu_ctx {
   int64_t h2d_piece = 0;
   bool h2d_pending = false;
   const int32_t* xp_host = nullptr;
-  // plaidgpu_score_group_moments: finish reduces the (fixed-up on the fly) scores instead of shipping them
-  const int32_t* mom_y = nullptr;
+  // plaidgpu_score_group_stats: finish reduces the (fixed-up on the fly) scores by group instead of shipping them
+  const int32_t* mom_labels = nullptr;
+  int mom_K = 0;
   double* mom_out = nullptr;
   // mailbox: pinned, device-mapped host memory the GPU writes small results into (launch_copy_words)
   void* mbox = nullptr;
@@ -944,6 +945,88 @@ double r_mean(const double* v, int64_t n) {  // base::mean(na.rm = TRUE): long d
   return (double)(s + t / (long double)m);
 }
 
+// ---- per-group moments (plaid.test "lm" for K groups) ---------------------------------------
+// labels: int32[N] in [-1, K); -1 = the column belongs to no group
+int check_groups(plaidgpu_ctx* c, const int32_t* labels, int64_t N, int K) {
+  if (K < 1) return fail(c, PLAIDGPU_ERR_ARG, "the number of groups K must be at least 1");
+  if (N > 0 && !labels) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  if (N >= INT32_MAX) return fail(c, PLAIDGPU_ERR_ARG, "group statistics take fewer than 2^31 columns per call");
+  for (int64_t j = 0; j < N; ++j)
+    if (labels[j] < -1 || labels[j] >= K)
+      return fail(c, PLAIDGPU_ERR_ARG, "label " + std::to_string(labels[j]) + " of column " + std::to_string(j) +
+                                           " is outside [-1, " + std::to_string(K) + ")");
+  return PLAIDGPU_OK;
+}
+
+// Column chunks of the reduction: up to 64 (and at least 64 columns each), fewer when the per-chunk partials of K
+// groups would exceed 1 GiB.  K <= 2 keeps min(64, N / 64) for any S below two million sets.
+int group_nchunk(int64_t N, int32_t S, int K) {
+  const double partial_budget = 1073741824.0;
+  int64_t n = std::min<int64_t>(64, N / 64);
+  n = std::min<int64_t>(n, (int64_t)(partial_budget / ((double)K * 2.0 * (double)S * 8.0)));
+  return (int)std::max<int64_t>(1, n);
+}
+
+// Per-group sums / sums of squares of the S x N device matrix dx (ld = S) into host out[K][2][S] (checked labels).
+// The host counting-sorts the labelled columns by (chunk, group), keeping column order inside a group, so each
+// group's values are added in column order within a chunk and the chunks in chunk order: for K = 2 and labels
+// y != 0 these are the additions of the two-group reduction this replaced, operation by operation.
+// fix / med / cc / alpha / beta: the fix-up of plaidgpu_score_finish, applied in registers to raw scores.
+int group_stats_device(plaidgpu_ctx* c, const double* dx, int32_t S, int64_t N, const int32_t* labels, int K, double* out,
+                       bool fix = false, const double* med = nullptr, double cc = 0.0, double alpha = 1.0,
+                       const double* beta = nullptr) {
+  const int nchunk = group_nchunk(N, S, K);
+  const int64_t nseg = (int64_t)nchunk * K;
+  std::vector<int32_t> plan((size_t)(nseg + 1 + N));  // seg[nseg + 1], then cols
+  int32_t* seg = plan.data();
+  int32_t* cols = seg + nseg + 1;
+  for (int ch = 0; ch < nchunk; ++ch)
+    for (int64_t j = (N * ch) / nchunk, j1 = (N * (ch + 1)) / nchunk; j < j1; ++j)
+      if (labels[j] >= 0) ++seg[(int64_t)ch * K + labels[j] + 1];
+  for (int64_t g = 0; g < nseg; ++g) seg[g + 1] += seg[g];
+  std::vector<int32_t> pos(seg, seg + nseg);
+  for (int ch = 0; ch < nchunk; ++ch)
+    for (int64_t j = (N * ch) / nchunk, j1 = (N * (ch + 1)) / nchunk; j < j1; ++j)
+      if (labels[j] >= 0) cols[pos[(size_t)((int64_t)ch * K + labels[j])]++] = (int32_t)j;
+  const int64_t words = nseg + 1 + seg[nseg];
+  CK(c->b_i32.reserve((size_t)words * sizeof(int32_t)));
+  CK(cudaMemcpyAsync(c->b_i32.p, plan.data(), (size_t)words * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+  const int64_t width = (int64_t)K * 2 * S;
+  CK(c->b_rowa.reserve((size_t)(nseg * 2 * S) * sizeof(double)));
+  CK(c->b_rowb.reserve((size_t)width * sizeof(double)));
+  CK(cudaEventRecord(c->ev[4], c->stream));
+  const int32_t* dseg = c->b_i32.as<int32_t>();
+  CK(launch_group_stats(dx, S, S, K, dseg + nseg + 1, dseg, nchunk, c->b_rowa.as<double>(), c->b_rowb.as<double>(),
+                        c->stream, fix, med, cc, alpha, beta));
+  c->launches += 2;
+  CK(cudaEventRecord(c->ev[5], c->stream));
+  const SmallRead it[1] = {{out, c->b_rowb.p, width}};
+  int rc = read_small(c, it, 1);  // synchronises the stream: `plan` may go
+  if (rc) return rc;
+  float ms = 0.f;
+  cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]);
+  c->ms[2] = ms;
+  return PLAIDGPU_OK;
+}
+
+// Host X and host output larger than the device can hold: the column tile width score_chunked should use, or 0
+// when one pass fits (the raw scores get 45 % of the free memory; X, ranks and slack share the rest)
+int host_chunk_cols(plaidgpu_ctx* c, const plaidgpu_matrix* X, int64_t* chunk) {
+  *chunk = 0;
+  if (!c->have_g || X->location != PLAIDGPU_HOST || X->N <= 1) return PLAIDGPU_OK;
+  CK(cudaSetDevice(c->device));
+  size_t free_b = 0, total_b = 0;
+  CK(cudaMemGetInfo(&free_b, &total_b));
+  double budget = 0.45 * (double)free_b + (double)c->b_raw.cap;
+  if (const char* e = getenv("PLAIDGPU_MAX_OUT_BYTES")) budget = atof(e);  // test knob
+  if ((double)c->S * (double)X->N * 8.0 <= budget) return PLAIDGPU_OK;
+  int64_t ch = (int64_t)(budget / ((double)c->S * 8.0));
+  if (ch < 1) ch = 1;
+  if (ch > 32) ch = (ch / 32) * 32;
+  *chunk = ch;
+  return PLAIDGPU_OK;
+}
+
 }  // namespace
 
 // =========================================================================================
@@ -1675,7 +1758,7 @@ int plaidgpu_combine_medians(int ignore_zero_opt, double score_min, const double
 
 int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double* out) try {
   if (!c) return PLAIDGPU_ERR_ARG;
-  if (!scal || (!out && c->N > 0 && !c->mom_y)) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  if (!scal || (!out && c->N > 0 && !c->mom_labels)) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
   if (!c->computed) return fail(c, PLAIDGPU_ERR_STATE, "plaidgpu_score_compute has not been called");
   CK(cudaSetDevice(c->device));
   const plaidgpu_opts& o = c->opts;
@@ -1705,30 +1788,15 @@ int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double*
     fix = true;
   }
 
-  if (c->mom_y) {
+  if (c->mom_labels) {
     // score -> test: per-set sums / sums of squares of the normalised scores by sample group, the fix-up applied in
-    // registers; the S x N matrix stays on the device as raw scores and nothing but 4 S doubles goes back
-    const int32_t* y = c->mom_y;
+    // registers; the S x N matrix stays on the device as raw scores and nothing but K * 2 * S doubles goes back
+    const int32_t* lab = c->mom_labels;
+    const int K = c->mom_K;
     double* mo = c->mom_out;
-    c->mom_y = nullptr;
+    c->mom_labels = nullptr;
     c->mom_out = nullptr;
-    const int nchunk = (int)std::max<int64_t>(1, std::min<int64_t>(64, N / 64));
-    CK(c->b_i32.reserve((size_t)std::max<int64_t>(N, 1) * sizeof(int32_t)));
-    if (N) CK(cudaMemcpyAsync(c->b_i32.p, y, (size_t)N * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
-    CK(c->b_rowa.reserve((size_t)nchunk * 4 * S * sizeof(double)));
-    CK(c->b_rowb.reserve((size_t)4 * S * sizeof(double)));
-    CK(cudaEventRecord(c->ev[4], c->stream));
-    CK(launch_group_moments(c->raw, S, S, N, c->b_i32.as<int32_t>(), nchunk, c->b_rowa.as<double>(), c->b_rowb.as<double>(),
-                            c->stream, fix, med, cc, alpha, beta));
-    c->launches += 2;
-    CK(cudaEventRecord(c->ev[5], c->stream));
-    const SmallRead it[1] = {{mo, c->b_rowb.p, 4 * (int64_t)S}};
-    int rcm = read_small(c, it, 1);
-    if (rcm) return rcm;
-    float msm = 0.f;
-    cudaEventElapsedTime(&msm, c->ev[4], c->ev[5]);
-    c->ms[2] = msm;
-    return PLAIDGPU_OK;
+    return group_stats_device(c, c->raw, S, N, lab, K, mo, fix, med, cc, alpha, beta);
   }
   c->raw_valid = false;  // the fix-up below rewrites the raw scores in place
   CK(cudaEventRecord(c->ev[4], c->stream));
@@ -1873,8 +1941,17 @@ int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double*
 // scores over PCIe twice).  Results are bit-identical to the un-chunked path.
 // `sink` (optional): instead of landing in `out`, every finished chunk is staged in a pinned buffer and
 // written to the file — tiled egress for results larger than host memory (scope row f4).
+// `groups` (optional): every finished chunk is reduced per set and sample group on the device instead
+// (plaidgpu_score_group_stats), into groups->tile, and `out` (K * 2 * S doubles, zeroed by the caller)
+// accumulates the tiles in tile order.
+struct GroupSink {
+  const int32_t* labels;  // int32[N] of the whole call
+  int K;
+  double* tile;           // K * 2 * S doubles of host scratch
+};
 static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
-                         double* out, int64_t chunk, FILE* sink = nullptr, double* stage = nullptr, double* stage2 = nullptr) {
+                         double* out, int64_t chunk, FILE* sink = nullptr, double* stage = nullptr, double* stage2 = nullptr,
+                         const GroupSink* groups = nullptr) {
   const int64_t N = X->N;
   const int32_t S = c->S;
   if (opts->scorer == PLAIDGPU_GSVA && opts->gsva_ecdf != PLAIDGPU_ROWTF_DONE &&
@@ -1964,6 +2041,17 @@ static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_
     if (rc) return rc;
     s.ignore_zero = g.ignore_zero;
     s.med_mean = g.med_mean;
+    if (groups) {
+      c->mom_labels = groups->labels + j0;
+      c->mom_K = groups->K;
+      c->mom_out = groups->tile;
+      rc = plaidgpu_score_finish(c, &s, nullptr);
+      c->mom_labels = nullptr;
+      c->mom_out = nullptr;
+      if (rc) return rc;
+      for (int64_t i = 0, w = (int64_t)groups->K * 2 * S; i < w; ++i) out[i] += groups->tile[i];
+      continue;
+    }
     double* dst = sink ? ((stage2 && (tile & 1)) ? stage2 : stage) : out + j0 * (int64_t)S;
     if (sink && !stage2 && writer.joinable()) writer.join();  // one buffer only: it must be free again
     rc = plaidgpu_score_finish(c, &s, dst);
@@ -2047,19 +2135,11 @@ int plaidgpu_score(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* row
   if (!c) return PLAIDGPU_ERR_ARG;
   if (!X || !opts) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
   // host in / host out larger than the device can hold -> column chunks
-  if (c->have_g && X->location == PLAIDGPU_HOST && opts->out_location == PLAIDGPU_HOST && X->N > 1) {
-    CK(cudaSetDevice(c->device));
-    size_t free_b = 0, total_b = 0;
-    CK(cudaMemGetInfo(&free_b, &total_b));
-    double budget = 0.45 * (double)free_b + (double)c->b_raw.cap;  // raw scores; X, ranks and slack share the rest
-    if (const char* e = getenv("PLAIDGPU_MAX_OUT_BYTES")) budget = atof(e);  // test knob
-    const double need = (double)c->S * (double)X->N * 8.0;
-    if (need > budget) {
-      int64_t chunk = (int64_t)(budget / ((double)c->S * 8.0));
-      if (chunk < 1) chunk = 1;
-      if (chunk > 32) chunk = (chunk / 32) * 32;
-      return score_chunked(c, X, rowmap, opts, out, chunk);
-    }
+  if (opts->out_location == PLAIDGPU_HOST) {
+    int64_t chunk = 0;
+    int rc = host_chunk_cols(c, X, &chunk);
+    if (rc) return rc;
+    if (chunk > 0) return score_chunked(c, X, rowmap, opts, out, chunk);
   }
   plaidgpu_scalars s;
   int rc = plaidgpu_score_begin(c, X, rowmap, opts, &s);
@@ -2084,15 +2164,28 @@ int plaidgpu_score(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* row
 
 // score -> test fused ("next" row f1 as specified): plaid() / a replaid.* scorer followed by the per-set group moments of
 // plaid.test(tests = "lm") (R/plaid.R:426-431) without the S x N matrix ever leaving the device or being written in
-// its normalised form.  Bit-identical to plaidgpu_score + plaidgpu_group_moments.
-int plaidgpu_score_group_moments(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
-                                 const int32_t* y, double* out) try {
+// its normalised form.  Bit-identical to plaidgpu_score + plaidgpu_group_stats.  Host X whose S x N scores exceed
+// the device goes through score_chunked (two passes when normalised) and adds the tiles' moments in tile order.
+int plaidgpu_score_group_stats(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
+                               const int32_t* labels, int K, double* out) try {
   if (!c) return PLAIDGPU_ERR_ARG;
-  if (!X || !opts || !y || !out) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  if (!X || !rowmap || !opts || !out) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  int rc = check_groups(c, labels, X->N, K);
+  if (rc) return rc;
   plaidgpu_opts o = *opts;
   o.out_location = PLAIDGPU_HOST;  // raw scores in the library's device buffer
+  int64_t chunk = 0;
+  rc = host_chunk_cols(c, X, &chunk);
+  if (rc) return rc;
+  if (chunk > 0) {
+    const size_t width = (size_t)K * 2 * (size_t)c->S;
+    std::vector<double> tile(width);
+    std::fill(out, out + width, 0.0);
+    const GroupSink gs{labels, K, tile.data()};
+    return score_chunked(c, X, rowmap, &o, out, chunk, nullptr, nullptr, nullptr, &gs);
+  }
   plaidgpu_scalars s;
-  int rc = plaidgpu_score_begin(c, X, rowmap, &o, &s);
+  rc = plaidgpu_score_begin(c, X, rowmap, &o, &s);
   if (rc) return rc;
   rc = plaidgpu_score_compute(c, &s, nullptr);
   if (rc) return rc;
@@ -2104,12 +2197,27 @@ int plaidgpu_score_group_moments(plaidgpu_ctx* c, const plaidgpu_matrix* X, cons
     rc = plaidgpu_combine_medians(o.ignore_zero, s.score_min, m, m, c->N, &s);
     if (rc) return fail(c, rc, "combine_medians failed");
   }
-  c->mom_y = y;
+  c->mom_labels = labels;
+  c->mom_K = K;
   c->mom_out = out;
   rc = plaidgpu_score_finish(c, &s, nullptr);
-  c->mom_y = nullptr;
+  c->mom_labels = nullptr;
   c->mom_out = nullptr;
   return rc;
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
+// two groups y != 0 / y == 0: the labels of plaidgpu_score_group_stats with K = 2
+int plaidgpu_score_group_moments(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
+                                 const int32_t* y, double* out) try {
+  if (!c) return PLAIDGPU_ERR_ARG;
+  if (!X || !opts || !y || !out) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  std::vector<int32_t> lab((size_t)std::max<int64_t>(X->N, 0));
+  for (size_t j = 0; j < lab.size(); ++j) lab[j] = y[j] != 0;
+  return plaidgpu_score_group_stats(c, X, rowmap, opts, lab.data(), 2, out);
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {
@@ -2141,22 +2249,21 @@ struct ShardBarrier {
 };
 }  // namespace
 
-int plaidgpu_score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
-                         const plaidgpu_opts* opts, double* out) try {
-  if (!ctxs || n <= 0 || !ctxs[0]) return PLAIDGPU_ERR_ARG;
+// labels == nullptr: the S x N scores land in `out` (plaidgpu_score_multi).  Otherwise every shard reduces its scores
+// per set and group on its device (plaidgpu_score_group_stats) and `out` (K * 2 * S doubles) receives the shards'
+// moments added in shard order (plaidgpu_score_group_stats_multi).
+static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
+                            const plaidgpu_opts* opts, double* out, const int32_t* labels, int K, const char* name) {
   plaidgpu_ctx* c = ctxs[0];
-  if (!X || !rowmap || !opts) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
-  if (X->location != PLAIDGPU_HOST || opts->out_location != PLAIDGPU_HOST)
-    return fail(c, PLAIDGPU_ERR_ARG, "plaidgpu_score_multi: X and out must be in host memory");
-  if (n == 1 || X->N < 2 * (int64_t)n) return plaidgpu_score(c, X, rowmap, opts, out);
+  const std::string who(name);
   for (int r = 0; r < n; ++r) {
-    if (!ctxs[r] || !ctxs[r]->have_g) return fail(c, PLAIDGPU_ERR_STATE, "plaidgpu_score_multi: every context needs plaidgpu_set_genesets");
-    if (ctxs[r]->S != c->S) return fail(c, PLAIDGPU_ERR_ARG, "plaidgpu_score_multi: contexts hold different gene sets");
+    if (!ctxs[r] || !ctxs[r]->have_g) return fail(c, PLAIDGPU_ERR_STATE, who + ": every context needs plaidgpu_set_genesets");
+    if (ctxs[r]->S != c->S) return fail(c, PLAIDGPU_ERR_ARG, who + ": contexts hold different gene sets");
     for (int q = 0; q < r; ++q)
-      if (ctxs[q] == ctxs[r]) return fail(c, PLAIDGPU_ERR_ARG, "plaidgpu_score_multi: the same context twice");
+      if (ctxs[q] == ctxs[r]) return fail(c, PLAIDGPU_ERR_ARG, who + ": the same context twice");
   }
   if (opts->scorer == PLAIDGPU_GSVA && opts->gsva_ecdf == PLAIDGPU_ROWTF_ECDF)
-    return fail(c, PLAIDGPU_ERR_ARG, "plaidgpu_score_multi: gsva rowtf = ecdf ranks across samples (use one context, or the row exchange of plaid_b200/sharded.py)");
+    return fail(c, PLAIDGPU_ERR_ARG, who + ": gsva rowtf = ecdf ranks across samples (use one context, or the row exchange of plaid_b200/sharded.py)");
   try {
     const int64_t N = X->N;
     const int32_t S = c->S, P = X->P;
@@ -2182,6 +2289,8 @@ int plaidgpu_score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix
     }
     std::vector<plaidgpu_scalars> loc((size_t)n);
     std::vector<int> rc((size_t)n, PLAIDGPU_OK);
+    const size_t width = labels ? (size_t)K * 2 * (size_t)S : 0;
+    std::vector<std::vector<double>> moments(labels ? (size_t)n : 0, std::vector<double>(width));
     std::vector<double> med((size_t)std::max<int64_t>(N, 1));
     std::vector<std::vector<double>> part(gsva_z ? (size_t)n : 0, std::vector<double>((size_t)P));
     std::vector<double> rmean(gsva_z ? (size_t)P : 0), rsd(gsva_z ? (size_t)P : 0);
@@ -2196,6 +2305,8 @@ int plaidgpu_score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix
     auto body = [&](int r) {
       plaidgpu_ctx* cr = ctxs[r];
       plaidgpu_opts o = *opts;
+      if (labels) o.out_location = PLAIDGPU_HOST;  // raw scores stay in the context's device buffer
+      double* dst = labels ? nullptr : out + lo[r] * (int64_t)S;
       if (gsva_z) {  // rowMeans / rowSds over ALL shards, summed in shard order (R/plaid.R:343)
         rc[r] = plaidgpu_row_moments(cr, &M[r], nullptr, part[r].data());
         bar.wait();
@@ -2229,7 +2340,7 @@ int plaidgpu_score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix
         s.x_max = fmax(s.x_max, loc[k].x_max);
         s.rank_max = fmax(s.rank_max, loc[k].rank_max);
       }
-      rc[r] = plaidgpu_score_compute(cr, &s, out + lo[r] * (int64_t)S);
+      rc[r] = plaidgpu_score_compute(cr, &s, dst);
       loc[r].score_min = s.score_min;
       bar.wait();
       if (failed()) return;
@@ -2247,7 +2358,14 @@ int plaidgpu_score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix
         s.med_mean = g.med_mean;
         s.score_min = smin;
       }
-      rc[r] = plaidgpu_score_finish(cr, &s, out + lo[r] * (int64_t)S);
+      if (labels) {
+        cr->mom_labels = labels + lo[r];
+        cr->mom_K = K;
+        cr->mom_out = moments[r].data();
+      }
+      rc[r] = plaidgpu_score_finish(cr, &s, dst);
+      cr->mom_labels = nullptr;
+      cr->mom_out = nullptr;
     };
     std::vector<std::thread> th;
     for (int r = 1; r < n; ++r) th.emplace_back(body, r);
@@ -2258,12 +2376,44 @@ int plaidgpu_score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix
         if (r > 0) c->err = "shard " + std::to_string(r) + ": " + ctxs[r]->err;
         return rc[r];
       }
+    if (labels) {
+      std::copy(moments[0].begin(), moments[0].end(), out);
+      for (int r = 1; r < n; ++r)
+        for (size_t i = 0; i < width; ++i) out[i] += moments[r][i];
+    }
     return PLAIDGPU_OK;
   } catch (const std::bad_alloc&) {
     return fail(c, PLAIDGPU_ERR_NOMEM, "out of host memory");
   } catch (...) {
-    return fail(c, PLAIDGPU_ERR_ARG, "unexpected failure in plaidgpu_score_multi");
+    return fail(c, PLAIDGPU_ERR_ARG, "unexpected failure in " + who);
   }
+}
+
+int plaidgpu_score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
+                         const plaidgpu_opts* opts, double* out) try {
+  if (!ctxs || n <= 0 || !ctxs[0]) return PLAIDGPU_ERR_ARG;
+  plaidgpu_ctx* c = ctxs[0];
+  if (!X || !rowmap || !opts) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  if (X->location != PLAIDGPU_HOST || opts->out_location != PLAIDGPU_HOST)
+    return fail(c, PLAIDGPU_ERR_ARG, "plaidgpu_score_multi: X and out must be in host memory");
+  if (n == 1 || X->N < 2 * (int64_t)n) return plaidgpu_score(c, X, rowmap, opts, out);
+  return score_multi_impl(ctxs, n, X, rowmap, opts, out, nullptr, 0, "plaidgpu_score_multi");
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
+int plaidgpu_score_group_stats_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
+                                     const plaidgpu_opts* opts, const int32_t* labels, int K, double* out) try {
+  if (!ctxs || n <= 0 || !ctxs[0]) return PLAIDGPU_ERR_ARG;
+  plaidgpu_ctx* c = ctxs[0];
+  if (!X || !rowmap || !opts || !out) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  if (X->location != PLAIDGPU_HOST) return fail(c, PLAIDGPU_ERR_ARG, "plaidgpu_score_group_stats_multi: X must be in host memory");
+  if (n == 1 || X->N < 2 * (int64_t)n) return plaidgpu_score_group_stats(c, X, rowmap, opts, labels, K, out);
+  int rc = check_groups(c, labels, X->N, K);
+  if (rc) return rc;
+  return score_multi_impl(ctxs, n, X, rowmap, opts, out, labels, K, "plaidgpu_score_group_stats_multi");
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {
@@ -2425,10 +2575,13 @@ int plaidgpu_colranks(plaidgpu_ctx* c, const plaidgpu_matrix* X, int ties, int i
   return PLAIDGPU_ERR_ARG;
 }
 
-int plaidgpu_group_moments(plaidgpu_ctx* c, const double* x, int32_t S, int64_t N, const int32_t* y, int location,
-                           double* out) try {
+int plaidgpu_group_stats(plaidgpu_ctx* c, const double* x, int32_t S, int64_t N, const int32_t* labels, int K, int location,
+                         double* out) try {
   if (!c) return PLAIDGPU_ERR_ARG;
-  if (S <= 0 || N < 0 || !out || (N > 0 && (!x || !y))) return fail(c, PLAIDGPU_ERR_ARG, "bad argument");
+  if (S <= 0 || N < 0) return fail(c, PLAIDGPU_ERR_ARG, "bad argument");
+  if (!out || (N > 0 && !x)) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  int rc = check_groups(c, labels, N, K);
+  if (rc) return rc;
   CK(cudaSetDevice(c->device));
   const int64_t total = (int64_t)S * N;
   const double* dx = x;
@@ -2437,17 +2590,21 @@ int plaidgpu_group_moments(plaidgpu_ctx* c, const double* x, int32_t S, int64_t 
     if (total) CK(cudaMemcpyAsync(c->b_raw.p, x, (size_t)total * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     dx = c->b_raw.as<double>();
   }
-  const int nchunk = (int)std::max<int64_t>(1, std::min<int64_t>(64, N / 64));
-  CK(c->b_i32.reserve((size_t)std::max<int64_t>(N, 1) * sizeof(int32_t)));
-  if (N) CK(cudaMemcpyAsync(c->b_i32.p, y, (size_t)N * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
-  CK(c->b_rowa.reserve((size_t)nchunk * 4 * S * sizeof(double)));
-  CK(c->b_rowb.reserve((size_t)4 * S * sizeof(double)));
-  CK(launch_group_moments(dx, S, S, N, c->b_i32.as<int32_t>(), nchunk, c->b_rowa.as<double>(), c->b_rowb.as<double>(),
-                          c->stream));
-  c->launches += 2;
-  CK(cudaMemcpyAsync(out, c->b_rowb.p, (size_t)4 * S * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-  CK(cudaStreamSynchronize(c->stream));
-  return PLAIDGPU_OK;
+  return group_stats_device(c, dx, S, N, labels, K, out);
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
+// two groups y != 0 / y == 0: the labels of plaidgpu_group_stats with K = 2
+int plaidgpu_group_moments(plaidgpu_ctx* c, const double* x, int32_t S, int64_t N, const int32_t* y, int location,
+                           double* out) try {
+  if (!c) return PLAIDGPU_ERR_ARG;
+  if (S <= 0 || N < 0 || !out || (N > 0 && (!x || !y))) return fail(c, PLAIDGPU_ERR_ARG, "bad argument");
+  std::vector<int32_t> lab((size_t)N);
+  for (int64_t j = 0; j < N; ++j) lab[(size_t)j] = y[j] != 0;
+  return plaidgpu_group_stats(c, x, S, N, lab.data(), 2, location, out);
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {

@@ -181,12 +181,14 @@ cudaError_t launch_colstats(const double* x, int64_t ld, int32_t S, int64_t N, d
 cudaError_t launch_fixup(const double* x, double* out, int64_t ld, int32_t S, int64_t j0, int64_t j1,
                          const double* med, double c, double alpha, const double* beta,
                          cudaStream_t st);
-// per-row sums / sums of squares by column group (plaid.test "lm"): partial = nchunk * 4 * S doubles of scratch,
-// out = 4 * S doubles {sum0, sumsq0, sum1, sumsq1}; fixed summation order
+// per-row sums / sums of squares by column group (plaid.test "lm" for K groups).  cols / seg: the labelled columns
+// sorted by (chunk, group), column order kept inside a group; segment g = chunk * K + group is cols[seg[g], seg[g+1])
+// (group_stats_plan in api.cu builds them).  partial = nchunk * K * 2 * S doubles of scratch, out = K * 2 * S doubles
+// {sum_k[S], sumsq_k[S]} per group; fixed summation order.
 // fix: x holds RAW scores and out = moments of alpha * (x - med_j + c) + beta_s, applied on the fly (k_fixup's arithmetic)
-cudaError_t launch_group_moments(const double* x, int64_t ld, int32_t S, int64_t N, const int32_t* y, int nchunk,
-                                 double* partial, double* out, cudaStream_t st, bool fix = false, const double* med = nullptr,
-                                 double c = 0.0, double alpha = 1.0, const double* beta = nullptr);
+cudaError_t launch_group_stats(const double* x, int64_t ld, int32_t S, int K, const int32_t* cols, const int32_t* seg,
+                               int nchunk, double* partial, double* out, cudaStream_t st, bool fix = false,
+                               const double* med = nullptr, double c = 0.0, double alpha = 1.0, const double* beta = nullptr);
 // nwords 8-byte words device -> host-mapped (cudaHostAllocMapped) memory by a kernel, bypassing the copy engine
 cudaError_t launch_copy_words(const void* src, void* dst_mapped, int64_t nwords, cudaStream_t st);
 // global min / max of a device array of n doubles, NaN ignored (na.rm = TRUE); res[0]=min res[1]=max

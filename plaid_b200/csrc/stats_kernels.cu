@@ -1100,50 +1100,48 @@ __global__ void __launch_bounds__(256) k_minmax(const double* __restrict__ x, in
   }
 }
 
-// row sums / sums of squares of a column-major S x N matrix by column group y[j] in {0,1}.
-// grid = (row blocks, column chunks); partial[chunk][4][S] are combined in chunk order by k_group_combine.
+// row sums / sums of squares of a column-major S x N matrix by column group (labels in [0, K); unlabelled columns
+// take no part).  The host sorts the labelled columns by (chunk, group), ascending inside each group, into `cols`;
+// segment g = chunk * K + group is cols[seg[g] .. seg[g + 1]).  grid = (segments, row blocks): each thread owns one
+// set row and adds the segment's columns in ascending order, so every score is read once whatever K is, and
+// partial[g][2][S] = {sum, sumsq} of that segment; k_group_combine adds the segments of one group in chunk order.
 // FIX: the values are RAW scores and the fix-up of normalize_medians / replaid.ucell (k_fixup: alpha * (x + (c - med_j))
 // [+ beta_s], the same operations in the same order) is applied in registers — the normalised matrix is never
-// written (plaidgpu_score_group_moments: score -> test without materialising S x N for the host).
+// written (plaidgpu_score_group_stats: score -> test without materialising S x N for the host).
 template <bool FIX>
-__global__ void __launch_bounds__(256) k_group_partial(const double* __restrict__ x, int64_t ld, int32_t S, int64_t N,
-                                                       const int32_t* __restrict__ y, int nchunk,
+__global__ void __launch_bounds__(256) k_group_partial(const double* __restrict__ x, int64_t ld, int32_t S,
+                                                       const int32_t* __restrict__ cols, const int32_t* __restrict__ seg,
                                                        double* __restrict__ partial, const double* __restrict__ med,
                                                        double c, double alpha, const double* __restrict__ beta) {
-  const int r = blockIdx.x * blockDim.x + threadIdx.x;
-  const int ch = blockIdx.y;
-  const int64_t j0 = (N * ch) / nchunk, j1 = (N * (ch + 1)) / nchunk;
-  double s0 = 0.0, q0 = 0.0, s1 = 0.0, q1 = 0.0;
-  if (r < S) {
-    const double b = (FIX && beta) ? beta[r] : 0.0;
-    for (int64_t j = j0; j < j1; ++j) {
-      double v = __ldcs(x + j * ld + r);
-      if (FIX) {
-        const double shift = (med ? -med[j] : 0.0) + c;
-        v = __dmul_rn(alpha, __dadd_rn(v, shift));
-        if (beta) v = __dadd_rn(v, b);
-      }
-      if (y[j]) {
-        s1 += v;
-        q1 += v * v;
-      } else {
-        s0 += v;
-        q0 += v * v;
-      }
+  const int r = blockIdx.y * blockDim.x + threadIdx.x;
+  const int64_t g = blockIdx.x;
+  if (r >= S) return;
+  const int32_t i0 = seg[g], i1 = seg[g + 1];
+  const double b = (FIX && beta) ? beta[r] : 0.0;
+  double s = 0.0, q = 0.0;
+#pragma unroll 4
+  for (int32_t i = i0; i < i1; ++i) {
+    const int64_t j = cols[i];
+    double v = __ldcs(x + j * ld + r);
+    if (FIX) {
+      const double shift = (med ? -med[j] : 0.0) + c;
+      v = __dmul_rn(alpha, __dadd_rn(v, shift));
+      if (beta) v = __dadd_rn(v, b);
     }
-    double* p = partial + (size_t)ch * 4 * S;
-    p[r] = s0;
-    p[S + r] = q0;
-    p[2 * (size_t)S + r] = s1;
-    p[3 * (size_t)S + r] = q1;
+    s += v;
+    q += v * v;
   }
+  double* p = partial + (size_t)g * 2 * S;
+  p[r] = s;
+  p[S + r] = q;
 }
-__global__ void __launch_bounds__(256) k_group_combine(const double* __restrict__ partial, int32_t S, int nchunk,
+// out[i] = sum over chunks, in chunk order, of partial[chunk][i]; i < width = K * 2 * S
+__global__ void __launch_bounds__(256) k_group_combine(const double* __restrict__ partial, int64_t width, int nchunk,
                                                        double* __restrict__ out) {
   const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (i >= 4 * (int64_t)S) return;
+  if (i >= width) return;
   double a = 0.0;
-  for (int ch = 0; ch < nchunk; ++ch) a += partial[(size_t)ch * 4 * S + i];
+  for (int ch = 0; ch < nchunk; ++ch) a += partial[(size_t)ch * width + i];
   out[i] = a;
 }
 
@@ -1271,16 +1269,17 @@ cudaError_t launch_fixup(const double* x, double* out, int64_t ld, int32_t S, in
   return cudaGetLastError();
 }
 
-cudaError_t launch_group_moments(const double* x, int64_t ld, int32_t S, int64_t N, const int32_t* y, int nchunk,
-                                 double* partial, double* out, cudaStream_t st, bool fix, const double* med, double c,
-                                 double alpha, const double* beta) {
-  if (S <= 0) return cudaSuccess;
-  dim3 g((unsigned)((S + 255) / 256), (unsigned)nchunk);
-  if (fix) k_group_partial<true><<<g, 256, 0, st>>>(x, ld, S, N, y, nchunk, partial, med, c, alpha, beta);
-  else k_group_partial<false><<<g, 256, 0, st>>>(x, ld, S, N, y, nchunk, partial, nullptr, 0.0, 1.0, nullptr);
+cudaError_t launch_group_stats(const double* x, int64_t ld, int32_t S, int K, const int32_t* cols, const int32_t* seg,
+                               int nchunk, double* partial, double* out, cudaStream_t st, bool fix, const double* med,
+                               double c, double alpha, const double* beta) {
+  if (S <= 0 || K <= 0) return cudaSuccess;
+  dim3 g((unsigned)((int64_t)nchunk * K), (unsigned)((S + 255) / 256));
+  if (fix) k_group_partial<true><<<g, 256, 0, st>>>(x, ld, S, cols, seg, partial, med, c, alpha, beta);
+  else k_group_partial<false><<<g, 256, 0, st>>>(x, ld, S, cols, seg, partial, nullptr, 0.0, 1.0, nullptr);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
-  k_group_combine<<<(unsigned)((4 * (int64_t)S + 255) / 256), 256, 0, st>>>(partial, S, nchunk, out);
+  const int64_t width = (int64_t)K * 2 * S;
+  k_group_combine<<<(unsigned)((width + 255) / 256), 256, 0, st>>>(partial, width, nchunk, out);
   return cudaGetLastError();
 }
 

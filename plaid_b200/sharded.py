@@ -250,6 +250,24 @@ def score_shard(ctx, comm, M: L.Matrix, rowmap: np.ndarray, opts: L.Opts, out_pt
     return scal
 
 
+def score_group_stats_shard(ctx, comm, M: L.Matrix, rowmap: np.ndarray, opts: L.Opts, labels, K: int, n_cols: int):
+    """Per-group sums / sums of squares of this rank's scores, summed over all ranks (in rank order): score_shard into
+    a device buffer, plaidgpu_group_stats on it, then one all-reduce of K * 2 * S doubles.  labels: int32[n_cols] of
+    this shard's columns in [-1, K).  `ctx` must hold the gene sets (Context.set_genesets).  Returns (K, 2, S)."""
+    import torch
+    S = ctx.n_sets
+    lab = np.ascontiguousarray(labels, dtype=np.int32)
+    if lab.size != n_cols:
+        raise ValueError("length(labels) must equal the shard's column count")
+    buf = torch.empty(max(S * n_cols, 1), dtype=torch.float64, device=f"cuda:{ctx.device}")
+    opts.out_location = L.DEVICE
+    score_shard(ctx, comm, M, rowmap, opts, buf.data_ptr(), n_cols)
+    out = np.empty((int(K), 2, S), dtype=np.float64)
+    ctx.check(ctx.lib.plaidgpu_group_stats(ctx.h, buf.data_ptr(), S, n_cols, lab.ctypes.data, int(K), L.DEVICE,
+                                           out.ctypes.data))
+    return comm.allreduce_sum_vec(out.ravel()).reshape(out.shape)
+
+
 def shard_columns(n_total: int, world: int, rank: int):
     """contiguous, equal-count column ranges (equal output bytes, the dominant cost)"""
     base, rem = divmod(n_total, world)

@@ -37,7 +37,7 @@
   }
 }
 
-.score <- function(X, matG, opts, y = NULL) {
+.score <- function(X, matG, opts, labels = NULL, K = NULL) {
   x <- .as_x(X)
   rn <- x$dimnames[[1]]
   gg <- intersect(rn, rownames(matG))                                 # R/plaid.R:65
@@ -51,9 +51,9 @@
   rowmap[is.na(rowmap) | duplicated(rn)] <- -1L
   G <- methods::as(matG, "CsparseMatrix")
   if (!inherits(G, "dgCMatrix")) G <- methods::as(methods::as(G, "dMatrix"), "generalMatrix")
-  if (!is.null(y)) {  # plaid.test("lm"): scores reduced per set and sample group on the device, S x 4 back
-    out <- .Call(C_plaidgpu_score_group_moments, .ctxs(), x$kind, x$p, x$i, x$x, as.integer(x$dim),
-                 G@p, G@i, G@x, as.integer(dim(G)), as.integer(rowmap), opts, as.integer(y))
+  if (!is.null(labels)) {  # plaid.test("lm"): scores reduced per set and sample group on the device, S x 2K back
+    out <- .Call(C_plaidgpu_score_group_stats, .ctxs(), x$kind, x$p, x$i, x$x, as.integer(x$dim),
+                 G@p, G@i, G@x, as.integer(dim(G)), as.integer(rowmap), opts, as.integer(labels), as.integer(K))
     rownames(out) <- colnames(matG)
     return(out)
   }
@@ -142,24 +142,9 @@ replaid.gsva <- function(X, matG, tau = 0, rowtf = c("z", "ecdf")[1]) {      # R
   .score(X, matG, list(scorer = 6L, tau = as.numeric(tau), gsva_ecdf = as.integer(rowtf == "ecdf")))
 }
 
-## plaid.test (R/plaid.R:392-474): same arguments and result table; the score matrix, the set-wise sums of
-## logFC / logFC^2 and the per-set group moments come from the GPU, pt / pchisq / p.adjust stay in R.
-plaid.test <- function(X, y, G, gsetX, tests = c("one", "two", "lm"),
-                       metap.method = "fisher", sort.by = "p.meta") {
-  if (!all(unique(y) %in% c(0, 1))) stop("elements of y must be 0 or 1")
-  if (is.list(G)) G <- gmt2mat(G)                                      # R/plaid.R: a GMT list is converted first
-  gg <- intersect(rownames(G), rownames(X))
-  X <- X[gg, , drop = FALSE]
-  G <- G[gg, , drop = FALSE]
-  n1 <- sum(y == 1); n0 <- sum(y == 0)
-  fc <- Matrix::rowMeans(X[, y == 1, drop = FALSE]) - Matrix::rowMeans(X[, y == 0, drop = FALSE])
-  B <- 1 * (G != 0)
-  sumG <- Matrix::colSums(B)
+## the "one" and "two" tests of plaid.test from crossprod(G != 0, [fc, fc^2]) = [s1, q1] (R/plaid.R:476-520)
+.set_tests <- function(tests, s1, q1, sumG, ngenes, fc) {
   pv <- list(); ff <- list()
-  if (any(c("one", "two") %in% tests)) {
-    sq <- chunked_crossprod(B, cbind(fc, fc^2))           # GPU: t(G != 0) %*% [F, F^2]
-    s1 <- sq[, 1]; q1 <- sq[, 2]
-  }
   if ("one" %in% tests) {
     mx <- s1 / (1e-8 + sumG)
     sdx <- sqrt((q1 - mx^2 * sumG) / (sumG - 1))
@@ -167,7 +152,7 @@ plaid.test <- function(X, y, G, gsetX, tests = c("one", "two", "lm"),
     pv$one <- 2 * stats::pt(abs(tt), df = pmax(sumG - 1, 1), lower.tail = FALSE); ff$one <- mx
   }
   if ("two" %in% tests) {
-    sum0 <- nrow(B) - sumG
+    sum0 <- ngenes - sumG
     mean1 <- s1 / (1e-8 + sumG); mean0 <- (sum(fc) - s1) / (1e-8 + sum0)
     var0 <- ((sum(fc^2) - q1) - mean0^2 * sum0) / (sum0 - 1)
     var1 <- (q1 - mean1^2 * sumG) / (sumG - 1)
@@ -176,20 +161,20 @@ plaid.test <- function(X, y, G, gsetX, tests = c("one", "two", "lm"),
     pv$two <- 2 * stats::pt(abs((mean1 - mean0) / sqrt(vs)), df = pmax(dof, 1), lower.tail = FALSE)
     ff$two <- mean1 - mean0
   }
-  if ("lm" %in% tests) {
-    if (missing(gsetX) || is.null(gsetX)) {
-      ## the S x N score matrix is never materialised for the host: plaid() and the group sums run as one device call
-      message("[plaid.test] computing plaid scores...")
-      gm <- .score(X, G, list(scorer = 0L, stats_mean = 1L, normalize = 1L), y = y)
-    } else {
-      gm <- .Call(C_plaidgpu_group_moments, .ctx(), as.matrix(gsetX), as.integer(y))
-    }
-    m0 <- gm[, 1] / n0; m1 <- gm[, 3] / n1
-    v0 <- (gm[, 2] - n0 * m0^2) / (n0 - 1); v1 <- (gm[, 4] - n1 * m1^2) / (n1 - 1)
-    fac <- v0 / n0 + v1 / n1
-    dof <- fac^2 / ((v0 / n0)^2 / (n0 - 1) + (v1 / n1)^2 / (n1 - 1))
-    pv$lm <- 2 * stats::pt(abs((m0 - m1) / sqrt(fac)), df = dof, lower.tail = FALSE); ff$lm <- m1 - m0
-  }
+  list(pv = pv, ff = ff)
+}
+
+## Rfast::ttests(t(gsetX), ina = y + 1) (R/plaid.R:429-431) from the group sums / sums of squares: group 1 vs group 0
+.lm_test <- function(s0, q0, n0, s1, q1, n1) {
+  m0 <- s0 / n0; m1 <- s1 / n1
+  v0 <- (q0 - n0 * m0^2) / (n0 - 1); v1 <- (q1 - n1 * m1^2) / (n1 - 1)
+  fac <- v0 / n0 + v1 / n1
+  dof <- fac^2 / ((v0 / n0)^2 / (n0 - 1) + (v1 / n1)^2 / (n1 - 1))
+  list(p = 2 * stats::pt(abs((m0 - m1) / sqrt(fac)), df = dof, lower.tail = FALSE), f = m1 - m0)
+}
+
+## p-value clamp, meta p-value, FDR and the sorted result table of plaid.test (R/plaid.R:440-474)
+.test_table <- function(pv, ff, G, metap.method, sort.by) {
   pv <- lapply(pv, function(p) { p[is.na(p)] <- 1; pmin(pmax(p, 1e-99), 1 - 1e-99) })
   gsetFC <- rowMeans(do.call(cbind, ff))
   if (length(pv) > 1) {
@@ -203,6 +188,94 @@ plaid.test <- function(X, y, G, gsetX, tests = c("one", "two", "lm"),
   res <- cbind(gsetFC = gsetFC, P, p.meta = pmeta, q.meta = stats::p.adjust(pmeta, method = "fdr"))
   rownames(res) <- colnames(G)
   if (sort.by %in% colnames(res)) res <- res[order(res[, sort.by]), ]
+  res
+}
+
+## plaid.test (R/plaid.R:392-474): same arguments and result table; the score matrix, the set-wise sums of
+## logFC / logFC^2 and the per-set group moments come from the GPU, pt / pchisq / p.adjust stay in R.
+plaid.test <- function(X, y, G, gsetX, tests = c("one", "two", "lm"),
+                       metap.method = "fisher", sort.by = "p.meta") {
+  if (!all(unique(y) %in% c(0, 1))) stop("elements of y must be 0 or 1")
+  if (is.list(G)) G <- gmt2mat(G)                                      # R/plaid.R: a GMT list is converted first
+  gg <- intersect(rownames(G), rownames(X))
+  X <- X[gg, , drop = FALSE]
+  G <- G[gg, , drop = FALSE]
+  n1 <- sum(y == 1); n0 <- sum(y == 0)
+  fc <- Matrix::rowMeans(X[, y == 1, drop = FALSE]) - Matrix::rowMeans(X[, y == 0, drop = FALSE])
+  B <- 1 * (G != 0)
+  pv <- list(); ff <- list()
+  if (any(c("one", "two") %in% tests)) {
+    sq <- chunked_crossprod(B, cbind(fc, fc^2))           # GPU: t(G != 0) %*% [F, F^2]
+    r <- .set_tests(tests, sq[, 1], sq[, 2], Matrix::colSums(B), nrow(B), fc)
+    pv <- r$pv; ff <- r$ff
+  }
+  if ("lm" %in% tests) {
+    lab <- as.integer(y != 0)  # groups 0 / 1: columns sum0, sumsq0, sum1, sumsq1
+    if (missing(gsetX) || is.null(gsetX)) {
+      ## the S x N score matrix is never materialised for the host: plaid() and the group sums run as one device call
+      message("[plaid.test] computing plaid scores...")
+      gm <- .score(X, G, list(scorer = 0L, stats_mean = 1L, normalize = 1L), labels = lab, K = 2L)
+    } else {
+      gm <- .Call(C_plaidgpu_group_stats, .ctx(), as.matrix(gsetX), lab, 2L)
+    }
+    r <- .lm_test(gm[, 1], gm[, 2], n0, gm[, 3], gm[, 4], n1)
+    pv$lm <- r$p; ff$lm <- r$f
+  }
+  .test_table(pv, ff, G, metap.method, sort.by)
+}
+
+## plaid.test for every sample group against all other labelled cells, from ONE scoring pass: a named list with one
+## result per level of factor(groups), each what plaid.test(X[, keep], groups[keep] == level, G, gsetX[, keep])
+## returns (keep = !is.na(groups)).  The per-group gene means are one sparse product on the host; the scores, their
+## per-group moments and crossprod(G != 0, [F_1..F_K, F_1^2..F_K^2]) run on the GPU (options(plaid.gpus) applies).
+plaid.test.groups <- function(X, groups, G, gsetX, tests = c("one", "two", "lm"),
+                              metap.method = "fisher", sort.by = "p.meta") {
+  if (length(groups) != ncol(X)) stop("length(groups) must equal ncol(X)")
+  keep <- !is.na(groups)
+  f <- factor(groups[keep])
+  lev <- levels(f); K <- length(lev)
+  if (K == 0) stop("no cell has a group label")
+  lab <- as.integer(f) - 1L
+  if (is.list(G)) G <- gmt2mat(G)
+  gg <- intersect(rownames(G), rownames(X))
+  X <- X[gg, keep, drop = FALSE]
+  G <- G[gg, , drop = FALSE]
+  n <- length(lab); nk <- tabulate(lab + 1L, K)
+  B <- 1 * (G != 0)
+  if (any(c("one", "two") %in% tests)) {
+    onehot <- Matrix::sparseMatrix(i = seq_len(n), j = lab + 1L, x = 1, dims = c(n, K))
+    gsum <- as.matrix(X %*% onehot)
+    tot <- Matrix::rowSums(X)
+    Fk <- sweep(gsum, 2, nk, "/") - sweep(tot - gsum, 2, n - nk, "/")   # mean(group) - mean(other labelled cells)
+    alone <- nk == n                                                   # no other cell: every statistic is NA
+    Fz <- Fk; Fz[, alone] <- 0
+    sq <- chunked_crossprod(B, cbind(Fz, Fz^2))
+    sq[, c(alone, alone)] <- NA
+  }
+  if ("lm" %in% tests) {
+    if (missing(gsetX) || is.null(gsetX)) {
+      message("[plaid.test] computing plaid scores...")
+      gm <- .score(X, G, list(scorer = 0L, stats_mean = 1L, normalize = 1L), labels = lab, K = K)
+    } else {
+      labs <- rep(-1L, length(groups)); labs[keep] <- lab
+      gm <- .Call(C_plaidgpu_group_stats, .ctx(), as.matrix(gsetX), labs, as.integer(K))
+    }
+    s_all <- rowSums(gm[, 2L * seq_len(K) - 1L, drop = FALSE]); q_all <- rowSums(gm[, 2L * seq_len(K), drop = FALSE])
+  }
+  res <- lapply(seq_len(K), function(k) {
+    pv <- list(); ff <- list()
+    if (any(c("one", "two") %in% tests)) {
+      r <- .set_tests(tests, sq[, k], sq[, K + k], Matrix::colSums(B), nrow(B), Fk[, k])
+      pv <- r$pv; ff <- r$ff
+    }
+    if ("lm" %in% tests) {
+      s1 <- gm[, 2L * k - 1L]; q1 <- gm[, 2L * k]
+      r <- .lm_test(s_all - s1, q_all - q1, n - nk[k], s1, q1, nk[k])
+      pv$lm <- r$p; ff$lm <- r$f
+    }
+    .test_table(pv, ff, G, metap.method, sort.by)
+  })
+  names(res) <- lev
   res
 }
 

@@ -10,6 +10,7 @@
 #include <R.h>
 #include <Rinternals.h>
 #include <R_ext/Rdynload.h>
+#include <limits.h>
 #include <string.h>
 
 #include "plaidgpu.h"
@@ -175,40 +176,56 @@ SEXP C_plaidgpu_colranks(SEXP ctx, SEXP kind, SEXP Xp, SEXP Xi, SEXP Xx, SEXP Xd
   return out;
 }
 
-/* per-set sums / sums of squares of gsetX by group y (plaid.test "lm"): 4 x S matrix */
-SEXP C_plaidgpu_group_moments(SEXP ctx, SEXP x, SEXP y) {
+/* per-set sums / sums of squares of gsetX by group (plaid.test "lm"): labels in [-1, K), -1 = no group.  An S x 2K
+ * matrix: columns 2k + 1, 2k + 2 (1-based) hold sum_k, sumsq_k */
+SEXP C_plaidgpu_group_stats(SEXP ctx, SEXP x, SEXP labels, SEXP K) {
   plaidgpu_ctx* c = get_ctx(ctx);
   SEXP dim = Rf_getAttrib(x, R_DimSymbol);
-  const int S = INTEGER(dim)[0], N = INTEGER(dim)[1];
-  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, S, 4)); /* columns: sum0, sumsq0, sum1, sumsq1 */
-  int rc = plaidgpu_group_moments(c, REAL(x), S, N, INTEGER(y), PLAIDGPU_HOST, REAL(out));
+  const int S = INTEGER(dim)[0], N = INTEGER(dim)[1], k = Rf_asInteger(K);
+  if (XLENGTH(labels) != N) Rf_error("plaidgpu: length(labels) must equal ncol(x)");
+  if (k < 1 || k > INT_MAX / 2) Rf_error("plaidgpu: K must be at least 1");
+  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, S, 2 * k));
+  int rc = plaidgpu_group_stats(c, REAL(x), S, N, INTEGER(labels), k, PLAIDGPU_HOST, REAL(out));
   if (rc != PLAIDGPU_OK) {
     UNPROTECT(1);
-    Rf_error("plaidgpu_group_moments: %s", plaidgpu_last_error(c));
+    Rf_error("plaidgpu_group_stats: %s", plaidgpu_last_error(c));
   }
   UNPROTECT(1);
   return out;
 }
 
-/* plaid.test(tests = "lm") without gsetX (R/plaid.R:423-431): plaid() fused with the per-set group reductions —
- * the S x N scores stay on the device, an S x 4 matrix (sum0, sumsq0, sum1, sumsq1) comes back */
-SEXP C_plaidgpu_score_group_moments(SEXP ctx, SEXP kind, SEXP Xp, SEXP Xi, SEXP Xx, SEXP Xdim, SEXP Gp, SEXP Gi, SEXP Gx,
-                                    SEXP Gdim, SEXP rowmap, SEXP opts, SEXP y) {
-  plaidgpu_ctx* c = get_ctx(TYPEOF(ctx) == VECSXP ? VECTOR_ELT(ctx, 0) : ctx);
-  const int PG = INTEGER(Gdim)[0], S = INTEGER(Gdim)[1];
-  if (plaidgpu_set_genesets(c, PG, S, INTEGER(Gp), INTEGER(Gi), REAL(Gx)) != PLAIDGPU_OK)
-    Rf_error("plaidgpu_set_genesets: %s", plaidgpu_last_error(c));
+/* plaid.test(tests = "lm") without gsetX (R/plaid.R:423-431), for K sample groups: plaid() fused with the per-set group
+ * reductions — the S x N scores stay on the device, an S x 2K matrix (sum_k, sumsq_k per group) comes back.  A list of
+ * contexts (options(plaid.gpus = n)) splits the columns over the devices (plaidgpu_score_group_stats_multi). */
+SEXP C_plaidgpu_score_group_stats(SEXP ctx, SEXP kind, SEXP Xp, SEXP Xi, SEXP Xx, SEXP Xdim, SEXP Gp, SEXP Gi, SEXP Gx,
+                                  SEXP Gdim, SEXP rowmap, SEXP opts, SEXP labels, SEXP K) {
+  plaidgpu_ctx* cs[16];
+  int nctx = 1;
+  if (TYPEOF(ctx) == VECSXP) {
+    nctx = (int)XLENGTH(ctx);
+    if (nctx < 1 || nctx > 16) Rf_error("plaidgpu: between 1 and 16 contexts expected");
+    for (int j = 0; j < nctx; ++j) cs[j] = get_ctx(VECTOR_ELT(ctx, j));
+  } else {
+    cs[0] = get_ctx(ctx);
+  }
+  plaidgpu_ctx* c = cs[0];
+  const int PG = INTEGER(Gdim)[0], S = INTEGER(Gdim)[1], k = Rf_asInteger(K);
+  for (int j = 0; j < nctx; ++j)
+    if (plaidgpu_set_genesets(cs[j], PG, S, INTEGER(Gp), INTEGER(Gi), REAL(Gx)) != PLAIDGPU_OK)
+      Rf_error("plaidgpu_set_genesets: %s", plaidgpu_last_error(cs[j]));
   plaidgpu_matrix M;
   fill_matrix(&M, Rf_asInteger(kind), Xp, Xi, Xx, Xdim);
-  if ((int64_t)XLENGTH(y) != M.N) Rf_error("plaidgpu: length(y) must equal ncol(X)");
+  if ((int64_t)XLENGTH(labels) != M.N) Rf_error("plaidgpu: length(labels) must equal ncol(X)");
+  if (k < 1 || k > INT_MAX / 2) Rf_error("plaidgpu: K must be at least 1");
   plaidgpu_opts o;
   fill_opts(&o, opts);
   R_CheckUserInterrupt();
-  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, S, 4));
-  int rc = plaidgpu_score_group_moments(c, &M, INTEGER(rowmap), &o, INTEGER(y), REAL(out));
+  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, S, 2 * k));
+  int rc = nctx > 1 ? plaidgpu_score_group_stats_multi(cs, nctx, &M, INTEGER(rowmap), &o, INTEGER(labels), k, REAL(out))
+                    : plaidgpu_score_group_stats(c, &M, INTEGER(rowmap), &o, INTEGER(labels), k, REAL(out));
   if (rc != PLAIDGPU_OK) {
     UNPROTECT(1);
-    Rf_error("plaidgpu_score_group_moments: %s", plaidgpu_last_error(c));
+    Rf_error("plaidgpu_score_group_stats: %s", plaidgpu_last_error(c));
   }
   UNPROTECT(1);
   return out;
@@ -219,8 +236,8 @@ static const R_CallMethodDef call_methods[] = {
     {"C_plaidgpu_score", (DL_FUNC)&C_plaidgpu_score, 12},
     {"C_plaidgpu_normalize_medians", (DL_FUNC)&C_plaidgpu_normalize_medians, 3},
     {"C_plaidgpu_colranks", (DL_FUNC)&C_plaidgpu_colranks, 9},
-    {"C_plaidgpu_group_moments", (DL_FUNC)&C_plaidgpu_group_moments, 3},
-    {"C_plaidgpu_score_group_moments", (DL_FUNC)&C_plaidgpu_score_group_moments, 13},
+    {"C_plaidgpu_group_stats", (DL_FUNC)&C_plaidgpu_group_stats, 4},
+    {"C_plaidgpu_score_group_stats", (DL_FUNC)&C_plaidgpu_score_group_stats, 14},
     {"C_plaidgpu_crossprod", (DL_FUNC)&C_plaidgpu_crossprod, 11},
     {NULL, NULL, 0}};
 
