@@ -299,6 +299,28 @@ int plaidgpu_score_group_stats(plaidgpu_ctx* ctx, const plaidgpu_matrix* X, cons
 int plaidgpu_score_group_stats_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
                                      const plaidgpu_opts* opts, const int32_t* labels, int K, double* out);
 
+/* Per column of a dense S x N matrix at `location`: the k largest (decreasing = 1) or smallest values and their row
+ * indices, i.e. the first k entries of R's order(v, decreasing = decreasing): ties (fp64 ==, so -0 == +0) by
+ * ascending row, NaN last in both directions and by ascending row.  idx int32[k * N] (0-based rows) and val
+ * double[k * N] (val = v[idx] bit for bit), host, column-major: entry t of column j at t + k * j.
+ * 1 <= k <= min(S, 256), otherwise PLAIDGPU_ERR_ARG; N = 0 does nothing.  Kernel time: plaidgpu_last_kernel_ms(, 2). */
+int plaidgpu_col_topk(plaidgpu_ctx* ctx, const double* x, int32_t S, int64_t N, int k, int decreasing,
+                      int location, int32_t* idx, double* val);
+
+/* The same fused onto the scoring call, for any scorer and option plaidgpu_score accepts: the scores stay on the
+ * device as raw scores and are normalised in registers while selecting; k * N indices and values come back.  Equal,
+ * bit for bit, to plaidgpu_score followed by plaidgpu_col_topk.  When X is in host memory and the S x N scores exceed
+ * the device, the columns are scored in tiles (two passes over X when normalised, like plaidgpu_score), each tile
+ * writing its own columns of idx / val. */
+int plaidgpu_score_topk(plaidgpu_ctx* ctx, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
+                        int k, int decreasing, int32_t* idx, double* val);
+
+/* plaidgpu_score_topk over n devices from ONE host process, split like plaidgpu_score_multi: shard r writes columns
+ * [lo_r, hi_r) of idx / val, and nothing is combined.  Each shard's scores must fit its device.  The same context
+ * twice, or gsva rowtf = "ecdf" with n > 1, is PLAIDGPU_ERR_ARG. */
+int plaidgpu_score_topk_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
+                              const plaidgpu_opts* opts, int k, int decreasing, int32_t* idx, double* val);
+
 /* ---- gene-set ingestion ("next" row f2): host-side, no GPU needed -------------------------- */
 
 /* read.gmt() + gmt2mat() with default arguments (reference R/gmt-utils.R:99-125, 19-66): a GMT text

@@ -63,6 +63,8 @@ SYMBOLS = {
     "plaidgpu_colranks": (C.c_int, [C.c_void_p, C.POINTER(Matrix), C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "plaidgpu_group_moments": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_int, C.c_void_p]),
     "plaidgpu_group_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "plaidgpu_col_topk": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                    C.c_void_p]),
     "plaidgpu_normalize_medians": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
     "plaidgpu_gmt_read": (C.c_int, [C.c_char_p, C.POINTER(C.c_void_p)]),
     "plaidgpu_gmt_from_buffer": (C.c_int, [C.c_char_p, C.c_int64, C.POINTER(C.c_void_p)]),
@@ -97,6 +99,10 @@ SYMBOLS = {
     "plaidgpu_score_group_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "plaidgpu_score_group_stats_multi": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                                    C.c_void_p, C.c_int, C.c_void_p]),
+    "plaidgpu_score_topk": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                       C.c_void_p]),
+    "plaidgpu_score_topk_multi": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                             C.c_int, C.c_void_p, C.c_void_p]),
     "plaidgpu_score_multi": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "plaidgpu_tc_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "plaidgpu_tail_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),

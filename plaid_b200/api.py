@@ -544,6 +544,71 @@ def score_group_stats(X: NamedMatrix, matG: NamedMatrix, labels, K=None, *, ctx=
     return out
 
 
+def col_topk(gsetX, k=10, decreasing=True, *, ctx=None):
+    """Per column of a dense S x N matrix: the first k entries of R's `order(v, decreasing = decreasing)`, i.e. the
+    k largest (or smallest) values with ties by ascending row and NaN last (`plaidgpu_col_topk`).  `gsetX` is a 2-D
+    array or a `DeviceDense` (S x N in device memory).  Returns (idx, val) of shape (k, N): 0-based row indices
+    (int32) and the values at those rows, bit for bit."""
+    ctx = ctx or default_context()
+    if isinstance(gsetX, DeviceDense):
+        S, N = (int(d) for d in gsetX.shape)
+        if gsetX.x.numel() != S * N:
+            raise ValueError("DeviceDense: the tensor does not hold shape[0] * shape[1] values")
+        loc, ptr = L.DEVICE, gsetX.x.data_ptr()
+    else:
+        if _is_torch(gsetX):
+            raise TypeError("pass dense device matrices as DeviceDense(t_colmajor, shape)")
+        a = np.asarray(gsetX, dtype=np.float64)
+        if a.ndim != 2:
+            raise ValueError("gsetX must be a matrix (S x N)")
+        a = np.asfortranarray(a)
+        S, N = a.shape
+        loc, ptr = L.HOST, a.ctypes.data
+    idx = np.empty((max(int(k), 0), N), dtype=np.int32, order="F")  # a bad k is the library's error
+    val = np.empty((max(int(k), 0), N), dtype=np.float64, order="F")
+    ctx.check(ctx.lib.plaidgpu_col_topk(ctx.h, ptr, S, N, int(k), 1 if decreasing else 0, loc, idx.ctypes.data,
+                                        val.ctypes.data))
+    return idx, val
+
+
+def score_topk(X: NamedMatrix, matG: NamedMatrix, k=10, decreasing=True, *, ctx=None, **opts_kw):
+    """plaid() (or another scorer through `opts_kw`) fused with col_topk (`plaidgpu_score_topk`): each cell's k
+    best gene sets, while the S x N scores stay on the device.  Equal, bit for bit, to scoring followed by col_topk.
+    `ctx` may be a list of Contexts on different devices: the columns are then split over them
+    (`plaidgpu_score_topk_multi`).  Returns (idx, val) of shape (k, N), or None on no overlap."""
+    ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else None
+    ctx = (ctxs[0] if ctxs else ctx) or default_context()
+    if X.rownames is None or matG.rownames is None:
+        _message("[plaid] ERROR. No overlapping features.")
+        return None
+    rowmap = make_rowmap(X.rownames, matG.rownames)
+    if not (rowmap >= 0).any():
+        _message("[plaid] ERROR. No overlapping features.")
+        return None
+    for cx in (ctxs or [ctx]):
+        cx.set_genesets(matG.mat)
+    keep: list = []
+    M = _matrix_struct(X.mat, keep)
+    kw = dict(scorer=L.PLAID, stats_mean=1, normalize=1)
+    kw.update(opts_kw)
+    o = _opts(ctx.lib, **kw)
+    idx = np.empty((max(int(k), 0), M.N), dtype=np.int32, order="F")
+    val = np.empty((max(int(k), 0), M.N), dtype=np.float64, order="F")
+    dec = 1 if decreasing else 0
+    if ctxs and len(ctxs) > 1:
+        hs = (C.c_void_p * len(ctxs))(*[cx.h for cx in ctxs])
+        rc = ctx.lib.plaidgpu_score_topk_multi(hs, len(ctxs), C.byref(M), rowmap.ctypes.data, C.byref(o), int(k), dec,
+                                               idx.ctypes.data, val.ctypes.data)
+    else:
+        rc = ctx.lib.plaidgpu_score_topk(ctx.h, C.byref(M), rowmap.ctypes.data, C.byref(o), int(k), dec,
+                                         idx.ctypes.data, val.ctypes.data)
+    if rc == L.ERR_NOOVERLAP:
+        _message("[plaid] ERROR. No overlapping features.")
+        return None
+    ctx.check(rc)
+    return idx, val
+
+
 def _align(X: NamedMatrix, G: NamedMatrix):
     """intersect(rownames(G), rownames(X)) and X[gg, ], G[gg, ] (R/plaid.R:402-404)"""
     xset = set(X.rownames)

@@ -210,6 +210,10 @@ struct plaidgpu_ctx {
   const int32_t* mom_labels = nullptr;
   int mom_K = 0;
   double* mom_out = nullptr;
+  // plaidgpu_score_topk: finish selects each column's top k of the (fixed-up on the fly) scores instead (host idx / val)
+  int topk_k = 0, topk_dec = 1;
+  int32_t* topk_idx = nullptr;
+  double* topk_val = nullptr;
   // mailbox: pinned, device-mapped host memory the GPU writes small results into (launch_copy_words)
   void* mbox = nullptr;
   void* mbox_dev = nullptr;
@@ -1009,6 +1013,38 @@ int group_stats_device(plaidgpu_ctx* c, const double* dx, int32_t S, int64_t N, 
   return PLAIDGPU_OK;
 }
 
+// ---- per-column top k (plaid.topsets) -------------------------------------------------------
+int check_topk(plaidgpu_ctx* c, int32_t S, int k) {
+  if (k < 1 || k > TOPK_MAX || k > S)
+    return fail(c, PLAIDGPU_ERR_ARG, "k = " + std::to_string(k) + " is outside [1, min(S = " + std::to_string(S) +
+                                         ", " + std::to_string(TOPK_MAX) + ")]");
+  return PLAIDGPU_OK;
+}
+
+// Each column's top k of the S x N device matrix dx (ld = S) into host idx / val[k * N] (checked k).  Kernel time in
+// ms[2].  fix / med / cc / alpha / beta: the fix-up of plaidgpu_score_finish, applied in registers to raw scores.
+int topk_device(plaidgpu_ctx* c, const double* dx, int32_t S, int64_t N, int k, int decreasing, int32_t* idx,
+                double* val, bool fix = false, const double* med = nullptr, double cc = 0.0, double alpha = 1.0,
+                const double* beta = nullptr) {
+  const size_t n = (size_t)k * (size_t)N;
+  CK(c->b_i32.reserve(std::max<size_t>(n, 1) * sizeof(int32_t)));
+  CK(c->b_rowb.reserve(std::max<size_t>(n, 1) * sizeof(double)));
+  CK(cudaEventRecord(c->ev[4], c->stream));
+  CK(launch_col_topk(dx, S, S, N, k, decreasing, c->b_i32.as<int32_t>(), c->b_rowb.as<double>(), c->stream, fix, med,
+                     cc, alpha, beta));
+  c->launches += 1;
+  CK(cudaEventRecord(c->ev[5], c->stream));
+  if (n) {
+    CK(cudaMemcpyAsync(idx, c->b_i32.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(val, c->b_rowb.p, n * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  }
+  CK(cudaStreamSynchronize(c->stream));
+  float ms = 0.f;
+  cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]);
+  c->ms[2] = ms;
+  return PLAIDGPU_OK;
+}
+
 // Host X and host output larger than the device can hold: the column tile width score_chunked should use, or 0
 // when one pass fits (the raw scores get 45 % of the free memory; X, ranks and slack share the rest)
 int host_chunk_cols(plaidgpu_ctx* c, const plaidgpu_matrix* X, int64_t* chunk) {
@@ -1758,7 +1794,7 @@ int plaidgpu_combine_medians(int ignore_zero_opt, double score_min, const double
 
 int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double* out) try {
   if (!c) return PLAIDGPU_ERR_ARG;
-  if (!scal || (!out && c->N > 0 && !c->mom_labels)) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  if (!scal || (!out && c->N > 0 && !c->mom_labels && !c->topk_idx)) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
   if (!c->computed) return fail(c, PLAIDGPU_ERR_STATE, "plaidgpu_score_compute has not been called");
   CK(cudaSetDevice(c->device));
   const plaidgpu_opts& o = c->opts;
@@ -1797,6 +1833,15 @@ int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double*
     c->mom_labels = nullptr;
     c->mom_out = nullptr;
     return group_stats_device(c, c->raw, S, N, lab, K, mo, fix, med, cc, alpha, beta);
+  }
+  if (c->topk_idx) {
+    // score -> top sets: each column's k first sets of the normalised scores, the fix-up applied in registers; the
+    // S x N matrix stays on the device as raw scores and k * N indices and values go back
+    int32_t* ti = c->topk_idx;
+    double* tv = c->topk_val;
+    c->topk_idx = nullptr;
+    c->topk_val = nullptr;
+    return topk_device(c, c->raw, S, N, c->topk_k, c->topk_dec, ti, tv, fix, med, cc, alpha, beta);
   }
   c->raw_valid = false;  // the fix-up below rewrites the raw scores in place
   CK(cudaEventRecord(c->ev[4], c->stream));
@@ -1941,19 +1986,45 @@ int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double*
 // scores over PCIe twice).  Results are bit-identical to the un-chunked path.
 // `sink` (optional): instead of landing in `out`, every finished chunk is staged in a pinned buffer and
 // written to the file — tiled egress for results larger than host memory (scope row f4).
-// `groups` (optional): every finished chunk is reduced per set and sample group on the device instead
-// (plaidgpu_score_group_stats), into groups->tile, and `out` (K * 2 * S doubles, zeroed by the caller)
-// accumulates the tiles in tile order.
-struct GroupSink {
-  const int32_t* labels;  // int32[N] of the whole call
+// `reduce` (optional): every finished chunk is reduced on the device instead (finish_into): per set and sample
+// group (plaidgpu_score_group_stats), with `out` (K * 2 * S doubles, zeroed by the caller) accumulating the tiles'
+// moments in tile order, or to each column's top k (plaidgpu_score_topk), the tile of columns [j0, j1) writing
+// idx / val + j0 * k.
+struct ScoreSink {
+  const int32_t* labels;  // group statistics: int32[N] of the whole call, or nullptr for top k
   int K;
-  double* tile;           // K * 2 * S doubles of host scratch
+  int k, decreasing;      // top k: idx / val hold k * N entries of the whole call
+  int32_t* idx;
+  double* val;
 };
+
+// plaidgpu_score_finish reducing the scores of columns [j0, ...) of the call as `sk` says instead of shipping them;
+// moments: K * 2 * S doubles for group statistics
+static int finish_into(plaidgpu_ctx* c, const plaidgpu_scalars* s, const ScoreSink& sk, int64_t j0, double* moments) {
+  if (sk.labels) {
+    c->mom_labels = sk.labels + j0;
+    c->mom_K = sk.K;
+    c->mom_out = moments;
+  } else {
+    c->topk_k = sk.k;
+    c->topk_dec = sk.decreasing;
+    c->topk_idx = sk.idx + j0 * sk.k;
+    c->topk_val = sk.val + j0 * sk.k;
+  }
+  const int rc = plaidgpu_score_finish(c, s, nullptr);
+  c->mom_labels = nullptr;
+  c->mom_out = nullptr;
+  c->topk_idx = nullptr;
+  c->topk_val = nullptr;
+  return rc;
+}
+
 static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
                          double* out, int64_t chunk, FILE* sink = nullptr, double* stage = nullptr, double* stage2 = nullptr,
-                         const GroupSink* groups = nullptr) {
+                         const ScoreSink* reduce = nullptr) {
   const int64_t N = X->N;
   const int32_t S = c->S;
+  std::vector<double> moments(reduce && reduce->labels ? (size_t)reduce->K * 2 * (size_t)S : 0);  // one tile's group moments
   if (opts->scorer == PLAIDGPU_GSVA && opts->gsva_ecdf != PLAIDGPU_ROWTF_DONE &&
       (opts->gsva_ecdf || !(opts->row_mean && opts->row_sd)))
     return fail(c, PLAIDGPU_ERR_ARG, "replaid.gsva: matrix too large for one device pass (rowtf ecdf needs all samples; rowtf z needs row_mean / row_sd)");
@@ -2041,15 +2112,10 @@ static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_
     if (rc) return rc;
     s.ignore_zero = g.ignore_zero;
     s.med_mean = g.med_mean;
-    if (groups) {
-      c->mom_labels = groups->labels + j0;
-      c->mom_K = groups->K;
-      c->mom_out = groups->tile;
-      rc = plaidgpu_score_finish(c, &s, nullptr);
-      c->mom_labels = nullptr;
-      c->mom_out = nullptr;
+    if (reduce) {
+      rc = finish_into(c, &s, *reduce, j0, moments.data());
       if (rc) return rc;
-      for (int64_t i = 0, w = (int64_t)groups->K * 2 * S; i < w; ++i) out[i] += groups->tile[i];
+      for (size_t i = 0; i < moments.size(); ++i) out[i] += moments[i];
       continue;
     }
     double* dst = sink ? ((stage2 && (tile & 1)) ? stage2 : stage) : out + j0 * (int64_t)S;
@@ -2166,23 +2232,18 @@ int plaidgpu_score(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* row
 // plaid.test(tests = "lm") (R/plaid.R:426-431) without the S x N matrix ever leaving the device or being written in
 // its normalised form.  Bit-identical to plaidgpu_score + plaidgpu_group_stats.  Host X whose S x N scores exceed
 // the device goes through score_chunked (two passes when normalised) and adds the tiles' moments in tile order.
-int plaidgpu_score_group_stats(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
-                               const int32_t* labels, int K, double* out) try {
-  if (!c) return PLAIDGPU_ERR_ARG;
-  if (!X || !rowmap || !opts || !out) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
-  int rc = check_groups(c, labels, X->N, K);
-  if (rc) return rc;
+// plaidgpu_score's pipeline with a finish step that reduces on the device (finish_into); `out`: the K * 2 * S moments
+// of group statistics.  Host X whose S x N scores exceed the device goes through score_chunked.
+static int score_reduce(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
+                        const ScoreSink& sk, double* out) {
   plaidgpu_opts o = *opts;
   o.out_location = PLAIDGPU_HOST;  // raw scores in the library's device buffer
   int64_t chunk = 0;
-  rc = host_chunk_cols(c, X, &chunk);
+  int rc = host_chunk_cols(c, X, &chunk);
   if (rc) return rc;
   if (chunk > 0) {
-    const size_t width = (size_t)K * 2 * (size_t)c->S;
-    std::vector<double> tile(width);
-    std::fill(out, out + width, 0.0);
-    const GroupSink gs{labels, K, tile.data()};
-    return score_chunked(c, X, rowmap, &o, out, chunk, nullptr, nullptr, nullptr, &gs);
+    if (sk.labels) std::fill(out, out + (size_t)sk.K * 2 * (size_t)c->S, 0.0);
+    return score_chunked(c, X, rowmap, &o, out, chunk, nullptr, nullptr, nullptr, &sk);
   }
   plaidgpu_scalars s;
   rc = plaidgpu_score_begin(c, X, rowmap, &o, &s);
@@ -2197,13 +2258,37 @@ int plaidgpu_score_group_stats(plaidgpu_ctx* c, const plaidgpu_matrix* X, const 
     rc = plaidgpu_combine_medians(o.ignore_zero, s.score_min, m, m, c->N, &s);
     if (rc) return fail(c, rc, "combine_medians failed");
   }
-  c->mom_labels = labels;
-  c->mom_K = K;
-  c->mom_out = out;
-  rc = plaidgpu_score_finish(c, &s, nullptr);
-  c->mom_labels = nullptr;
-  c->mom_out = nullptr;
-  return rc;
+  return finish_into(c, &s, sk, 0, out);
+}
+
+int plaidgpu_score_group_stats(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
+                               const int32_t* labels, int K, double* out) try {
+  if (!c) return PLAIDGPU_ERR_ARG;
+  if (!X || !rowmap || !opts || !out) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  int rc = check_groups(c, labels, X->N, K);
+  if (rc) return rc;
+  const ScoreSink sk{labels, K, 0, 0, nullptr, nullptr};
+  return score_reduce(c, X, rowmap, opts, sk, out);
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
+// score -> top sets fused: plaid() / a replaid.* scorer followed by each column's top k (plaid.topsets) without the
+// S x N matrix leaving the device or being written in its normalised form.  Bit-identical to plaidgpu_score +
+// plaidgpu_col_topk.  Host X whose S x N scores exceed the device is scored in column tiles, each writing its own
+// columns of idx / val.
+int plaidgpu_score_topk(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
+                        int k, int decreasing, int32_t* idx, double* val) try {
+  if (!c) return PLAIDGPU_ERR_ARG;
+  if (!X || !rowmap || !opts || !idx || !val) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  if (!c->have_g) return fail(c, PLAIDGPU_ERR_STATE, "plaidgpu_set_genesets has not been called");
+  int rc = check_topk(c, c->S, k);
+  if (rc) return rc;
+  if (X->N == 0) return PLAIDGPU_OK;
+  const ScoreSink sk{nullptr, 0, k, decreasing != 0, idx, val};
+  return score_reduce(c, X, rowmap, opts, sk, nullptr);
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {
@@ -2249,13 +2334,10 @@ struct ShardBarrier {
 };
 }  // namespace
 
-// labels == nullptr: the S x N scores land in `out` (plaidgpu_score_multi).  Otherwise every shard reduces its scores
-// per set and group on its device (plaidgpu_score_group_stats) and `out` (K * 2 * S doubles) receives the shards'
-// moments added in shard order (plaidgpu_score_group_stats_multi).
-static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
-                            const plaidgpu_opts* opts, double* out, const int32_t* labels, int K, const char* name) {
+// the contexts of a multi-device call: distinct, each holding the same gene sets, and no scorer that ranks across
+// samples
+static int check_shard_ctxs(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_opts* opts, const std::string& who) {
   plaidgpu_ctx* c = ctxs[0];
-  const std::string who(name);
   for (int r = 0; r < n; ++r) {
     if (!ctxs[r] || !ctxs[r]->have_g) return fail(c, PLAIDGPU_ERR_STATE, who + ": every context needs plaidgpu_set_genesets");
     if (ctxs[r]->S != c->S) return fail(c, PLAIDGPU_ERR_ARG, who + ": contexts hold different gene sets");
@@ -2264,6 +2346,22 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
   }
   if (opts->scorer == PLAIDGPU_GSVA && opts->gsva_ecdf == PLAIDGPU_ROWTF_ECDF)
     return fail(c, PLAIDGPU_ERR_ARG, who + ": gsva rowtf = ecdf ranks across samples (use one context, or the row exchange of plaid_b200/sharded.py)");
+  return PLAIDGPU_OK;
+}
+
+// reduce == nullptr: the S x N scores land in `out` (plaidgpu_score_multi).  Otherwise every shard reduces its scores
+// on its device (finish_into): per set and group, `out` (K * 2 * S doubles) receiving the shards' moments added in
+// shard order (plaidgpu_score_group_stats_multi), or to each column's top k, shard r writing columns [lo_r, hi_r) of
+// idx / val (plaidgpu_score_topk_multi).
+static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
+                            const plaidgpu_opts* opts, double* out, const ScoreSink* reduce, const char* name) {
+  plaidgpu_ctx* c = ctxs[0];
+  const std::string who(name);
+  {
+    const int rcc = check_shard_ctxs(ctxs, n, opts, who);
+    if (rcc) return rcc;
+  }
+  const int32_t* labels = reduce ? reduce->labels : nullptr;
   try {
     const int64_t N = X->N;
     const int32_t S = c->S, P = X->P;
@@ -2289,7 +2387,7 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
     }
     std::vector<plaidgpu_scalars> loc((size_t)n);
     std::vector<int> rc((size_t)n, PLAIDGPU_OK);
-    const size_t width = labels ? (size_t)K * 2 * (size_t)S : 0;
+    const size_t width = labels ? (size_t)reduce->K * 2 * (size_t)S : 0;
     std::vector<std::vector<double>> moments(labels ? (size_t)n : 0, std::vector<double>(width));
     std::vector<double> med((size_t)std::max<int64_t>(N, 1));
     std::vector<std::vector<double>> part(gsva_z ? (size_t)n : 0, std::vector<double>((size_t)P));
@@ -2305,8 +2403,8 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
     auto body = [&](int r) {
       plaidgpu_ctx* cr = ctxs[r];
       plaidgpu_opts o = *opts;
-      if (labels) o.out_location = PLAIDGPU_HOST;  // raw scores stay in the context's device buffer
-      double* dst = labels ? nullptr : out + lo[r] * (int64_t)S;
+      if (reduce) o.out_location = PLAIDGPU_HOST;  // raw scores stay in the context's device buffer
+      double* dst = reduce ? nullptr : out + lo[r] * (int64_t)S;
       if (gsva_z) {  // rowMeans / rowSds over ALL shards, summed in shard order (R/plaid.R:343)
         rc[r] = plaidgpu_row_moments(cr, &M[r], nullptr, part[r].data());
         bar.wait();
@@ -2358,14 +2456,8 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
         s.med_mean = g.med_mean;
         s.score_min = smin;
       }
-      if (labels) {
-        cr->mom_labels = labels + lo[r];
-        cr->mom_K = K;
-        cr->mom_out = moments[r].data();
-      }
-      rc[r] = plaidgpu_score_finish(cr, &s, dst);
-      cr->mom_labels = nullptr;
-      cr->mom_out = nullptr;
+      rc[r] = reduce ? finish_into(cr, &s, *reduce, lo[r], labels ? moments[r].data() : nullptr)
+                     : plaidgpu_score_finish(cr, &s, dst);
     };
     std::vector<std::thread> th;
     for (int r = 1; r < n; ++r) th.emplace_back(body, r);
@@ -2397,7 +2489,7 @@ int plaidgpu_score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix
   if (X->location != PLAIDGPU_HOST || opts->out_location != PLAIDGPU_HOST)
     return fail(c, PLAIDGPU_ERR_ARG, "plaidgpu_score_multi: X and out must be in host memory");
   if (n == 1 || X->N < 2 * (int64_t)n) return plaidgpu_score(c, X, rowmap, opts, out);
-  return score_multi_impl(ctxs, n, X, rowmap, opts, out, nullptr, 0, "plaidgpu_score_multi");
+  return score_multi_impl(ctxs, n, X, rowmap, opts, out, nullptr, "plaidgpu_score_multi");
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {
@@ -2413,7 +2505,29 @@ int plaidgpu_score_group_stats_multi(plaidgpu_ctx* const* ctxs, int n, const pla
   if (n == 1 || X->N < 2 * (int64_t)n) return plaidgpu_score_group_stats(c, X, rowmap, opts, labels, K, out);
   int rc = check_groups(c, labels, X->N, K);
   if (rc) return rc;
-  return score_multi_impl(ctxs, n, X, rowmap, opts, out, labels, K, "plaidgpu_score_group_stats_multi");
+  const ScoreSink sk{labels, K, 0, 0, nullptr, nullptr};
+  return score_multi_impl(ctxs, n, X, rowmap, opts, out, &sk, "plaidgpu_score_group_stats_multi");
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
+int plaidgpu_score_topk_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
+                              const plaidgpu_opts* opts, int k, int decreasing, int32_t* idx, double* val) try {
+  if (!ctxs || n <= 0 || !ctxs[0]) return PLAIDGPU_ERR_ARG;
+  plaidgpu_ctx* c = ctxs[0];
+  if (!X || !rowmap || !opts || !idx || !val) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  if (X->location != PLAIDGPU_HOST) return fail(c, PLAIDGPU_ERR_ARG, "plaidgpu_score_topk_multi: X must be in host memory");
+  if (n > 1) {  // also when the columns are too few to split: the same arguments fail whatever N is
+    int rc = check_shard_ctxs(ctxs, n, opts, "plaidgpu_score_topk_multi");
+    if (rc) return rc;
+  }
+  if (n == 1 || X->N < 2 * (int64_t)n) return plaidgpu_score_topk(c, X, rowmap, opts, k, decreasing, idx, val);
+  int rc = check_topk(c, c->S, k);
+  if (rc) return rc;
+  const ScoreSink sk{nullptr, 0, k, decreasing != 0, idx, val};
+  return score_multi_impl(ctxs, n, X, rowmap, opts, nullptr, &sk, "plaidgpu_score_topk_multi");
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {
@@ -2605,6 +2719,30 @@ int plaidgpu_group_moments(plaidgpu_ctx* c, const double* x, int32_t S, int64_t 
   std::vector<int32_t> lab((size_t)N);
   for (int64_t j = 0; j < N; ++j) lab[(size_t)j] = y[j] != 0;
   return plaidgpu_group_stats(c, x, S, N, lab.data(), 2, location, out);
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
+int plaidgpu_col_topk(plaidgpu_ctx* c, const double* x, int32_t S, int64_t N, int k, int decreasing, int location,
+                      int32_t* idx, double* val) try {
+  if (!c) return PLAIDGPU_ERR_ARG;
+  if (S <= 0 || N < 0) return fail(c, PLAIDGPU_ERR_ARG, "bad argument");
+  if (!idx || !val || (N > 0 && !x)) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  if (location != PLAIDGPU_HOST && location != PLAIDGPU_DEVICE) return fail(c, PLAIDGPU_ERR_ARG, "unknown location");
+  int rc = check_topk(c, S, k);
+  if (rc) return rc;
+  if (N == 0) return PLAIDGPU_OK;
+  CK(cudaSetDevice(c->device));
+  const double* dx = x;
+  if (location == PLAIDGPU_HOST) {
+    const size_t total = (size_t)S * (size_t)N;
+    CK(c->b_raw.reserve(total * sizeof(double)));
+    CK(cudaMemcpyAsync(c->b_raw.p, x, total * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    dx = c->b_raw.as<double>();
+  }
+  return topk_device(c, dx, S, N, k, decreasing != 0, idx, val);
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {

@@ -189,6 +189,13 @@ cudaError_t launch_fixup(const double* x, double* out, int64_t ld, int32_t S, in
 cudaError_t launch_group_stats(const double* x, int64_t ld, int32_t S, int K, const int32_t* cols, const int32_t* seg,
                                int nchunk, double* partial, double* out, cudaStream_t st, bool fix = false,
                                const double* med = nullptr, double c = 0.0, double alpha = 1.0, const double* beta = nullptr);
+// per column of a column-major S x N matrix: the k (1 <= k <= min(S, TOPK_MAX)) rows first in R's
+// order(v, decreasing = decreasing) (ties by ascending row, NaN last) into idx / val[k * N] (device, column-major).
+// fix: x holds RAW scores and the selection is over alpha * (x - med_j + c) + beta_s (k_fixup's arithmetic)
+constexpr int TOPK_MAX = 256;
+cudaError_t launch_col_topk(const double* x, int64_t ld, int32_t S, int64_t N, int k, int decreasing, int32_t* idx,
+                            double* val, cudaStream_t st, bool fix = false, const double* med = nullptr, double c = 0.0,
+                            double alpha = 1.0, const double* beta = nullptr);
 // nwords 8-byte words device -> host-mapped (cudaHostAllocMapped) memory by a kernel, bypassing the copy engine
 cudaError_t launch_copy_words(const void* src, void* dst_mapped, int64_t nwords, cudaStream_t st);
 // global min / max of a device array of n doubles, NaN ignored (na.rm = TRUE); res[0]=min res[1]=max

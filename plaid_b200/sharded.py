@@ -268,6 +268,22 @@ def score_group_stats_shard(ctx, comm, M: L.Matrix, rowmap: np.ndarray, opts: L.
     return comm.allreduce_sum_vec(out.ravel()).reshape(out.shape)
 
 
+def score_topk_shard(ctx, comm, M: L.Matrix, rowmap: np.ndarray, opts: L.Opts, k: int, decreasing: bool, n_cols: int):
+    """Each of this rank's cells' k best gene sets: score_shard into a device buffer, then plaidgpu_col_topk on it.
+    The selection is column-local, so nothing is exchanged beyond what scoring needs.  `ctx` must hold the gene sets
+    (Context.set_genesets).  Returns (idx, val) of shape (k, n_cols) for this shard's columns."""
+    import torch
+    S = ctx.n_sets
+    buf = torch.empty(max(S * n_cols, 1), dtype=torch.float64, device=f"cuda:{ctx.device}")
+    opts.out_location = L.DEVICE
+    score_shard(ctx, comm, M, rowmap, opts, buf.data_ptr(), n_cols)
+    idx = np.empty((max(int(k), 0), n_cols), dtype=np.int32, order="F")
+    val = np.empty((max(int(k), 0), n_cols), dtype=np.float64, order="F")
+    ctx.check(ctx.lib.plaidgpu_col_topk(ctx.h, buf.data_ptr(), S, n_cols, int(k), 1 if decreasing else 0, L.DEVICE,
+                                        idx.ctypes.data, val.ctypes.data))
+    return idx, val
+
+
 def shard_columns(n_total: int, world: int, rank: int):
     """contiguous, equal-count column ranges (equal output bytes, the dominant cost)"""
     base, rem = divmod(n_total, world)

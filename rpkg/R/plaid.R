@@ -37,7 +37,7 @@
   }
 }
 
-.score <- function(X, matG, opts, labels = NULL, K = NULL) {
+.score <- function(X, matG, opts, labels = NULL, K = NULL, topk = NULL, decreasing = TRUE) {
   x <- .as_x(X)
   rn <- x$dimnames[[1]]
   gg <- intersect(rn, rownames(matG))                                 # R/plaid.R:65
@@ -57,10 +57,43 @@
     rownames(out) <- colnames(matG)
     return(out)
   }
+  if (!is.null(topk)) {  # plaid.topsets: each column's top k sets selected on the device, k x 2N back
+    out <- .Call(C_plaidgpu_score_topk, .ctxs(), x$kind, x$p, x$i, x$x, as.integer(x$dim),
+                 G@p, G@i, G@x, as.integer(dim(G)), as.integer(rowmap), opts, as.integer(topk),
+                 as.integer(isTRUE(decreasing)))
+    return(.topsets(out, topk, x$dimnames[[2]]))
+  }
   out <- .Call(C_plaidgpu_score, .ctxs(), x$kind, x$p, x$i, x$x, as.integer(x$dim),
                G@p, G@i, G@x, as.integer(dim(G)), as.integer(rowmap), opts)
   dimnames(out) <- list(colnames(matG), x$dimnames[[2]])
   out
+}
+
+## the k x 2N matrix of the top-k shim entries (1-based indices, then scores) -> list(index, score)
+.topsets <- function(out, k, cn) {
+  N <- ncol(out) %/% 2L
+  index <- matrix(as.integer(out[, seq_len(N)]), k, N)
+  score <- out[, N + seq_len(N), drop = FALSE]
+  colnames(index) <- cn
+  colnames(score) <- cn
+  list(index = index, score = score)
+}
+
+## Each cell's k best gene sets: the first k entries of order(v, decreasing = decreasing) for every column v of
+## plaid(X, matG) (ties by set order, NA last), i.e. apply(plaid(X, matG), 2, order, decreasing = TRUE)[1:k, ] and
+## the scores at those sets, without the S x N score matrix ever reaching R: plaid() and the selection run as one
+## device call (options(plaid.gpus) applies).  With gsetX (the scores of any scorer, sets x cells) the selection
+## runs on that matrix instead.  1 <= k <= min(ncol(matG), 256).  Returns list(index = integer k x N (rows of matG,
+## 1-based), score = double k x N), both with colnames(X); colnames(matG)[index] names the sets.
+plaid.topsets <- function(X, matG, k = 10, decreasing = TRUE, gsetX = NULL) {
+  if (is.null(gsetX))
+    return(.score(X, matG, list(scorer = 0L, stats_mean = 1L, normalize = 1L), topk = k, decreasing = decreasing))
+  gsetX <- as.matrix(gsetX)
+  storage.mode(gsetX) <- "double"
+  out <- .Call(C_plaidgpu_col_topk, .ctx(), gsetX, as.integer(k), as.integer(isTRUE(decreasing)))
+  cn <- colnames(X)
+  if (is.null(cn)) cn <- colnames(gsetX)
+  .topsets(out, k, cn)
 }
 
 plaid <- function(X, matG, stats = c("mean", "sum"), chunk = NULL, normalize = TRUE) {

@@ -231,6 +231,74 @@ SEXP C_plaidgpu_score_group_stats(SEXP ctx, SEXP kind, SEXP Xp, SEXP Xi, SEXP Xx
   return out;
 }
 
+/* per-column top k as one k x 2N matrix: columns 1..N the 1-based row indices (exact in a double), N+1..2N the values;
+ * idx / val are what plaidgpu_col_topk / plaidgpu_score_topk wrote, val already in place */
+static void topk_indices_to_r(SEXP out, const int32_t* idx, int k, int N) {
+  double* o = REAL(out);
+  for (R_xlen_t t = 0, n = (R_xlen_t)k * N; t < n; ++t) o[t] = (double)idx[t] + 1.0;
+}
+
+/* plaid.topsets(gsetX = ): each column's k first rows of order(x[, j], decreasing = decreasing) */
+SEXP C_plaidgpu_col_topk(SEXP ctx, SEXP x, SEXP k, SEXP decreasing) {
+  plaidgpu_ctx* c = get_ctx(ctx);
+  SEXP dim = Rf_getAttrib(x, R_DimSymbol);
+  const int S = INTEGER(dim)[0], N = INTEGER(dim)[1], kk = Rf_asInteger(k);
+  if (kk < 1 || kk > 256 || kk > S) Rf_error("plaidgpu: k must be in [1, min(nrow(x), 256)]");
+  int32_t* idx = (int32_t*)R_alloc((size_t)kk * (size_t)N + 1, sizeof(int32_t));
+  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, kk, 2 * N));
+  int rc = plaidgpu_col_topk(c, REAL(x), S, N, kk, Rf_asInteger(decreasing), PLAIDGPU_HOST, idx,
+                             REAL(out) + (R_xlen_t)kk * N);
+  if (rc != PLAIDGPU_OK) {
+    UNPROTECT(1);
+    Rf_error("plaidgpu_col_topk: %s", plaidgpu_last_error(c));
+  }
+  topk_indices_to_r(out, idx, kk, N);
+  UNPROTECT(1);
+  return out;
+}
+
+/* plaid.topsets(): plaid() fused with each cell's top k sets — the S x N scores stay on the device, a k x 2N matrix
+ * (indices, then scores) comes back.  A list of contexts (options(plaid.gpus = n)) splits the columns over the
+ * devices (plaidgpu_score_topk_multi). */
+SEXP C_plaidgpu_score_topk(SEXP ctx, SEXP kind, SEXP Xp, SEXP Xi, SEXP Xx, SEXP Xdim, SEXP Gp, SEXP Gi, SEXP Gx,
+                           SEXP Gdim, SEXP rowmap, SEXP opts, SEXP k, SEXP decreasing) {
+  plaidgpu_ctx* cs[16];
+  int nctx = 1;
+  if (TYPEOF(ctx) == VECSXP) {
+    nctx = (int)XLENGTH(ctx);
+    if (nctx < 1 || nctx > 16) Rf_error("plaidgpu: between 1 and 16 contexts expected");
+    for (int j = 0; j < nctx; ++j) cs[j] = get_ctx(VECTOR_ELT(ctx, j));
+  } else {
+    cs[0] = get_ctx(ctx);
+  }
+  plaidgpu_ctx* c = cs[0];
+  const int PG = INTEGER(Gdim)[0], S = INTEGER(Gdim)[1], kk = Rf_asInteger(k);
+  if (kk < 1 || kk > 256 || kk > S) Rf_error("plaidgpu: k must be in [1, min(ncol(matG), 256)]");
+  for (int j = 0; j < nctx; ++j)
+    if (plaidgpu_set_genesets(cs[j], PG, S, INTEGER(Gp), INTEGER(Gi), REAL(Gx)) != PLAIDGPU_OK)
+      Rf_error("plaidgpu_set_genesets: %s", plaidgpu_last_error(cs[j]));
+  plaidgpu_matrix M;
+  fill_matrix(&M, Rf_asInteger(kind), Xp, Xi, Xx, Xdim);
+  if (M.N > INT_MAX / 2) Rf_error("plaidgpu: too many columns for one k x 2N result");
+  const int N = (int)M.N;
+  plaidgpu_opts o;
+  fill_opts(&o, opts);
+  R_CheckUserInterrupt();
+  int32_t* idx = (int32_t*)R_alloc((size_t)kk * (size_t)N + 1, sizeof(int32_t));
+  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, kk, 2 * N));
+  double* val = REAL(out) + (R_xlen_t)kk * N;
+  const int dec = Rf_asInteger(decreasing);
+  int rc = nctx > 1 ? plaidgpu_score_topk_multi(cs, nctx, &M, INTEGER(rowmap), &o, kk, dec, idx, val)
+                    : plaidgpu_score_topk(c, &M, INTEGER(rowmap), &o, kk, dec, idx, val);
+  if (rc != PLAIDGPU_OK) {
+    UNPROTECT(1);
+    Rf_error("plaidgpu_score_topk: %s", plaidgpu_last_error(c));
+  }
+  topk_indices_to_r(out, idx, kk, N);
+  UNPROTECT(1);
+  return out;
+}
+
 static const R_CallMethodDef call_methods[] = {
     {"C_plaidgpu_ctx", (DL_FUNC)&C_plaidgpu_ctx, 1},
     {"C_plaidgpu_score", (DL_FUNC)&C_plaidgpu_score, 12},
@@ -238,6 +306,8 @@ static const R_CallMethodDef call_methods[] = {
     {"C_plaidgpu_colranks", (DL_FUNC)&C_plaidgpu_colranks, 9},
     {"C_plaidgpu_group_stats", (DL_FUNC)&C_plaidgpu_group_stats, 4},
     {"C_plaidgpu_score_group_stats", (DL_FUNC)&C_plaidgpu_score_group_stats, 14},
+    {"C_plaidgpu_col_topk", (DL_FUNC)&C_plaidgpu_col_topk, 4},
+    {"C_plaidgpu_score_topk", (DL_FUNC)&C_plaidgpu_score_topk, 14},
     {"C_plaidgpu_crossprod", (DL_FUNC)&C_plaidgpu_crossprod, 11},
     {NULL, NULL, 0}};
 
