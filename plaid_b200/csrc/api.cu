@@ -206,14 +206,6 @@ struct plaidgpu_ctx {
   int64_t h2d_piece = 0;
   bool h2d_pending = false;
   const int32_t* xp_host = nullptr;
-  // plaidgpu_score_group_stats: finish reduces the (fixed-up on the fly) scores by group instead of shipping them
-  const int32_t* mom_labels = nullptr;
-  int mom_K = 0;
-  double* mom_out = nullptr;
-  // plaidgpu_score_topk: finish selects each column's top k of the (fixed-up on the fly) scores instead (host idx / val)
-  int topk_k = 0, topk_dec = 1;
-  int32_t* topk_idx = nullptr;
-  double* topk_val = nullptr;
   // mailbox: pinned, device-mapped host memory the GPU writes small results into (launch_copy_words)
   void* mbox = nullptr;
   void* mbox_dev = nullptr;
@@ -777,6 +769,12 @@ bool is_rank_scorer(int s) {
   return s == PLAIDGPU_SING || s == PLAIDGPU_SSGSEA || s == PLAIDGPU_UCELL || s == PLAIDGPU_AUCELL;
 }
 
+// the scores of the call are median-normalised (normalize_medians, R/plaid.R)
+bool needs_norm(const plaidgpu_opts& o) {
+  return (o.scorer == PLAIDGPU_PLAID && o.normalize) || o.scorer == PLAIDGPU_SSGSEA || o.scorer == PLAIDGPU_UCELL ||
+         o.scorer == PLAIDGPU_AUCELL || o.scorer == PLAIDGPU_GSVA;
+}
+
 // order-preserving key -> double on the host (inverse of key_of in common.cuh)
 double host_value_of(unsigned long long k) {
   const unsigned long long b = (k & 0x8000000000000000ull) ? (k & 0x7fffffffffffffffull) : ~k;
@@ -1062,6 +1060,62 @@ int host_chunk_cols(plaidgpu_ctx* c, const plaidgpu_matrix* X, int64_t* chunk) {
   *chunk = ch;
   return PLAIDGPU_OK;
 }
+
+// columns [j0, j1) of the host matrix X; a CSC slice's rebased column pointers live in pbuf
+plaidgpu_matrix column_slice(const plaidgpu_matrix* X, int64_t j0, int64_t j1, std::vector<int32_t>& pbuf) {
+  plaidgpu_matrix M = *X;
+  M.N = j1 - j0;
+  if (X->kind == PLAIDGPU_CSC) {
+    const int32_t base = X->p[j0];
+    pbuf.resize((size_t)(j1 - j0 + 1));
+    for (int64_t j = j0; j <= j1; ++j) pbuf[(size_t)(j - j0)] = X->p[j] - base;
+    M.p = pbuf.data();
+    M.i = X->i + base;
+    M.x = X->x + base;
+  } else {
+    M.x = X->x + j0 * (int64_t)X->P;
+  }
+  return M;
+}
+
+// What the finish step of a scoring call makes of the raw S x N scores.  Every kind but SCORES keeps the raw scores
+// in the library's device buffer (out_location = PLAIDGPU_HOST) and applies the fix-up in registers.
+struct Target {
+  enum Kind { SCORES, GROUP_STATS, TOPK, FILE_TILES } kind = SCORES;
+  double* out = nullptr;            // SCORES: the S x N scores at opts.out_location; GROUP_STATS: K * 2 * S moments
+  const int32_t* labels = nullptr;  // GROUP_STATS: int32[N] in [-1, K)
+  int K = 0;
+  int k = 0, decreasing = 0;        // TOPK: idx / val hold k * N entries
+  int32_t* idx = nullptr;
+  double* val = nullptr;
+  FILE* file = nullptr;             // FILE_TILES (score_chunked): tile t is staged in stage[t & 1] (stage[0] when
+  double* stage[2] = {};            // stage[1] is null) and written to `file` by a helper thread
+
+  static Target scores(double* out) { Target t; t.out = out; return t; }
+  static Target group_stats(const int32_t* labels, int K, double* out) {
+    Target t; t.kind = GROUP_STATS; t.labels = labels; t.K = K; t.out = out; return t;
+  }
+  static Target topk(int k, int decreasing, int32_t* idx, double* val) {
+    Target t; t.kind = TOPK; t.k = k; t.decreasing = decreasing != 0; t.idx = idx; t.val = val; return t;
+  }
+  static Target to_file(FILE* file, double* stage0, double* stage1) {
+    Target t; t.kind = FILE_TILES; t.file = file; t.stage[0] = stage0; t.stage[1] = stage1; return t;
+  }
+  // the same target for the columns from j0 on; group statistics write those columns' moments to `moments`
+  Target from(int64_t j0, int32_t S, double* moments) const {
+    Target t = *this;
+    if (kind == SCORES) t.out = out + j0 * (int64_t)S;
+    if (kind == GROUP_STATS) {
+      t.labels = labels + j0;
+      t.out = moments;
+    }
+    if (kind == TOPK) {
+      t.idx = idx + j0 * k;
+      t.val = val + j0 * k;
+    }
+    return t;
+  }
+};
 
 }  // namespace
 
@@ -1401,11 +1455,10 @@ int plaidgpu_score_compute(plaidgpu_ctx* c, plaidgpu_scalars* scal, double* out)
   p.ld = c->S;
   int colnorm = 0;
   bool mean = true;
-  c->need_norm = false;
+  c->need_norm = needs_norm(o);
   switch (o.scorer) {
     case PLAIDGPU_PLAID:
       mean = o.stats_mean != 0;
-      c->need_norm = o.normalize != 0;
       break;
     case PLAIDGPU_SCSE: {
       const bool rl = o.remove_log2 < 0 ? (scal->x_min == 0.0 && scal->x_max < 20.0) : (o.remove_log2 != 0);
@@ -1422,25 +1475,21 @@ int plaidgpu_score_compute(plaidgpu_ctx* c, plaidgpu_scalars* scal, double* out)
       p.mode = XF_SSGSEA;
       p.a1 = o.alpha;
       p.a0 = (o.alpha != 0.0) ? pow(scal->rank_max, 1.0 + o.alpha) : scal->rank_max;
-      c->need_norm = true;
       break;
     case PLAIDGPU_UCELL:
       p.mode = XF_UCELL;
       p.a0 = scal->rank_max;
       p.a1 = o.rmax + 1.0;
-      c->need_norm = true;
       break;
     case PLAIDGPU_AUCELL:
       p.mode = XF_AUCELL;
       p.a0 = scal->rank_max;
       p.a1 = o.auc_max_rank > 0.0 ? o.auc_max_rank : ceil(0.05 * (double)c->P);
-      c->need_norm = true;
       break;
     case PLAIDGPU_GSVA:
       p.mode = XF_GSVA;
       p.a0 = scal->rank_max;
       p.a1 = o.tau;
-      c->need_norm = true;
       break;
     default:
       return fail(c, PLAIDGPU_ERR_ARG, "unknown scorer");
@@ -1792,9 +1841,9 @@ int plaidgpu_combine_medians(int ignore_zero_opt, double score_min, const double
   return PLAIDGPU_ERR_ARG;
 }
 
-int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double* out) try {
-  if (!c) return PLAIDGPU_ERR_ARG;
-  if (!scal || (!out && c->N > 0 && !c->mom_labels && !c->topk_idx)) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+// plaidgpu_score_finish into target t (SCORES, GROUP_STATS or TOPK)
+static int score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, const Target& t) try {
+  if (t.kind == Target::SCORES && !t.out && c->N > 0) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
   if (!c->computed) return fail(c, PLAIDGPU_ERR_STATE, "plaidgpu_score_compute has not been called");
   CK(cudaSetDevice(c->device));
   const plaidgpu_opts& o = c->opts;
@@ -1804,6 +1853,7 @@ int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double*
   double alpha = 1.0, cc = 0.0;
   const double* med = nullptr;
   const double* beta = nullptr;
+  std::vector<double> hbeta;  // host copy of beta (outlives the early-column patcher below)
   bool fix = false;
   if (c->need_norm) {
     int rc = ensure_median(c, scal->ignore_zero != 0);
@@ -1813,36 +1863,22 @@ int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double*
     fix = true;
   }
   if (o.scorer == PLAIDGPU_UCELL) {  // 1 - S/rmax + (colSums(matG != 0) + 1) / (2 rmax)   (R/plaid.R:280)
-    std::vector<double> b((size_t)S);
+    hbeta.resize((size_t)S);
     const double* gs = o.matg_full_colsums ? o.matg_full_colsums : c->g_colsums.data();
-    for (int32_t s = 0; s < S; ++s) b[s] = 1.0 + (gs[s] + 1.0) / (2.0 * o.rmax);
+    for (int32_t s = 0; s < S; ++s) hbeta[s] = 1.0 + (gs[s] + 1.0) / (2.0 * o.rmax);
     CK(c->d_beta.reserve((size_t)S * sizeof(double)));
-    CK(cudaMemcpyAsync(c->d_beta.p, b.data(), (size_t)S * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(c->d_beta.p, hbeta.data(), (size_t)S * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     beta = c->d_beta.as<double>();
     alpha = -1.0 / o.rmax;
     fix = true;
   }
 
-  if (c->mom_labels) {
-    // score -> test: per-set sums / sums of squares of the normalised scores by sample group, the fix-up applied in
-    // registers; the S x N matrix stays on the device as raw scores and nothing but K * 2 * S doubles goes back
-    const int32_t* lab = c->mom_labels;
-    const int K = c->mom_K;
-    double* mo = c->mom_out;
-    c->mom_labels = nullptr;
-    c->mom_out = nullptr;
-    return group_stats_device(c, c->raw, S, N, lab, K, mo, fix, med, cc, alpha, beta);
-  }
-  if (c->topk_idx) {
-    // score -> top sets: each column's k first sets of the normalised scores, the fix-up applied in registers; the
-    // S x N matrix stays on the device as raw scores and k * N indices and values go back
-    int32_t* ti = c->topk_idx;
-    double* tv = c->topk_val;
-    c->topk_idx = nullptr;
-    c->topk_val = nullptr;
-    return topk_device(c, c->raw, S, N, c->topk_k, c->topk_dec, ti, tv, fix, med, cc, alpha, beta);
-  }
+  // the reductions read the raw scores with the fix-up applied in registers: the S x N matrix stays on the device
+  // and only K * 2 * S moments, or k * N indices and values, go back
+  if (t.kind == Target::GROUP_STATS) return group_stats_device(c, c->raw, S, N, t.labels, t.K, t.out, fix, med, cc, alpha, beta);
+  if (t.kind == Target::TOPK) return topk_device(c, c->raw, S, N, t.k, t.decreasing, t.idx, t.val, fix, med, cc, alpha, beta);
+  double* out = t.out;
   c->raw_valid = false;  // the fix-up below rewrites the raw scores in place
   CK(cudaEventRecord(c->ev[4], c->stream));
   if (o.out_location == PLAIDGPU_DEVICE) {
@@ -1907,13 +1943,7 @@ int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double*
         if (t.joinable()) t.join();
       }
     } joiner{patcher};  // also on the error returns below
-    std::vector<double> hbeta;
     if (E > 0 && fix) {
-      if (beta) {
-        hbeta.resize((size_t)S);
-        const double* gs = o.matg_full_colsums ? o.matg_full_colsums : c->g_colsums.data();
-        for (int32_t s = 0; s < S; ++s) hbeta[s] = 1.0 + (gs[s] + 1.0) / (2.0 * o.rmax);
-      }
       if (!c->pool) {
         int nt = (int)std::min<unsigned>(8, std::max(2u, std::thread::hardware_concurrency() / 2));
         if (const char* e = getenv("PLAIDGPU_COPY_THREADS")) nt = std::max(1, std::min(64, atoi(e)));
@@ -1978,71 +2008,35 @@ int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double*
   return PLAIDGPU_ERR_ARG;
 }
 
+int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double* out) try {
+  if (!c) return PLAIDGPU_ERR_ARG;
+  if (!scal) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  return score_finish(c, scal, Target::scores(out));
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
 // Column-chunked scoring for host input / host output when the S x N result does not fit the device
 // (e.g. 30k sets x 1M cells = 240 GB): the same begin / compute / finish pipeline runs per chunk of
 // columns (the axis chunked_crossprod splits on, R/plaid.R:110-119).  The global scalars need all
 // columns, so a normalised call recomputes the scores: pass 1 keeps only the per-column medians,
 // pass 2 recomputes, fixes up and streams each chunk out (recomputing costs less than moving the raw
 // scores over PCIe twice).  Results are bit-identical to the un-chunked path.
-// `sink` (optional): instead of landing in `out`, every finished chunk is staged in a pinned buffer and
-// written to the file — tiled egress for results larger than host memory (scope row f4).
-// `reduce` (optional): every finished chunk is reduced on the device instead (finish_into): per set and sample
-// group (plaidgpu_score_group_stats), with `out` (K * 2 * S doubles, zeroed by the caller) accumulating the tiles'
-// moments in tile order, or to each column's top k (plaidgpu_score_topk), the tile of columns [j0, j1) writing
-// idx / val + j0 * k.
-struct ScoreSink {
-  const int32_t* labels;  // group statistics: int32[N] of the whole call, or nullptr for top k
-  int K;
-  int k, decreasing;      // top k: idx / val hold k * N entries of the whole call
-  int32_t* idx;
-  double* val;
-};
-
-// plaidgpu_score_finish reducing the scores of columns [j0, ...) of the call as `sk` says instead of shipping them;
-// moments: K * 2 * S doubles for group statistics
-static int finish_into(plaidgpu_ctx* c, const plaidgpu_scalars* s, const ScoreSink& sk, int64_t j0, double* moments) {
-  if (sk.labels) {
-    c->mom_labels = sk.labels + j0;
-    c->mom_K = sk.K;
-    c->mom_out = moments;
-  } else {
-    c->topk_k = sk.k;
-    c->topk_dec = sk.decreasing;
-    c->topk_idx = sk.idx + j0 * sk.k;
-    c->topk_val = sk.val + j0 * sk.k;
-  }
-  const int rc = plaidgpu_score_finish(c, s, nullptr);
-  c->mom_labels = nullptr;
-  c->mom_out = nullptr;
-  c->topk_idx = nullptr;
-  c->topk_val = nullptr;
-  return rc;
-}
-
+// The tile of columns [j0, j1) finishes into t.from(j0): its columns of the scores or of idx / val, or its group
+// moments, which are added to t.out (zeroed here) in tile order.  FILE_TILES stages every finished tile in a pinned
+// buffer and writes it to the file: tiled egress for results larger than host memory (scope row f4).
 static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
-                         double* out, int64_t chunk, FILE* sink = nullptr, double* stage = nullptr, double* stage2 = nullptr,
-                         const ScoreSink* reduce = nullptr) {
+                         const Target& t, int64_t chunk) {
   const int64_t N = X->N;
   const int32_t S = c->S;
-  std::vector<double> moments(reduce && reduce->labels ? (size_t)reduce->K * 2 * (size_t)S : 0);  // one tile's group moments
+  std::vector<double> moments(t.kind == Target::GROUP_STATS ? (size_t)t.K * 2 * (size_t)S : 0);  // one tile's group moments
+  if (t.kind == Target::GROUP_STATS) std::fill(t.out, t.out + moments.size(), 0.0);
   if (opts->scorer == PLAIDGPU_GSVA && opts->gsva_ecdf != PLAIDGPU_ROWTF_DONE &&
       (opts->gsva_ecdf || !(opts->row_mean && opts->row_sd)))
     return fail(c, PLAIDGPU_ERR_ARG, "replaid.gsva: matrix too large for one device pass (rowtf ecdf needs all samples; rowtf z needs row_mean / row_sd)");
   std::vector<int32_t> pbuf;
-  auto sub = [&](int64_t j0, int64_t j1, plaidgpu_matrix* M) {
-    *M = *X;
-    M->N = j1 - j0;
-    if (X->kind == PLAIDGPU_CSC) {
-      const int32_t base = X->p[j0];
-      pbuf.resize((size_t)(j1 - j0 + 1));
-      for (int64_t j = j0; j <= j1; ++j) pbuf[(size_t)(j - j0)] = X->p[j] - base;
-      M->p = pbuf.data();
-      M->i = X->i + base;
-      M->x = X->x + base;
-    } else {
-      M->x = X->x + j0 * (int64_t)X->P;
-    }
-  };
   plaidgpu_scalars g;
   memset(&g, 0, sizeof(g));
   g.x_min = INFINITY;
@@ -2056,7 +2050,7 @@ static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_
   int rc;
   if (need_pre) {
     for (int64_t j0 = 0; j0 < N; j0 += chunk) {
-      sub(j0, std::min(N, j0 + chunk), &M);
+      M = column_slice(X, j0, std::min(N, j0 + chunk), pbuf);
       rc = plaidgpu_score_begin(c, &M, rowmap, opts, &loc);
       if (rc) return rc;
       g.x_min = fmin(g.x_min, loc.x_min);
@@ -2064,8 +2058,7 @@ static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_
       g.rank_max = fmax(g.rank_max, loc.rank_max);
     }
   }
-  const bool norm = (opts->scorer == PLAIDGPU_PLAID && opts->normalize) || opts->scorer == PLAIDGPU_SSGSEA ||
-                    opts->scorer == PLAIDGPU_UCELL || opts->scorer == PLAIDGPU_AUCELL || opts->scorer == PLAIDGPU_GSVA;
+  const bool norm = needs_norm(*opts);
   if (norm) {
     std::vector<double> ma((size_t)N), mz((size_t)N);
     double smin = INFINITY;
@@ -2077,7 +2070,7 @@ static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_
     c->want_both = opts->ignore_zero < 0;
     for (int64_t j0 = 0; j0 < N; j0 += chunk) {
       const int64_t j1 = std::min(N, j0 + chunk);
-      sub(j0, j1, &M);
+      M = column_slice(X, j0, j1, pbuf);
       rc = plaidgpu_score_begin(c, &M, rowmap, opts, &loc);
       if (rc) return rc;
       plaidgpu_scalars s = g;
@@ -2104,7 +2097,7 @@ static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_
   int64_t tile = 0;
   for (int64_t j0 = 0; j0 < N; j0 += chunk, ++tile) {
     const int64_t j1 = std::min(N, j0 + chunk);
-    sub(j0, j1, &M);
+    M = column_slice(X, j0, j1, pbuf);
     rc = plaidgpu_score_begin(c, &M, rowmap, &o2, &loc);
     if (rc) return rc;
     plaidgpu_scalars s = g;
@@ -2112,24 +2105,23 @@ static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_
     if (rc) return rc;
     s.ignore_zero = g.ignore_zero;
     s.med_mean = g.med_mean;
-    if (reduce) {
-      rc = finish_into(c, &s, *reduce, j0, moments.data());
+    if (t.kind != Target::FILE_TILES) {
+      rc = score_finish(c, &s, t.from(j0, S, moments.data()));
       if (rc) return rc;
-      for (size_t i = 0; i < moments.size(); ++i) out[i] += moments[i];
+      for (size_t i = 0; i < moments.size(); ++i) t.out[i] += moments[i];
       continue;
     }
-    double* dst = sink ? ((stage2 && (tile & 1)) ? stage2 : stage) : out + j0 * (int64_t)S;
-    if (sink && !stage2 && writer.joinable()) writer.join();  // one buffer only: it must be free again
-    rc = plaidgpu_score_finish(c, &s, dst);
+    double* dst = (t.stage[1] && (tile & 1)) ? t.stage[1] : t.stage[0];
+    if (!t.stage[1] && writer.joinable()) writer.join();  // one buffer only: it must be free again
+    rc = score_finish(c, &s, Target::scores(dst));
     if (rc) return rc;
-    if (sink) {
-      if (writer.joinable()) writer.join();  // tile k - 1 on disk (its buffer is the one tile k + 1 will use)
-      if (short_write) return fail(c, PLAIDGPU_ERR_ARG, "short write to the output file");
-      const size_t cnt = (size_t)(j1 - j0) * (size_t)S;
-      writer = std::thread([dst, cnt, sink, &short_write] {
-        if (fwrite(dst, sizeof(double), cnt, sink) != cnt) short_write = true;
-      });
-    }
+    if (writer.joinable()) writer.join();  // tile k - 1 on disk (its buffer is the one tile k + 1 will use)
+    if (short_write) return fail(c, PLAIDGPU_ERR_ARG, "short write to the output file");
+    const size_t cnt = (size_t)(j1 - j0) * (size_t)S;
+    FILE* f = t.file;
+    writer = std::thread([dst, cnt, f, &short_write] {
+      if (fwrite(dst, sizeof(double), cnt, f) != cnt) short_write = true;
+    });
   }
   if (writer.joinable()) writer.join();
   if (short_write) return fail(c, PLAIDGPU_ERR_ARG, "short write to the output file");
@@ -2185,7 +2177,7 @@ int plaidgpu_score_to_file(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int3
     const size_t cnt = (size_t)N * (size_t)S;
     if (!rc && cnt && fwrite(stage, sizeof(double), cnt, f) != cnt) rc = fail(c, PLAIDGPU_ERR_ARG, "short write to the output file");
   } else {
-    rc = score_chunked(c, X, rowmap, &o, nullptr, chunk, f, stage, stage + stage_elems);
+    rc = score_chunked(c, X, rowmap, &o, Target::to_file(f, stage, stage + stage_elems), chunk);
   }
   cudaFreeHost(stage);
   if (fclose(f) != 0 && !rc) rc = fail(c, PLAIDGPU_ERR_ARG, "closing the output file failed");
@@ -2196,32 +2188,40 @@ int plaidgpu_score_to_file(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int3
   return PLAIDGPU_ERR_ARG;
 }
 
+// One device: begin -> compute -> the single shard's median combine -> finish into t.  Host X whose S x N scores
+// exceed the device goes through score_chunked.
+static int score_one(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
+                     const Target& t) {
+  plaidgpu_opts o = *opts;
+  if (t.kind != Target::SCORES) o.out_location = PLAIDGPU_HOST;  // raw scores in the library's device buffer
+  if (o.out_location == PLAIDGPU_HOST) {  // host in / host out larger than the device can hold -> column chunks
+    int64_t chunk = 0;
+    int rc = host_chunk_cols(c, X, &chunk);
+    if (rc) return rc;
+    if (chunk > 0) return score_chunked(c, X, rowmap, &o, t, chunk);
+  }
+  plaidgpu_scalars s;
+  int rc = plaidgpu_score_begin(c, X, rowmap, &o, &s);
+  if (rc) return rc;
+  rc = plaidgpu_score_compute(c, &s, t.kind == Target::SCORES ? t.out : nullptr);
+  if (rc) return rc;
+  if (c->need_norm) {
+    // one shard holds every column: its own minimum decides, and only that median was computed
+    const bool iz = o.ignore_zero < 0 ? (s.score_min == 0.0) : (o.ignore_zero != 0);
+    rc = ensure_median(c, iz);
+    if (rc) return rc;
+    const double* m = iz ? c->h_med_nz.data() : c->h_med_all.data();
+    rc = plaidgpu_combine_medians(o.ignore_zero, s.score_min, m, m, c->N, &s);
+    if (rc) return fail(c, rc, "combine_medians failed");
+  }
+  return score_finish(c, &s, t);
+}
+
 int plaidgpu_score(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
                    double* out) try {
   if (!c) return PLAIDGPU_ERR_ARG;
   if (!X || !opts) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
-  // host in / host out larger than the device can hold -> column chunks
-  if (opts->out_location == PLAIDGPU_HOST) {
-    int64_t chunk = 0;
-    int rc = host_chunk_cols(c, X, &chunk);
-    if (rc) return rc;
-    if (chunk > 0) return score_chunked(c, X, rowmap, opts, out, chunk);
-  }
-  plaidgpu_scalars s;
-  int rc = plaidgpu_score_begin(c, X, rowmap, opts, &s);
-  if (rc) return rc;
-  rc = plaidgpu_score_compute(c, &s, out);
-  if (rc) return rc;
-  if (c->need_norm) {
-    // one shard holds every column: its own minimum decides, and only that median was computed
-    const bool iz = opts->ignore_zero < 0 ? (s.score_min == 0.0) : (opts->ignore_zero != 0);
-    rc = ensure_median(c, iz);
-    if (rc) return rc;
-    const double* m = iz ? c->h_med_nz.data() : c->h_med_all.data();
-    rc = plaidgpu_combine_medians(opts->ignore_zero, s.score_min, m, m, c->N, &s);
-    if (rc) return fail(c, rc, "combine_medians failed");
-  }
-  return plaidgpu_score_finish(c, &s, out);
+  return score_one(c, X, rowmap, opts, Target::scores(out));
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {
@@ -2232,43 +2232,13 @@ int plaidgpu_score(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* row
 // plaid.test(tests = "lm") (R/plaid.R:426-431) without the S x N matrix ever leaving the device or being written in
 // its normalised form.  Bit-identical to plaidgpu_score + plaidgpu_group_stats.  Host X whose S x N scores exceed
 // the device goes through score_chunked (two passes when normalised) and adds the tiles' moments in tile order.
-// plaidgpu_score's pipeline with a finish step that reduces on the device (finish_into); `out`: the K * 2 * S moments
-// of group statistics.  Host X whose S x N scores exceed the device goes through score_chunked.
-static int score_reduce(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
-                        const ScoreSink& sk, double* out) {
-  plaidgpu_opts o = *opts;
-  o.out_location = PLAIDGPU_HOST;  // raw scores in the library's device buffer
-  int64_t chunk = 0;
-  int rc = host_chunk_cols(c, X, &chunk);
-  if (rc) return rc;
-  if (chunk > 0) {
-    if (sk.labels) std::fill(out, out + (size_t)sk.K * 2 * (size_t)c->S, 0.0);
-    return score_chunked(c, X, rowmap, &o, out, chunk, nullptr, nullptr, nullptr, &sk);
-  }
-  plaidgpu_scalars s;
-  rc = plaidgpu_score_begin(c, X, rowmap, &o, &s);
-  if (rc) return rc;
-  rc = plaidgpu_score_compute(c, &s, nullptr);
-  if (rc) return rc;
-  if (c->need_norm) {
-    const bool iz = o.ignore_zero < 0 ? (s.score_min == 0.0) : (o.ignore_zero != 0);
-    rc = ensure_median(c, iz);
-    if (rc) return rc;
-    const double* m = iz ? c->h_med_nz.data() : c->h_med_all.data();
-    rc = plaidgpu_combine_medians(o.ignore_zero, s.score_min, m, m, c->N, &s);
-    if (rc) return fail(c, rc, "combine_medians failed");
-  }
-  return finish_into(c, &s, sk, 0, out);
-}
-
 int plaidgpu_score_group_stats(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
                                const int32_t* labels, int K, double* out) try {
   if (!c) return PLAIDGPU_ERR_ARG;
   if (!X || !rowmap || !opts || !out) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
   int rc = check_groups(c, labels, X->N, K);
   if (rc) return rc;
-  const ScoreSink sk{labels, K, 0, 0, nullptr, nullptr};
-  return score_reduce(c, X, rowmap, opts, sk, out);
+  return score_one(c, X, rowmap, opts, Target::group_stats(labels, K, out));
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {
@@ -2287,8 +2257,7 @@ int plaidgpu_score_topk(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t
   int rc = check_topk(c, c->S, k);
   if (rc) return rc;
   if (X->N == 0) return PLAIDGPU_OK;
-  const ScoreSink sk{nullptr, 0, k, decreasing != 0, idx, val};
-  return score_reduce(c, X, rowmap, opts, sk, nullptr);
+  return score_one(c, X, rowmap, opts, Target::topk(k, decreasing, idx, val));
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {
@@ -2349,46 +2318,26 @@ static int check_shard_ctxs(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_opt
   return PLAIDGPU_OK;
 }
 
-// reduce == nullptr: the S x N scores land in `out` (plaidgpu_score_multi).  Otherwise every shard reduces its scores
-// on its device (finish_into): per set and group, `out` (K * 2 * S doubles) receiving the shards' moments added in
-// shard order (plaidgpu_score_group_stats_multi), or to each column's top k, shard r writing columns [lo_r, hi_r) of
-// idx / val (plaidgpu_score_topk_multi).
+// Shard r (columns [lo_r, lo_{r+1})) finishes on ctxs[r] into t.from(lo_r): its block of the scores, its columns of
+// idx / val, or its own group moments, of which shard 0's are copied to t.out and shards 1 to n - 1 added in shard
+// order.
 static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
-                            const plaidgpu_opts* opts, double* out, const ScoreSink* reduce, const char* name) {
+                            const plaidgpu_opts* opts, const Target& t, const std::string& who) {
   plaidgpu_ctx* c = ctxs[0];
-  const std::string who(name);
-  {
-    const int rcc = check_shard_ctxs(ctxs, n, opts, who);
-    if (rcc) return rcc;
-  }
-  const int32_t* labels = reduce ? reduce->labels : nullptr;
   try {
     const int64_t N = X->N;
     const int32_t S = c->S, P = X->P;
-    const bool norm = (opts->scorer == PLAIDGPU_PLAID && opts->normalize) || opts->scorer == PLAIDGPU_SSGSEA ||
-                      opts->scorer == PLAIDGPU_UCELL || opts->scorer == PLAIDGPU_AUCELL || opts->scorer == PLAIDGPU_GSVA;
+    const bool norm = needs_norm(*opts);
     const bool gsva_z = opts->scorer == PLAIDGPU_GSVA && opts->gsva_ecdf == PLAIDGPU_ROWTF_Z && !(opts->row_mean && opts->row_sd);
     std::vector<int64_t> lo((size_t)n + 1);
     for (int r = 0; r <= n; ++r) lo[r] = N * r / n;
     std::vector<std::vector<int32_t>> pbuf((size_t)n);
-    std::vector<plaidgpu_matrix> M((size_t)n, *X);
-    for (int r = 0; r < n; ++r) {
-      M[r].N = lo[r + 1] - lo[r];
-      if (X->kind == PLAIDGPU_CSC) {
-        const int32_t base = X->p[lo[r]];
-        pbuf[r].resize((size_t)M[r].N + 1);
-        for (int64_t j = lo[r]; j <= lo[r + 1]; ++j) pbuf[r][(size_t)(j - lo[r])] = X->p[j] - base;
-        M[r].p = pbuf[r].data();
-        M[r].i = X->i + base;
-        M[r].x = X->x + base;
-      } else {
-        M[r].x = X->x + lo[r] * (int64_t)P;
-      }
-    }
+    std::vector<plaidgpu_matrix> M((size_t)n);
+    for (int r = 0; r < n; ++r) M[r] = column_slice(X, lo[r], lo[r + 1], pbuf[r]);
     std::vector<plaidgpu_scalars> loc((size_t)n);
     std::vector<int> rc((size_t)n, PLAIDGPU_OK);
-    const size_t width = labels ? (size_t)reduce->K * 2 * (size_t)S : 0;
-    std::vector<std::vector<double>> moments(labels ? (size_t)n : 0, std::vector<double>(width));
+    const size_t width = t.kind == Target::GROUP_STATS ? (size_t)t.K * 2 * (size_t)S : 0;
+    std::vector<std::vector<double>> moments((size_t)n, std::vector<double>(width));
     std::vector<double> med((size_t)std::max<int64_t>(N, 1));
     std::vector<std::vector<double>> part(gsva_z ? (size_t)n : 0, std::vector<double>((size_t)P));
     std::vector<double> rmean(gsva_z ? (size_t)P : 0), rsd(gsva_z ? (size_t)P : 0);
@@ -2403,8 +2352,9 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
     auto body = [&](int r) {
       plaidgpu_ctx* cr = ctxs[r];
       plaidgpu_opts o = *opts;
-      if (reduce) o.out_location = PLAIDGPU_HOST;  // raw scores stay in the context's device buffer
-      double* dst = reduce ? nullptr : out + lo[r] * (int64_t)S;
+      if (t.kind != Target::SCORES) o.out_location = PLAIDGPU_HOST;  // raw scores stay in the context's device buffer
+      const Target tr = t.from(lo[r], S, moments[r].data());
+      double* dst = t.kind == Target::SCORES ? tr.out : nullptr;
       if (gsva_z) {  // rowMeans / rowSds over ALL shards, summed in shard order (R/plaid.R:343)
         rc[r] = plaidgpu_row_moments(cr, &M[r], nullptr, part[r].data());
         bar.wait();
@@ -2456,8 +2406,7 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
         s.med_mean = g.med_mean;
         s.score_min = smin;
       }
-      rc[r] = reduce ? finish_into(cr, &s, *reduce, lo[r], labels ? moments[r].data() : nullptr)
-                     : plaidgpu_score_finish(cr, &s, dst);
+      rc[r] = score_finish(cr, &s, tr);
     };
     std::vector<std::thread> th;
     for (int r = 1; r < n; ++r) th.emplace_back(body, r);
@@ -2468,10 +2417,10 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
         if (r > 0) c->err = "shard " + std::to_string(r) + ": " + ctxs[r]->err;
         return rc[r];
       }
-    if (labels) {
-      std::copy(moments[0].begin(), moments[0].end(), out);
+    if (t.kind == Target::GROUP_STATS) {
+      std::copy(moments[0].begin(), moments[0].end(), t.out);
       for (int r = 1; r < n; ++r)
-        for (size_t i = 0; i < width; ++i) out[i] += moments[r][i];
+        for (size_t i = 0; i < width; ++i) t.out[i] += moments[r][i];
     }
     return PLAIDGPU_OK;
   } catch (const std::bad_alloc&) {
@@ -2481,15 +2430,33 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
   }
 }
 
+// The multi-context entry points after their own argument checks: X in host memory, then the contexts (n > 1, so bad
+// contexts fail whatever N is), then the single-device entry point on ctxs[0] (n == 1 or N < 2n) or the shards
+static int score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
+                       const plaidgpu_opts* opts, const Target& t, const char* name) {
+  plaidgpu_ctx* c = ctxs[0];
+  const std::string who(name);
+  if (t.kind == Target::SCORES && (X->location != PLAIDGPU_HOST || opts->out_location != PLAIDGPU_HOST))
+    return fail(c, PLAIDGPU_ERR_ARG, who + ": X and out must be in host memory");
+  if (X->location != PLAIDGPU_HOST) return fail(c, PLAIDGPU_ERR_ARG, who + ": X must be in host memory");
+  int rc = n > 1 ? check_shard_ctxs(ctxs, n, opts, who) : PLAIDGPU_OK;
+  if (rc) return rc;
+  if (n == 1 || X->N < 2 * (int64_t)n) {
+    if (t.kind == Target::GROUP_STATS) return plaidgpu_score_group_stats(c, X, rowmap, opts, t.labels, t.K, t.out);
+    if (t.kind == Target::TOPK) return plaidgpu_score_topk(c, X, rowmap, opts, t.k, t.decreasing, t.idx, t.val);
+    return plaidgpu_score(c, X, rowmap, opts, t.out);
+  }
+  if (t.kind == Target::GROUP_STATS) rc = check_groups(c, t.labels, X->N, t.K);
+  if (t.kind == Target::TOPK) rc = check_topk(c, c->S, t.k);
+  if (rc) return rc;
+  return score_multi_impl(ctxs, n, X, rowmap, opts, t, who);
+}
+
 int plaidgpu_score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
                          const plaidgpu_opts* opts, double* out) try {
   if (!ctxs || n <= 0 || !ctxs[0]) return PLAIDGPU_ERR_ARG;
-  plaidgpu_ctx* c = ctxs[0];
-  if (!X || !rowmap || !opts) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
-  if (X->location != PLAIDGPU_HOST || opts->out_location != PLAIDGPU_HOST)
-    return fail(c, PLAIDGPU_ERR_ARG, "plaidgpu_score_multi: X and out must be in host memory");
-  if (n == 1 || X->N < 2 * (int64_t)n) return plaidgpu_score(c, X, rowmap, opts, out);
-  return score_multi_impl(ctxs, n, X, rowmap, opts, out, nullptr, "plaidgpu_score_multi");
+  if (!X || !rowmap || !opts) return fail(ctxs[0], PLAIDGPU_ERR_ARG, "null argument");
+  return score_multi(ctxs, n, X, rowmap, opts, Target::scores(out), "plaidgpu_score_multi");
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {
@@ -2499,14 +2466,8 @@ int plaidgpu_score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix
 int plaidgpu_score_group_stats_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
                                      const plaidgpu_opts* opts, const int32_t* labels, int K, double* out) try {
   if (!ctxs || n <= 0 || !ctxs[0]) return PLAIDGPU_ERR_ARG;
-  plaidgpu_ctx* c = ctxs[0];
-  if (!X || !rowmap || !opts || !out) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
-  if (X->location != PLAIDGPU_HOST) return fail(c, PLAIDGPU_ERR_ARG, "plaidgpu_score_group_stats_multi: X must be in host memory");
-  if (n == 1 || X->N < 2 * (int64_t)n) return plaidgpu_score_group_stats(c, X, rowmap, opts, labels, K, out);
-  int rc = check_groups(c, labels, X->N, K);
-  if (rc) return rc;
-  const ScoreSink sk{labels, K, 0, 0, nullptr, nullptr};
-  return score_multi_impl(ctxs, n, X, rowmap, opts, out, &sk, "plaidgpu_score_group_stats_multi");
+  if (!X || !rowmap || !opts || !out) return fail(ctxs[0], PLAIDGPU_ERR_ARG, "null argument");
+  return score_multi(ctxs, n, X, rowmap, opts, Target::group_stats(labels, K, out), "plaidgpu_score_group_stats_multi");
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {
@@ -2516,18 +2477,8 @@ int plaidgpu_score_group_stats_multi(plaidgpu_ctx* const* ctxs, int n, const pla
 int plaidgpu_score_topk_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
                               const plaidgpu_opts* opts, int k, int decreasing, int32_t* idx, double* val) try {
   if (!ctxs || n <= 0 || !ctxs[0]) return PLAIDGPU_ERR_ARG;
-  plaidgpu_ctx* c = ctxs[0];
-  if (!X || !rowmap || !opts || !idx || !val) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
-  if (X->location != PLAIDGPU_HOST) return fail(c, PLAIDGPU_ERR_ARG, "plaidgpu_score_topk_multi: X must be in host memory");
-  if (n > 1) {  // also when the columns are too few to split: the same arguments fail whatever N is
-    int rc = check_shard_ctxs(ctxs, n, opts, "plaidgpu_score_topk_multi");
-    if (rc) return rc;
-  }
-  if (n == 1 || X->N < 2 * (int64_t)n) return plaidgpu_score_topk(c, X, rowmap, opts, k, decreasing, idx, val);
-  int rc = check_topk(c, c->S, k);
-  if (rc) return rc;
-  const ScoreSink sk{nullptr, 0, k, decreasing != 0, idx, val};
-  return score_multi_impl(ctxs, n, X, rowmap, opts, nullptr, &sk, "plaidgpu_score_topk_multi");
+  if (!X || !rowmap || !opts || !idx || !val) return fail(ctxs[0], PLAIDGPU_ERR_ARG, "null argument");
+  return score_multi(ctxs, n, X, rowmap, opts, Target::topk(k, decreasing, idx, val), "plaidgpu_score_topk_multi");
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {

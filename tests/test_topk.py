@@ -231,6 +231,15 @@ def test_bad_arguments_are_rejected(small_case, gpu_ctx):
     assert lib.plaidgpu_score_topk_multi(hs, 2, *args, ti.ctypes.data, tv.ctypes.data) == L.ERR_ARG
     assert lib.plaidgpu_score_topk_multi(hs, 2, None, rowmap.ctypes.data, C.byref(o), 5, 1, ti.ctypes.data,
                                          tv.ctypes.data) == L.ERR_ARG
+    # every multi-context entry point rejects the same context twice also with too few columns to split (N < 2n)
+    M3 = _matrix_struct(Xn.mat[:, :3], keep)
+    out3 = np.empty((S, 3), order="F")
+    lab3 = np.zeros(3, dtype=np.int32)
+    mom = np.empty((2, 2, S))
+    args3 = (C.byref(M3), rowmap.ctypes.data, C.byref(o))
+    assert lib.plaidgpu_score_multi(hs, 2, *args3, out3.ctypes.data) == L.ERR_ARG
+    assert lib.plaidgpu_score_group_stats_multi(hs, 2, *args3, lab3.ctypes.data, 2, mom.ctypes.data) == L.ERR_ARG
+    assert lib.plaidgpu_score_topk_multi(hs, 2, *args3, 5, 1, ti.ctypes.data, tv.ctypes.data) == L.ERR_ARG
     other = pb.Context(0)
     other.set_genesets(Gn.mat)
     hs = (C.c_void_p * 2)(gpu_ctx.h, other.h)
@@ -239,3 +248,13 @@ def test_bad_arguments_are_rejected(small_case, gpu_ctx):
                                          tv.ctypes.data) == L.ERR_ARG
     # and a good call still works on this context afterwards
     assert lib.plaidgpu_score_topk(gpu_ctx.h, *args, ti.ctypes.data, tv.ctypes.data) == L.OK
+    # after the fused calls, begin / compute / finish on the same context returns the scores themselves
+    from plaid_b200 import sharded
+    want = pb.plaid(Xn, Gn, ctx=other).mat
+    lab = np.zeros(N, dtype=np.int32)
+    mom = np.empty((2, 2, S))
+    assert lib.plaidgpu_score_group_stats(gpu_ctx.h, *args[:3], lab.ctypes.data, 2, mom.ctypes.data) == L.OK
+    assert lib.plaidgpu_score_topk(gpu_ctx.h, *args, ti.ctypes.data, tv.ctypes.data) == L.OK
+    got = np.empty((S, N), order="F")
+    sharded.score_shard(gpu_ctx, sharded.ThreadComm.group(1)[0], M, rowmap, o, got.ctypes.data, N)
+    assert np.array_equal(got.view(np.int64), want.view(np.int64))
