@@ -6,13 +6,12 @@
 //   * the cells are cut into tiles of TAIL_C columns; per tile the tail entries of X are regrouped GENE-major
 //     (k_tile_scan / k_tile_place: counting sort by tail row -> `rowptr` and 8-byte records `ent` = {value in the
 //     column's fixed point (the same 2^e_j the tensor-core pass uses, int32), cell inside the tile});
-//   * one warp owns one (tile, set) item at a time: it walks the set's tail members and adds each member's
-//     sparse row of the tile into TAIL_C accumulators in shared memory, LANES = the row's ENTRIES.  The cells
-//     of one row are distinct, and rows are handled one after the other, so there are no duplicate addresses
-//     inside a step: no tags, no retries, no atomics — a step is one 32-bit LDS / IADD / STS per lane;
-//   * accumulators are 64-bit integers split into a u32 low word (touched by every add) and an i16 high word
-//     (touched only on carry / borrow): random 32-bit accesses cost ~3 shared-memory wavefronts per warp
-//     instead of the ~6 of a 64-bit access, and integer sums are exact and order-independent;
+//   * one warp owns one (tile, set) item at a time: it walks the set's tail members 32 at a time, concatenates
+//     their sparse rows of the tile into one stream and adds it 32 entries per step (LANES = ENTRIES, whatever
+//     row each belongs to) into TAIL_C accumulators in shared memory;
+//   * accumulators are 64-bit integers split into a u32 low word (a shared-memory atomic on every add) and a
+//     16-bit high counter (a second atomic only on carry / borrow, see acc_add): lanes of one step may hit the
+//     same cell, and integer sums are exact and order-independent;
 //   * the finished row (TAIL_C sums of one set) is written as int64 to `tmp[set][cell]` with coalesced stores;
 //     the tensor-core kernel fetches its 128 sets x 48 cells by TMA and adds it to its own integer sums
 //     before the one conversion to fp64 (so tail + block is exact, then scaled by 2^-e_j).
@@ -132,6 +131,29 @@ __global__ void __launch_bounds__(256) k_fill_u32(uint32_t* __restrict__ p, uint
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) p[i] = v;
 }
 
+// One addend {q, cell} into a 64-bit accumulator kept as a u32 low word and a 16-bit high counter.  The low word
+// takes a shared-memory atomic that returns the old value; the high counter moves by d = carry out of the low word
+// minus the sign extension of q (-1, 0 or +1), through a no-return atomic on the lane's own predicate.  Every
+// atomic sees a consistent old value, so (hi << 32) + lo is the exact int64 sum whatever order the adds land in,
+// and lanes of one step may share a cell.
+// There are no 16-bit atomics: the counters of cells 2i and 2i + 1 are the two halves of hiw[i], each biased by
+// 2^15 so that a borrow never reaches the other half.  A set has fewer than 2^16 tail members (tail ids are u16)
+// and each adds at most one entry to a cell, |q| < 2^30, so every partial sum of a cell lies in (-2^46, 2^46) and
+// its high word in [-2^14, 2^14); the counter runs ahead of or behind that by the few adds of one warp whose
+// second atomic has not landed yet, far inside the 2^15 either side that the bias allows.
+constexpr uint32_t HI_BIAS = 0x8000u, HI_BIAS2 = 0x80008000u;
+
+__device__ __forceinline__ void acc_add(uint32_t lo_sa, uint32_t hi_sa, const uint2 rec) {
+  const uint32_t q = rec.x, c = rec.y;
+  uint32_t old, d;
+  asm volatile("atom.shared.add.u32 %0, [%1], %2;" : "=r"(old) : "r"(lo_sa + c * 4u), "r"(q) : "memory");
+  asm("{\n\t.reg .u32 t;\n\tadd.cc.u32 t, %1, %2;\n\taddc.u32 %0, %3, 0;\n\t}"  // d = carry + (q >> 31)
+      : "=r"(d) : "r"(old), "r"(q), "r"((uint32_t)((int32_t)q >> 31)));
+  // d << 16 * (c & 1): the funnel shift takes its amount modulo 32
+  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %1, 0;\n\t@p red.shared.add.u32 [%0], %2;\n\t}"
+               ::"r"(hi_sa + (c & ~1u) * 2u), "r"(d), "r"(__funnelshift_l(0u, d, c << 4)) : "memory");
+}
+
 struct TailParams {
   const uint32_t* tptr;    // [S + 1] set -> its tail members
   const uint16_t* tidx;    // tail ids, ascending inside a set
@@ -151,14 +173,21 @@ __global__ void __launch_bounds__(TAIL_WARPS * 32, 1) k_tail(const TailParams p)
   extern __shared__ uint32_t tail_sm[];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int C = p.C;
+  // cell c: low word lo[c], high counter in half c & 1 of hiw[c >> 1], biased by 2^15 (see acc_add); scr: the
+  // non-empty rows of a member batch
   uint32_t* __restrict__ lo = tail_sm + (size_t)w * C;
-  short* __restrict__ hi = reinterpret_cast<short*>(tail_sm + (size_t)TAIL_WARPS * C) + (size_t)w * C;
-  for (int c = lane; c < C; c += 32) {
-    lo[c] = 0u;
-    hi[c] = 0;
+  uint32_t* __restrict__ hiw = tail_sm + (size_t)TAIL_WARPS * C + (size_t)w * (C / 2);
+  uint2* __restrict__ scr = reinterpret_cast<uint2*>(tail_sm + (size_t)TAIL_WARPS * C * 3 / 2) + w * 32;
+  for (int c = lane; c < C / 2; c += 32) {
+    lo[2 * c] = 0u;
+    lo[2 * c + 1] = 0u;
+    hiw[c] = HI_BIAS2;
   }
   __syncwarp();
-  const uint32_t lo_sa = (uint32_t)__cvta_generic_to_shared(lo), hi_sa = (uint32_t)__cvta_generic_to_shared(hi);
+  const uint32_t lo_sa = (uint32_t)__cvta_generic_to_shared(lo), hi_sa = (uint32_t)__cvta_generic_to_shared(hiw);
+  uint32_t le, lt;
+  asm("mov.u32 %0, %%lanemask_le;" : "=r"(le));
+  asm("mov.u32 %0, %%lanemask_lt;" : "=r"(lt));
   const unsigned nitems = (unsigned)p.tiles * (unsigned)p.S;
   for (;;) {
     unsigned item = 0;
@@ -172,7 +201,8 @@ __global__ void __launch_bounds__(TAIL_WARPS * 32, 1) k_tail(const TailParams p)
     for (int u = lane; u < t; u += 32) base += p.total[u];
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) base += __shfl_xor_sync(FULL, base, o);
-    const uint2* __restrict__ ent = p.ent + base;
+    const uint2* ent = p.ent + base + lane;
+    asm("mov.b64 %0, %0;" : "+l"(ent));  // keeps the lane's base address in a register: one IMAD.WIDE per load
     const uint32_t m0 = p.tptr[s], m1 = p.tptr[s + 1];
     for (uint32_t mb = m0; mb < m1; mb += 32) {
       // lane i looks up the row of member mb + i in this tile
@@ -182,81 +212,63 @@ __global__ void __launch_bounds__(TAIL_WARPS * 32, 1) k_tail(const TailParams p)
         r0 = rp[g];
         rn = rp[g + 1] - r0;
       }
-      const int cnt = (int)min(32u, m1 - mb);
-      // member k's row: segments of 32 entries, lanes = entries.  The first segments of the next four members are
-      // in flight while a member is added (entries come from L2, ~350 clocks away; most rows are one segment)
-      auto add = [&](const uint2 rec) {
-        if (rec.y != 0xFFFFu) {
-          const uint32_t a = lo_sa + rec.y * 4u;
-          uint32_t old;
-          asm volatile("ld.shared.u32 %0, [%1];" : "=r"(old) : "r"(a) : "memory");
-          const uint32_t nv = old + rec.x;
-          asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(nv) : "memory");
-          // carry out of the low word vs. sign extension of the addend: equal -> the high word keeps its value
-          if ((nv < rec.x) != ((int32_t)rec.x < 0)) {
-            const uint32_t ah = hi_sa + rec.y * 2u;
-            short hv;
-            asm volatile("ld.shared.s16 %0, [%1];" : "=h"(hv) : "r"(ah) : "memory");
-            hv = (short)(hv + ((nv < rec.x) ? 1 : -1));
-            asm volatile("st.shared.s16 [%0], %1;" ::"r"(ah), "h"(hv) : "memory");
-          }
-        }
-        __syncwarp();
+      // the rows of the 32 members, concatenated, form one stream of `total` entries cut into 32-entry segments:
+      // lane l of a segment starting at stream position P0 adds entry P0 + l, whatever row it belongs to
+      uint32_t incl = rn;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t v = __shfl_up_sync(FULL, incl, o);
+        if (lane >= o) incl += v;
+      }
+      const uint32_t total = __shfl_sync(FULL, incl, 31);
+      if (total == 0u) continue;
+      // compact the non-empty rows (an empty row would share its start with the next one): lane k holds the k-th
+      // non-empty row's start in the stream and its offset in `ent` relative to that start
+      const uint32_t ne = __ballot_sync(FULL, rn != 0u);
+      __syncwarp();  // the previous batch has read scr
+      if (rn != 0u) scr[__popc(ne & lt)] = make_uint2(incl - rn, r0 - (incl - rn));
+      __syncwarp();
+      const uint2 so = scr[lane];
+      const uint32_t start = (uint32_t)lane < (uint32_t)__popc(ne) ? so.x : 0xFFFFFFFFu, off = so.y;
+      // rows that start before the current segment, minus one
+      int before = -1;
+      // the row of each lane's entry: the rows starting inside the segment (one OR over the lanes), counted up to
+      // the lane, after the `before` rows that started earlier
+      auto fetch = [&](uint32_t P0) {
+        uint32_t bit;  // PTX shl yields 0 for a shift of 32 or more
+        asm("shl.b32 %0, 1, %1;" : "=r"(bit) : "r"(start - P0));
+        const uint32_t m = __reduce_or_sync(FULL, bit);
+        const uint32_t o = __shfl_sync(FULL, off, before + __popc(m & le));
+        before += __popc(m);
+        uint2 rec = make_uint2(0u, (uint32_t)lane);  // padding: adds 0, each lane at its own cell
+        if (P0 + lane < total) rec = __ldg(ent + (o + P0));
+        return rec;
       };
-      auto prefetch = [&](int kk, uint2& rec, uint32_t& nk, uint32_t& pk) {
-        nk = kk < cnt ? __shfl_sync(FULL, rn, kk & 31) : 0u;
-        pk = __shfl_sync(FULL, r0, kk & 31);
-        rec = make_uint2(0u, 0xFFFFu);
-        if ((uint32_t)lane < nk) rec = __ldg(ent + pk + lane);
-      };
-      auto seg = [&](uint32_t off, uint32_t nk, uint32_t pk) {
-        uint2 r = make_uint2(0u, 0xFFFFu);
-        if (off + lane < nk) r = __ldg(ent + pk + off + lane);
-        return r;
-      };
-      auto member = [&](const uint2 rec, uint32_t nk, uint32_t pk) {
-        if (nk <= 32u) {  // warp-uniform
-          add(rec);
-          return;
-        }
-        // long row (a highly expressed gene in few sets): its entries are one contiguous stream — three segments in
-        // flight while three are added, so the L2 latency is paid once per 96 entries instead of once per 32
-        uint2 q1 = seg(32u, nk, pk), q2 = seg(64u, nk, pk), q3 = seg(96u, nk, pk);
-        add(rec);
-        for (uint32_t off = 32; off < nk; off += 96) {
-          const uint2 a = q1, b = q2, c = q3;
-          q1 = seg(off + 96u, nk, pk);
-          q2 = seg(off + 128u, nk, pk);
-          q3 = seg(off + 160u, nk, pk);
-          add(a);
-          if (off + 32u < nk) add(b);
-          if (off + 64u < nk) add(c);
-        }
-      };
-      uint2 e0, e1, e2, e3;
-      uint32_t n0, n1, n2, n3, p0, p1, p2, p3;
-      prefetch(0, e0, n0, p0);
-      prefetch(1, e1, n1, p1);
-      prefetch(2, e2, n2, p2);
-      prefetch(3, e3, n3, p3);
-      for (int k = 0; k < cnt; k += 4) {
-        member(e0, n0, p0);
-        prefetch(k + 4, e0, n0, p0);
-        member(e1, n1, p1);
-        prefetch(k + 5, e1, n1, p1);
-        member(e2, n2, p2);
-        prefetch(k + 6, e2, n2, p2);
-        member(e3, n3, p3);
-        prefetch(k + 7, e3, n3, p3);
+      // three segments in flight while one is added: entries come from L2, ~350 clocks away
+      uint2 q0 = fetch(0u), q1 = fetch(32u), q2 = fetch(64u);
+      for (uint32_t P0 = 0;; P0 += 96u) {
+        acc_add(lo_sa, hi_sa, q0);
+        q0 = fetch(P0 + 96u);
+        if (P0 + 32u >= total) break;
+        acc_add(lo_sa, hi_sa, q1);
+        q1 = fetch(P0 + 128u);
+        if (P0 + 64u >= total) break;
+        acc_add(lo_sa, hi_sa, q2);
+        q2 = fetch(P0 + 160u);
+        if (P0 + 96u >= total) break;
       }
     }
-    // flush: int64 sums of set s over the tile's cells, coalesced; re-zero
+    // flush: int64 sums of set s over the tile's cells, two cells per lane, coalesced; re-zero
+    __syncwarp();
     long long* __restrict__ o = p.tmp + (size_t)s * p.ld + (size_t)t * C;
-    for (int c = lane; c < C; c += 32) {
-      const long long v = ((long long)hi[c] << 32) | (long long)lo[c];
-      lo[c] = 0u;
-      hi[c] = 0;
-      __stcs(o + c, v);
+    for (int c = lane; c < C / 2; c += 32) {
+      const uint2 l = *reinterpret_cast<const uint2*>(lo + 2 * c);
+      const uint32_t h = hiw[c];
+      const long long v0 = (long long)(((uint64_t)(h & 0xFFFFu) - HI_BIAS) << 32) + l.x;
+      const long long v1 = (long long)(((uint64_t)(h >> 16) - HI_BIAS) << 32) + l.y;
+      *reinterpret_cast<uint2*>(lo + 2 * c) = make_uint2(0u, 0u);
+      hiw[c] = HI_BIAS2;
+      __stcs(reinterpret_cast<longlong2*>(o + 2 * c), make_longlong2(v0, v1));
     }
     __syncwarp();
   }
@@ -274,7 +286,7 @@ cudaError_t launch_fill_u32(void* p, uint32_t v, int64_t n, cudaStream_t st) {
 
 int tail_tile_cells() { return 1056; }  // 22 tensor-core cell tiles of 48
 
-size_t tail_smem_bytes() { return (size_t)TAIL_WARPS * tail_tile_cells() * 6; }
+size_t tail_smem_bytes() { return (size_t)TAIL_WARPS * (tail_tile_cells() * 6 + 32 * sizeof(uint2)); }
 
 cudaError_t launch_tile_scan(uint32_t* cnt, int32_t Pt, int tiles, uint32_t* rowptr, uint32_t* total, cudaStream_t st) {
   if (tiles <= 0) return cudaSuccess;
