@@ -299,6 +299,32 @@ int plaidgpu_score_group_stats(plaidgpu_ctx* ctx, const plaidgpu_matrix* X, cons
 int plaidgpu_score_group_stats_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
                                      const plaidgpu_opts* opts, const int32_t* labels, int K, double* out);
 
+/* Per gene set the products of its scores with the columns of a dense design basis, and its sum and sum of squares:
+ * the reductions behind plaid.lm (ordinary least squares of every set's scores on a design; the host takes a thin
+ * QR D = U R of the design and passes B = U).  x: S x N column-major doubles at `location`; B: host double,
+ * column-major N x Q (ld = N); 1 <= Q <= 64, every entry finite.  out: host double[(Q + 2) * S] =
+ * {sum_j x[s,j]*B[j,q] for q < Q [S each], sum_j x[s,j] [S], sum_j x[s,j]^2 [S]}.  Columns are added in a fixed
+ * order: bit-reproducible.  Q outside [1, 64], a null pointer or a non-finite entry of B is PLAIDGPU_ERR_ARG.
+ * Kernel time: plaidgpu_last_kernel_ms(ctx, 2). */
+int plaidgpu_design_stats(plaidgpu_ctx* ctx, const double* x, int32_t S, int64_t N, const double* B, int Q,
+                          int location, double* out);
+
+/* The same reductions fused onto the scoring call, for any scorer and option plaidgpu_score accepts: the scores stay
+ * on the device as raw scores and are normalised in registers while reducing; (Q + 2) * S doubles come back (layout
+ * as above, B has X->N rows).  Equal, bit for bit, to plaidgpu_score followed by plaidgpu_design_stats.  When X is in
+ * host memory and the S x N scores exceed the device, the columns are scored in tiles (two passes over X when
+ * normalised, like plaidgpu_score), each tile uploads only its own rows of B, and the tiles' moments are added in
+ * tile order. */
+int plaidgpu_score_design_stats(plaidgpu_ctx* ctx, const plaidgpu_matrix* X, const int32_t* rowmap,
+                                const plaidgpu_opts* opts, const double* B, int Q, double* out);
+
+/* plaidgpu_score_design_stats over n devices from ONE host process, split like plaidgpu_score_multi: shard r reduces
+ * its own scores with rows [lo_r, hi_r) of B and the shards' moments are added in shard order.  Each shard's scores
+ * must fit its device.  The same context twice, or gsva rowtf = "ecdf" with n > 1, is PLAIDGPU_ERR_ARG. */
+int plaidgpu_score_design_stats_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X,
+                                      const int32_t* rowmap, const plaidgpu_opts* opts, const double* B, int Q,
+                                      double* out);
+
 /* Per column of a dense S x N matrix at `location`: the k largest (decreasing = 1) or smallest values and their row
  * indices, i.e. the first k entries of R's order(v, decreasing = decreasing): ties (fp64 ==, so -0 == +0) by
  * ascending row, NaN last in both directions and by ascending row.  idx int32[k * N] (0-based rows) and val

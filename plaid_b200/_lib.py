@@ -63,6 +63,12 @@ SYMBOLS = {
     "plaidgpu_colranks": (C.c_int, [C.c_void_p, C.POINTER(Matrix), C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "plaidgpu_group_moments": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_int, C.c_void_p]),
     "plaidgpu_group_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "plaidgpu_design_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_int, C.c_int,
+                                        C.c_void_p]),
+    "plaidgpu_score_design_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                              C.c_void_p]),
+    "plaidgpu_score_design_stats_multi": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                    C.c_void_p, C.c_int, C.c_void_p]),
     "plaidgpu_col_topk": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                     C.c_void_p]),
     "plaidgpu_normalize_medians": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int, C.c_int, C.c_void_p]),

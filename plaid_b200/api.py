@@ -544,30 +544,34 @@ def score_group_stats(X: NamedMatrix, matG: NamedMatrix, labels, K=None, *, ctx=
     return out
 
 
+def _dense_input(gsetX):
+    """(S, N, location, pointer, keep) of a dense S x N matrix given as a 2-D array or a DeviceDense"""
+    if isinstance(gsetX, DeviceDense):
+        S, N = (int(d) for d in gsetX.shape)
+        if gsetX.x.numel() != S * N:
+            raise ValueError("DeviceDense: the tensor does not hold shape[0] * shape[1] values")
+        return S, N, L.DEVICE, gsetX.x.data_ptr(), gsetX
+    if _is_torch(gsetX):
+        raise TypeError("pass dense device matrices as DeviceDense(t_colmajor, shape)")
+    a = np.asarray(gsetX, dtype=np.float64)
+    if a.ndim != 2:
+        raise ValueError("gsetX must be a matrix (S x N)")
+    a = np.asfortranarray(a)
+    return a.shape[0], a.shape[1], L.HOST, a.ctypes.data, a
+
+
 def col_topk(gsetX, k=10, decreasing=True, *, ctx=None):
     """Per column of a dense S x N matrix: the first k entries of R's `order(v, decreasing = decreasing)`, i.e. the
     k largest (or smallest) values with ties by ascending row and NaN last (`plaidgpu_col_topk`).  `gsetX` is a 2-D
     array or a `DeviceDense` (S x N in device memory).  Returns (idx, val) of shape (k, N): 0-based row indices
     (int32) and the values at those rows, bit for bit."""
     ctx = ctx or default_context()
-    if isinstance(gsetX, DeviceDense):
-        S, N = (int(d) for d in gsetX.shape)
-        if gsetX.x.numel() != S * N:
-            raise ValueError("DeviceDense: the tensor does not hold shape[0] * shape[1] values")
-        loc, ptr = L.DEVICE, gsetX.x.data_ptr()
-    else:
-        if _is_torch(gsetX):
-            raise TypeError("pass dense device matrices as DeviceDense(t_colmajor, shape)")
-        a = np.asarray(gsetX, dtype=np.float64)
-        if a.ndim != 2:
-            raise ValueError("gsetX must be a matrix (S x N)")
-        a = np.asfortranarray(a)
-        S, N = a.shape
-        loc, ptr = L.HOST, a.ctypes.data
+    S, N, loc, ptr, keep = _dense_input(gsetX)
     idx = np.empty((max(int(k), 0), N), dtype=np.int32, order="F")  # a bad k is the library's error
     val = np.empty((max(int(k), 0), N), dtype=np.float64, order="F")
     ctx.check(ctx.lib.plaidgpu_col_topk(ctx.h, ptr, S, N, int(k), 1 if decreasing else 0, loc, idx.ctypes.data,
                                         val.ctypes.data))
+    del keep
     return idx, val
 
 
@@ -607,6 +611,184 @@ def score_topk(X: NamedMatrix, matG: NamedMatrix, k=10, decreasing=True, *, ctx=
         return None
     ctx.check(rc)
     return idx, val
+
+
+def _design_basis(B, n):
+    b = np.asarray(B, dtype=np.float64)
+    if b.ndim == 1:
+        b = b[:, None]
+    if b.ndim != 2 or b.shape[0] != n:
+        raise ValueError("nrow(B) must equal ncol(X)")
+    return np.asfortranarray(b)  # a bad Q or a non-finite entry is the library's error
+
+
+def design_stats(gsetX, B, *, ctx=None):
+    """Per row s of a dense S x N matrix x: sum_j x[s, j] * B[j, q] for every column q of the N x Q matrix B
+    (1 <= Q <= 64, finite), then sum_j x[s, j] and sum_j x[s, j]^2 (`plaidgpu_design_stats`): the reductions behind
+    plaid_lm, one pass over x.  `gsetX` is a 2-D array or a `DeviceDense`.  Returns an array of shape (Q + 2, S)."""
+    ctx = ctx or default_context()
+    S, N, loc, ptr, keep = _dense_input(gsetX)
+    b = _design_basis(B, N)
+    out = np.empty((b.shape[1] + 2, S), dtype=np.float64)
+    ctx.check(ctx.lib.plaidgpu_design_stats(ctx.h, ptr, S, N, b.ctypes.data, b.shape[1], loc, out.ctypes.data))
+    del keep
+    return out
+
+
+def score_design_stats(X: NamedMatrix, matG: NamedMatrix, B, *, ctx=None, **opts_kw):
+    """plaid() (or another scorer through `opts_kw`) fused with design_stats (`plaidgpu_score_design_stats`): the S x N
+    scores stay on the device, (Q + 2) x S doubles come back.  B: N x Q, one row per column of X.  `ctx` may be a list
+    of Contexts on different devices: the columns are then split over them (`plaidgpu_score_design_stats_multi`).
+    Returns an array of shape (Q + 2, S), or None on no overlap."""
+    ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else None
+    ctx = (ctxs[0] if ctxs else ctx) or default_context()
+    if X.rownames is None or matG.rownames is None:
+        _message("[plaid] ERROR. No overlapping features.")
+        return None
+    rowmap = make_rowmap(X.rownames, matG.rownames)
+    if not (rowmap >= 0).any():
+        _message("[plaid] ERROR. No overlapping features.")
+        return None
+    for cx in (ctxs or [ctx]):
+        cx.set_genesets(matG.mat)
+    keep: list = []
+    M = _matrix_struct(X.mat, keep)
+    b = _design_basis(B, M.N)
+    kw = dict(scorer=L.PLAID, stats_mean=1, normalize=1)
+    kw.update(opts_kw)
+    o = _opts(ctx.lib, **kw)
+    out = np.empty((b.shape[1] + 2, int(matG.mat.shape[1])), dtype=np.float64)
+    if ctxs and len(ctxs) > 1:
+        hs = (C.c_void_p * len(ctxs))(*[cx.h for cx in ctxs])
+        rc = ctx.lib.plaidgpu_score_design_stats_multi(hs, len(ctxs), C.byref(M), rowmap.ctypes.data, C.byref(o),
+                                                       b.ctypes.data, b.shape[1], out.ctypes.data)
+    else:
+        rc = ctx.lib.plaidgpu_score_design_stats(ctx.h, C.byref(M), rowmap.ctypes.data, C.byref(o), b.ctypes.data,
+                                                 b.shape[1], out.ctypes.data)
+    if rc == L.ERR_NOOVERLAP:
+        _message("[plaid] ERROR. No overlapping features.")
+        return None
+    ctx.check(rc)
+    return out
+
+
+LM_COLUMNS = ["logFC", "SE", "AveExpr", "t", "P.Value", "adj.P.Val"]
+
+
+def design_qr(design):
+    """Thin QR D = U R of an N x Q design (U: N x Q with orthonormal columns, R: Q x Q upper triangular).  Raises
+    ValueError for a non-finite entry, Q outside [1, 64], or a design that is not of full column rank (a column whose
+    part orthogonal to the columns before it is below 1e-7 of its norm, the tolerance of R's qr())."""
+    D = np.asarray(design, dtype=np.float64)
+    if D.ndim == 1:
+        D = D[:, None]
+    if D.ndim != 2 or not 1 <= D.shape[1] <= 64:
+        raise ValueError("the design must be a matrix with 1 to 64 columns")
+    if not np.all(np.isfinite(D)):
+        raise ValueError("the design must be finite (no NA)")
+    if D.shape[0] < D.shape[1]:
+        raise ValueError("the design is not of full column rank")
+    U, R = np.linalg.qr(D)
+    if np.any(np.abs(np.diag(R)) <= 1e-7 * np.linalg.norm(D, axis=0)):
+        raise ValueError("the design is not of full column rank")
+    return U, R
+
+
+def _bh(p):
+    """p.adjust(p, "BH"); NaN stays NaN and does not count"""
+    q = np.full(p.shape, np.nan)
+    ok = ~np.isnan(p)
+    pv = p[ok]
+    n = pv.size
+    if n:
+        o = np.argsort(-pv, kind="stable")
+        q[ok] = np.minimum(1.0, np.minimum.accumulate((n / np.arange(n, 0, -1)) * pv[o]))[np.argsort(o, kind="stable")]
+    return q
+
+
+def lm_from_moments(mom, R, N, contrasts=None):
+    """Ordinary least squares of every gene set's N scores on a design D = U R, from the moments design_stats(x, U)
+    returns (z = U^T x_s, a = sum x_s, t = sum x_s^2, per set): beta = R^-1 z, RSS = max(t - |z|^2, 0), df = N - Q,
+    sigma^2 = RSS / df; per contrast vector c (a column of `contrasts`, Q x L; None = the coefficients themselves):
+    logFC = c^T beta, SE = sigma |R^-T c|, t = logFC / SE, P.Value = 2 pt(-|t|, df), adj.P.Val = BH over the sets,
+    AveExpr = a / N.  SE, t and P.Value are NaN when df <= 0 or sigma = 0; a set with a NaN score gives NaN throughout.
+    Returns one S x 6 table per contrast, columns LM_COLUMNS."""
+    from scipy import linalg, stats
+    R = np.asarray(R, dtype=np.float64)
+    Q = R.shape[0]
+    mom = np.asarray(mom, dtype=np.float64)
+    if mom.ndim != 2 or mom.shape[0] != Q + 2:
+        raise ValueError("the moments must have Q + 2 rows")
+    Cm = np.eye(Q) if contrasts is None else np.asarray(contrasts, dtype=np.float64)
+    if Cm.ndim == 1:
+        Cm = Cm[:, None]
+    if Cm.ndim != 2 or Cm.shape[0] != Q:
+        raise ValueError("the contrasts must have one row per column of the design")
+    z, a, t2 = mom[:Q], mom[Q], mom[Q + 1]
+    df = N - Q
+    with np.errstate(invalid="ignore", divide="ignore"):
+        beta = linalg.solve_triangular(R, z, check_finite=False)
+        rss = np.maximum(t2 - (z * z).sum(axis=0), 0.0)
+        sigma = np.sqrt(rss / df) if df > 0 else np.full(a.shape, np.nan)
+        sefac = np.sqrt((linalg.solve_triangular(R, Cm, trans="T") ** 2).sum(axis=0))
+        tabs = []
+        for l in range(Cm.shape[1]):
+            logfc = Cm[:, l] @ beta
+            se = sigma * sefac[l]
+            se[(sigma == 0)] = np.nan
+            tt = logfc / se
+            p = 2.0 * stats.t.sf(np.abs(tt), df) if df > 0 else np.full(a.shape, np.nan)
+            tabs.append(np.column_stack([logfc, se, a / N, tt, p, _bh(p)]))
+    return tabs
+
+
+def _named_columns(m, prefix):
+    if isinstance(m, NamedMatrix):
+        a = np.asarray(m.mat, dtype=np.float64)
+        names = m.colnames
+    else:
+        a, names = np.asarray(m, dtype=np.float64), None
+    if a.ndim == 1:
+        a = a[:, None]
+    if names is None:
+        names = [f"{prefix}{k + 1}" for k in range(a.shape[1] if a.ndim == 2 else 0)]
+    return a, list(names)
+
+
+def plaid_lm(X: NamedMatrix, G: NamedMatrix, design, contrasts=None, gsetX: Optional[NamedMatrix] = None,
+             sort_by: str = "none", *, ctx=None, **opts_kw):
+    """Ordinary least squares of every gene set's plaid scores on `design` (N x Q, one row per column of X, finite,
+    full column rank, 1 <= Q <= 64): R's lm(gsetX[s, ] ~ design - 1) for every set s, or limma's lmFit +
+    contrasts.fit without eBayes.  `design` / `contrasts` (Q x L) are arrays or NamedMatrix (their colnames name the
+    results; otherwise coef1.. / contrast1..).  The host takes a thin QR D = U R; the GPU returns U^T x_s, sum x_s and
+    sum x_s^2 per set, fused onto the scoring call (score_design_stats; `opts_kw` selects another scorer, a list of
+    Contexts splits the columns) or from gsetX (design_stats); lm_from_moments does the rest.  A NaN score makes that
+    set's statistics NaN (lm would drop the sample instead).  Returns {name: (table, LM_COLUMNS, set names)}, tables
+    sorted by `sort_by` when it names a column, or None on no overlap."""
+    ctx0 = (ctx[0] if isinstance(ctx, (list, tuple)) else ctx) or default_context()
+    D, coef = _named_columns(design, "coef")
+    if D.ndim != 2 or D.shape[0] != X.shape[1]:
+        raise ValueError("nrow(design) must equal ncol(X)")
+    U, R = design_qr(D)
+    Cm, names = (None, coef) if contrasts is None else _named_columns(contrasts, "contrast")
+    if Cm is not None and (Cm.ndim != 2 or Cm.shape[0] != D.shape[1]):
+        raise ValueError("nrow(contrasts) must equal ncol(design)")
+    if gsetX is None:
+        mom = score_design_stats(X, G, U, ctx=ctx, **opts_kw)
+        if mom is None:
+            return None
+    else:
+        mom = design_stats(gsetX.mat if isinstance(gsetX, NamedMatrix) else gsetX, U, ctx=ctx0)
+    tabs = lm_from_moments(mom, R, D.shape[0], Cm)
+    rows = list(G.colnames) if G.colnames is not None else [str(k) for k in range(mom.shape[1])]
+    res = {}
+    for name, tab in zip(names, tabs):
+        r = rows
+        if sort_by in LM_COLUMNS:
+            o = np.argsort(tab[:, LM_COLUMNS.index(sort_by)], kind="stable")
+            tab, r = tab[o], [rows[k] for k in o]
+        res[name] = (tab, list(LM_COLUMNS), r)
+    return res
 
 
 def _align(X: NamedMatrix, G: NamedMatrix):

@@ -260,6 +260,7 @@ struct plaidgpu_ctx {
   bool have_all = false, have_nz = false, raw_valid = false, want_both = false;
   double local_min = INFINITY;
   DevBuf b_smin;
+  DevBuf b_design;  // this call's rows of the design basis (plaidgpu_design_stats)
   std::vector<double> h_med_all, h_med_nz, h_colmin;
   const double* score_vals = nullptr;  // what the score kernel reads as values
   const double* score_r0 = nullptr;
@@ -960,12 +961,13 @@ int check_groups(plaidgpu_ctx* c, const int32_t* labels, int64_t N, int K) {
   return PLAIDGPU_OK;
 }
 
-// Column chunks of the reduction: up to 64 (and at least 64 columns each), fewer when the per-chunk partials of K
-// groups would exceed 1 GiB.  K <= 2 keeps min(64, N / 64) for any S below two million sets.
-int group_nchunk(int64_t N, int32_t S, int K) {
+// Column chunks of a reduction whose result is `width` doubles: up to 64 (and at least 64 columns each), fewer when
+// the per-chunk partials would exceed 1 GiB.  K <= 2 groups (width 2 K S) keep min(64, N / 64) for any S below two
+// million sets.
+int reduce_nchunk(int64_t N, int64_t width) {
   const double partial_budget = 1073741824.0;
   int64_t n = std::min<int64_t>(64, N / 64);
-  n = std::min<int64_t>(n, (int64_t)(partial_budget / ((double)K * 2.0 * (double)S * 8.0)));
+  n = std::min<int64_t>(n, (int64_t)(partial_budget / ((double)width * 8.0)));
   return (int)std::max<int64_t>(1, n);
 }
 
@@ -977,7 +979,7 @@ int group_nchunk(int64_t N, int32_t S, int K) {
 int group_stats_device(plaidgpu_ctx* c, const double* dx, int32_t S, int64_t N, const int32_t* labels, int K, double* out,
                        bool fix = false, const double* med = nullptr, double cc = 0.0, double alpha = 1.0,
                        const double* beta = nullptr) {
-  const int nchunk = group_nchunk(N, S, K);
+  const int nchunk = reduce_nchunk(N, (int64_t)K * 2 * S);
   const int64_t nseg = (int64_t)nchunk * K;
   std::vector<int32_t> plan((size_t)(nseg + 1 + N));  // seg[nseg + 1], then cols
   int32_t* seg = plan.data();
@@ -1004,6 +1006,50 @@ int group_stats_device(plaidgpu_ctx* c, const double* dx, int32_t S, int64_t N, 
   CK(cudaEventRecord(c->ev[5], c->stream));
   const SmallRead it[1] = {{out, c->b_rowb.p, width}};
   int rc = read_small(c, it, 1);  // synchronises the stream: `plan` may go
+  if (rc) return rc;
+  float ms = 0.f;
+  cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]);
+  c->ms[2] = ms;
+  return PLAIDGPU_OK;
+}
+
+// ---- per-set products with a design (plaid.lm) -------------------------------------------------
+// B: host double, column-major N x Q with leading dimension ldb >= N; 1 <= Q <= 64, every entry finite
+int check_design(plaidgpu_ctx* c, const double* B, int64_t N, int64_t ldb, int Q) {
+  if (Q < 1 || Q > DESIGN_Q_MAX)
+    return fail(c, PLAIDGPU_ERR_ARG, "the design has Q = " + std::to_string(Q) + " columns, outside [1, " +
+                                         std::to_string(DESIGN_Q_MAX) + "]");
+  if (N > 0 && !B) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  for (int q = 0; q < Q; ++q)
+    for (int64_t j = 0; j < N; ++j)
+      if (!std::isfinite(B[j + q * ldb]))
+        return fail(c, PLAIDGPU_ERR_ARG, "design entry (" + std::to_string(j) + ", " + std::to_string(q) +
+                                             ") is not finite");
+  return PLAIDGPU_OK;
+}
+
+// {x B, row sums, row sums of squares} of the S x N device matrix dx (ld = S) into host out[(Q + 2) * S] (checked B,
+// host, ld = ldb).  Only the N rows of B this call needs go to the device.  The columns are split into chunks like
+// group_stats_device, added in column order within a chunk and the chunks in chunk order.  Kernel time in ms[2].
+// fix / med / cc / alpha / beta: the fix-up of plaidgpu_score_finish, applied in registers to raw scores.
+int design_stats_device(plaidgpu_ctx* c, const double* dx, int32_t S, int64_t N, const double* B, int64_t ldb, int Q,
+                        double* out, bool fix = false, const double* med = nullptr, double cc = 0.0,
+                        double alpha = 1.0, const double* beta = nullptr) {
+  const int64_t width = (int64_t)(Q + 2) * S;
+  const int nchunk = reduce_nchunk(N, width);
+  CK(c->b_design.reserve((size_t)std::max<int64_t>(N * Q, 1) * sizeof(double)));
+  if (N > 0)
+    CK(cudaMemcpy2DAsync(c->b_design.p, (size_t)N * sizeof(double), B, (size_t)ldb * sizeof(double),
+                         (size_t)N * sizeof(double), (size_t)Q, cudaMemcpyHostToDevice, c->stream));
+  CK(c->b_rowa.reserve((size_t)nchunk * (size_t)width * sizeof(double)));
+  CK(c->b_rowb.reserve((size_t)width * sizeof(double)));
+  CK(cudaEventRecord(c->ev[4], c->stream));
+  CK(launch_design_stats(dx, S, S, N, c->b_design.as<double>(), N, Q, nchunk, c->b_rowa.as<double>(),
+                         c->b_rowb.as<double>(), c->stream, fix, med, cc, alpha, beta));
+  c->launches += 2;
+  CK(cudaEventRecord(c->ev[5], c->stream));
+  const SmallRead it[1] = {{out, c->b_rowb.p, width}};
+  int rc = read_small(c, it, 1);  // synchronises the stream: B may go
   if (rc) return rc;
   float ms = 0.f;
   cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]);
@@ -1081,10 +1127,14 @@ plaidgpu_matrix column_slice(const plaidgpu_matrix* X, int64_t j0, int64_t j1, s
 // What the finish step of a scoring call makes of the raw S x N scores.  Every kind but SCORES keeps the raw scores
 // in the library's device buffer (out_location = PLAIDGPU_HOST) and applies the fix-up in registers.
 struct Target {
-  enum Kind { SCORES, GROUP_STATS, TOPK, FILE_TILES } kind = SCORES;
-  double* out = nullptr;            // SCORES: the S x N scores at opts.out_location; GROUP_STATS: K * 2 * S moments
+  enum Kind { SCORES, GROUP_STATS, DESIGN_STATS, TOPK, FILE_TILES } kind = SCORES;
+  double* out = nullptr;            // SCORES: the S x N scores at opts.out_location; GROUP_STATS: K * 2 * S moments;
+                                    // DESIGN_STATS: (Q + 2) * S moments
   const int32_t* labels = nullptr;  // GROUP_STATS: int32[N] in [-1, K)
   int K = 0;
+  const double* B = nullptr;        // DESIGN_STATS: host, column-major N x Q, leading dimension ldb
+  int64_t ldb = 0;
+  int Q = 0;
   int k = 0, decreasing = 0;        // TOPK: idx / val hold k * N entries
   int32_t* idx = nullptr;
   double* val = nullptr;
@@ -1095,18 +1145,32 @@ struct Target {
   static Target group_stats(const int32_t* labels, int K, double* out) {
     Target t; t.kind = GROUP_STATS; t.labels = labels; t.K = K; t.out = out; return t;
   }
+  static Target design_stats(const double* B, int64_t ldb, int Q, double* out) {
+    Target t; t.kind = DESIGN_STATS; t.B = B; t.ldb = ldb; t.Q = Q; t.out = out; return t;
+  }
   static Target topk(int k, int decreasing, int32_t* idx, double* val) {
     Target t; t.kind = TOPK; t.k = k; t.decreasing = decreasing != 0; t.idx = idx; t.val = val; return t;
   }
   static Target to_file(FILE* file, double* stage0, double* stage1) {
     Target t; t.kind = FILE_TILES; t.file = file; t.stage[0] = stage0; t.stage[1] = stage1; return t;
   }
-  // the same target for the columns from j0 on; group statistics write those columns' moments to `moments`
+  // doubles of moments a GROUP_STATS / DESIGN_STATS target returns (0 for the other kinds)
+  size_t moment_count(int32_t S) const {
+    if (kind == GROUP_STATS) return (size_t)K * 2 * (size_t)S;
+    if (kind == DESIGN_STATS) return (size_t)(Q + 2) * (size_t)S;
+    return 0;
+  }
+  // the same target for the columns from j0 on; group and design statistics write those columns' moments to
+  // `moments`
   Target from(int64_t j0, int32_t S, double* moments) const {
     Target t = *this;
     if (kind == SCORES) t.out = out + j0 * (int64_t)S;
     if (kind == GROUP_STATS) {
       t.labels = labels + j0;
+      t.out = moments;
+    }
+    if (kind == DESIGN_STATS) {
+      t.B = B + j0;  // rows j0.. of B, same leading dimension
       t.out = moments;
     }
     if (kind == TOPK) {
@@ -1841,7 +1905,7 @@ int plaidgpu_combine_medians(int ignore_zero_opt, double score_min, const double
   return PLAIDGPU_ERR_ARG;
 }
 
-// plaidgpu_score_finish into target t (SCORES, GROUP_STATS or TOPK)
+// plaidgpu_score_finish into target t (SCORES, GROUP_STATS, DESIGN_STATS or TOPK)
 static int score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, const Target& t) try {
   if (t.kind == Target::SCORES && !t.out && c->N > 0) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
   if (!c->computed) return fail(c, PLAIDGPU_ERR_STATE, "plaidgpu_score_compute has not been called");
@@ -1875,8 +1939,10 @@ static int score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, const Tar
   }
 
   // the reductions read the raw scores with the fix-up applied in registers: the S x N matrix stays on the device
-  // and only K * 2 * S moments, or k * N indices and values, go back
+  // and only K * 2 * S or (Q + 2) * S moments, or k * N indices and values, go back
   if (t.kind == Target::GROUP_STATS) return group_stats_device(c, c->raw, S, N, t.labels, t.K, t.out, fix, med, cc, alpha, beta);
+  if (t.kind == Target::DESIGN_STATS)
+    return design_stats_device(c, c->raw, S, N, t.B, t.ldb, t.Q, t.out, fix, med, cc, alpha, beta);
   if (t.kind == Target::TOPK) return topk_device(c, c->raw, S, N, t.k, t.decreasing, t.idx, t.val, fix, med, cc, alpha, beta);
   double* out = t.out;
   c->raw_valid = false;  // the fix-up below rewrites the raw scores in place
@@ -2024,15 +2090,15 @@ int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double*
 // columns, so a normalised call recomputes the scores: pass 1 keeps only the per-column medians,
 // pass 2 recomputes, fixes up and streams each chunk out (recomputing costs less than moving the raw
 // scores over PCIe twice).  Results are bit-identical to the un-chunked path.
-// The tile of columns [j0, j1) finishes into t.from(j0): its columns of the scores or of idx / val, or its group
-// moments, which are added to t.out (zeroed here) in tile order.  FILE_TILES stages every finished tile in a pinned
+// The tile of columns [j0, j1) finishes into t.from(j0): its columns of the scores or of idx / val, or its group or
+// design moments, which are added to t.out (zeroed here) in tile order.  FILE_TILES stages every finished tile in a pinned
 // buffer and writes it to the file: tiled egress for results larger than host memory (scope row f4).
 static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
                          const Target& t, int64_t chunk) {
   const int64_t N = X->N;
   const int32_t S = c->S;
-  std::vector<double> moments(t.kind == Target::GROUP_STATS ? (size_t)t.K * 2 * (size_t)S : 0);  // one tile's group moments
-  if (t.kind == Target::GROUP_STATS) std::fill(t.out, t.out + moments.size(), 0.0);
+  std::vector<double> moments(t.moment_count(S));  // one tile's group or design moments
+  std::fill(t.out, t.out + moments.size(), 0.0);
   if (opts->scorer == PLAIDGPU_GSVA && opts->gsva_ecdf != PLAIDGPU_ROWTF_DONE &&
       (opts->gsva_ecdf || !(opts->row_mean && opts->row_sd)))
     return fail(c, PLAIDGPU_ERR_ARG, "replaid.gsva: matrix too large for one device pass (rowtf ecdf needs all samples; rowtf z needs row_mean / row_sd)");
@@ -2245,6 +2311,23 @@ int plaidgpu_score_group_stats(plaidgpu_ctx* c, const plaidgpu_matrix* X, const 
   return PLAIDGPU_ERR_ARG;
 }
 
+// score -> linear model fused: plaid() / a replaid.* scorer followed by the per-set products with the design basis B
+// (plaid.lm) without the S x N matrix leaving the device or being written in its normalised form.  Bit-identical to
+// plaidgpu_score + plaidgpu_design_stats.  Host X whose S x N scores exceed the device goes through score_chunked
+// (two passes when normalised) and adds the tiles' moments in tile order.
+int plaidgpu_score_design_stats(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap,
+                                const plaidgpu_opts* opts, const double* B, int Q, double* out) try {
+  if (!c) return PLAIDGPU_ERR_ARG;
+  if (!X || !rowmap || !opts || !out) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  int rc = check_design(c, B, X->N, X->N, Q);
+  if (rc) return rc;
+  return score_one(c, X, rowmap, opts, Target::design_stats(B, X->N, Q, out));
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
 // score -> top sets fused: plaid() / a replaid.* scorer followed by each column's top k (plaid.topsets) without the
 // S x N matrix leaving the device or being written in its normalised form.  Bit-identical to plaidgpu_score +
 // plaidgpu_col_topk.  Host X whose S x N scores exceed the device is scored in column tiles, each writing its own
@@ -2319,8 +2402,8 @@ static int check_shard_ctxs(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_opt
 }
 
 // Shard r (columns [lo_r, lo_{r+1})) finishes on ctxs[r] into t.from(lo_r): its block of the scores, its columns of
-// idx / val, or its own group moments, of which shard 0's are copied to t.out and shards 1 to n - 1 added in shard
-// order.
+// idx / val, or its own group or design moments, of which shard 0's are copied to t.out and shards 1 to n - 1 added
+// in shard order.
 static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
                             const plaidgpu_opts* opts, const Target& t, const std::string& who) {
   plaidgpu_ctx* c = ctxs[0];
@@ -2336,7 +2419,7 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
     for (int r = 0; r < n; ++r) M[r] = column_slice(X, lo[r], lo[r + 1], pbuf[r]);
     std::vector<plaidgpu_scalars> loc((size_t)n);
     std::vector<int> rc((size_t)n, PLAIDGPU_OK);
-    const size_t width = t.kind == Target::GROUP_STATS ? (size_t)t.K * 2 * (size_t)S : 0;
+    const size_t width = t.moment_count(S);
     std::vector<std::vector<double>> moments((size_t)n, std::vector<double>(width));
     std::vector<double> med((size_t)std::max<int64_t>(N, 1));
     std::vector<std::vector<double>> part(gsva_z ? (size_t)n : 0, std::vector<double>((size_t)P));
@@ -2417,7 +2500,7 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
         if (r > 0) c->err = "shard " + std::to_string(r) + ": " + ctxs[r]->err;
         return rc[r];
       }
-    if (t.kind == Target::GROUP_STATS) {
+    if (width) {
       std::copy(moments[0].begin(), moments[0].end(), t.out);
       for (int r = 1; r < n; ++r)
         for (size_t i = 0; i < width; ++i) t.out[i] += moments[r][i];
@@ -2443,10 +2526,12 @@ static int score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* 
   if (rc) return rc;
   if (n == 1 || X->N < 2 * (int64_t)n) {
     if (t.kind == Target::GROUP_STATS) return plaidgpu_score_group_stats(c, X, rowmap, opts, t.labels, t.K, t.out);
+    if (t.kind == Target::DESIGN_STATS) return plaidgpu_score_design_stats(c, X, rowmap, opts, t.B, t.Q, t.out);
     if (t.kind == Target::TOPK) return plaidgpu_score_topk(c, X, rowmap, opts, t.k, t.decreasing, t.idx, t.val);
     return plaidgpu_score(c, X, rowmap, opts, t.out);
   }
   if (t.kind == Target::GROUP_STATS) rc = check_groups(c, t.labels, X->N, t.K);
+  if (t.kind == Target::DESIGN_STATS) rc = check_design(c, t.B, X->N, t.ldb, t.Q);
   if (t.kind == Target::TOPK) rc = check_topk(c, c->S, t.k);
   if (rc) return rc;
   return score_multi_impl(ctxs, n, X, rowmap, opts, t, who);
@@ -2468,6 +2553,17 @@ int plaidgpu_score_group_stats_multi(plaidgpu_ctx* const* ctxs, int n, const pla
   if (!ctxs || n <= 0 || !ctxs[0]) return PLAIDGPU_ERR_ARG;
   if (!X || !rowmap || !opts || !out) return fail(ctxs[0], PLAIDGPU_ERR_ARG, "null argument");
   return score_multi(ctxs, n, X, rowmap, opts, Target::group_stats(labels, K, out), "plaidgpu_score_group_stats_multi");
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
+int plaidgpu_score_design_stats_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
+                                      const plaidgpu_opts* opts, const double* B, int Q, double* out) try {
+  if (!ctxs || n <= 0 || !ctxs[0]) return PLAIDGPU_ERR_ARG;
+  if (!X || !rowmap || !opts || !out) return fail(ctxs[0], PLAIDGPU_ERR_ARG, "null argument");
+  return score_multi(ctxs, n, X, rowmap, opts, Target::design_stats(B, X->N, Q, out), "plaidgpu_score_design_stats_multi");
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {
@@ -2656,6 +2752,29 @@ int plaidgpu_group_stats(plaidgpu_ctx* c, const double* x, int32_t S, int64_t N,
     dx = c->b_raw.as<double>();
   }
   return group_stats_device(c, dx, S, N, labels, K, out);
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
+int plaidgpu_design_stats(plaidgpu_ctx* c, const double* x, int32_t S, int64_t N, const double* B, int Q, int location,
+                          double* out) try {
+  if (!c) return PLAIDGPU_ERR_ARG;
+  if (S <= 0 || N < 0) return fail(c, PLAIDGPU_ERR_ARG, "bad argument");
+  if (!out || (N > 0 && !x)) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  if (location != PLAIDGPU_HOST && location != PLAIDGPU_DEVICE) return fail(c, PLAIDGPU_ERR_ARG, "unknown location");
+  int rc = check_design(c, B, N, N, Q);
+  if (rc) return rc;
+  CK(cudaSetDevice(c->device));
+  const int64_t total = (int64_t)S * N;
+  const double* dx = x;
+  if (location == PLAIDGPU_HOST) {
+    CK(c->b_raw.reserve((size_t)std::max<int64_t>(total, 1) * sizeof(double)));
+    if (total) CK(cudaMemcpyAsync(c->b_raw.p, x, (size_t)total * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    dx = c->b_raw.as<double>();
+  }
+  return design_stats_device(c, dx, S, N, B, N, Q, out);
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {

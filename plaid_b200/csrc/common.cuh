@@ -189,6 +189,16 @@ cudaError_t launch_fixup(const double* x, double* out, int64_t ld, int32_t S, in
 cudaError_t launch_group_stats(const double* x, int64_t ld, int32_t S, int K, const int32_t* cols, const int32_t* seg,
                                int nchunk, double* partial, double* out, cudaStream_t st, bool fix = false,
                                const double* med = nullptr, double c = 0.0, double alpha = 1.0, const double* beta = nullptr);
+// per-row products with a dense design (plaid.lm): out[(Q + 2) * S] = {sum_j x[s,j] * B[j,q] for q < Q [S each],
+// sum_j x[s,j] [S], sum_j x[s,j]^2 [S]}; B is device, column-major N x Q with leading dimension ldb.  Columns are
+// split into nchunk chunks as in launch_group_stats (partial = nchunk * (Q + 2) * S doubles of scratch), added in
+// ascending order inside a chunk and the chunks in chunk order; one pass over x for every Q (two launches).
+// fix: as for launch_group_stats
+constexpr int DESIGN_Q_MAX = 64;
+cudaError_t launch_design_stats(const double* x, int64_t ld, int32_t S, int64_t N, const double* B, int64_t ldb, int Q,
+                                int nchunk, double* partial, double* out, cudaStream_t st, bool fix = false,
+                                const double* med = nullptr, double c = 0.0, double alpha = 1.0,
+                                const double* beta = nullptr);
 // per column of a column-major S x N matrix: the k (1 <= k <= min(S, TOPK_MAX)) rows first in R's
 // order(v, decreasing = decreasing) (ties by ascending row, NaN last) into idx / val[k * N] (device, column-major).
 // fix: x holds RAW scores and the selection is over alpha * (x - med_j + c) + beta_s (k_fixup's arithmetic)

@@ -1100,6 +1100,15 @@ __global__ void __launch_bounds__(256) k_minmax(const double* __restrict__ x, in
   }
 }
 
+// k_fixup's operations, in its order, on one raw score v of column j (b = beta[row], read once by the caller)
+__device__ __forceinline__ double fixup_value(double v, int64_t j, const double* __restrict__ med, double c, double alpha,
+                                              const double* __restrict__ beta, double b) {
+  const double shift = (med ? -med[j] : 0.0) + c;
+  v = __dmul_rn(alpha, __dadd_rn(v, shift));
+  if (beta) v = __dadd_rn(v, b);
+  return v;
+}
+
 // row sums / sums of squares of a column-major S x N matrix by column group (labels in [0, K); unlabelled columns
 // take no part).  The host sorts the labelled columns by (chunk, group), ascending inside each group, into `cols`;
 // segment g = chunk * K + group is cols[seg[g] .. seg[g + 1]).  grid = (segments, row blocks): each thread owns one
@@ -1123,11 +1132,7 @@ __global__ void __launch_bounds__(256) k_group_partial(const double* __restrict_
   for (int32_t i = i0; i < i1; ++i) {
     const int64_t j = cols[i];
     double v = __ldcs(x + j * ld + r);
-    if (FIX) {
-      const double shift = (med ? -med[j] : 0.0) + c;
-      v = __dmul_rn(alpha, __dadd_rn(v, shift));
-      if (beta) v = __dadd_rn(v, b);
-    }
+    if (FIX) v = fixup_value(v, j, med, c, alpha, beta, b);
     s += v;
     q += v * v;
   }
@@ -1143,6 +1148,82 @@ __global__ void __launch_bounds__(256) k_group_combine(const double* __restrict_
   double a = 0.0;
   for (int ch = 0; ch < nchunk; ++ch) a += partial[(size_t)ch * width + i];
   out[i] = a;
+}
+
+// Per set row of a column-major S x N matrix and one chunk of columns (chunk ch is [N ch / nchunk, N (ch + 1) / nchunk),
+// the split of group_stats_device): sum_j x[s, j] * B[j, q] for the Q <= QB columns of B, sum_j x[s, j] and
+// sum_j x[s, j]^2.  grid = (set blocks, chunks): each thread owns one set and adds its chunk's columns in ascending
+// order, so every raw score is read once; the CTAs that run together share a chunk, so its rows of B come from DRAM
+// about once.  The chunk's rows of B are staged DESIGN_TJ at a time in shared memory, zero-padded to QB columns, and
+// read as 16-byte broadcasts (the row stride QB + 2 keeps them aligned).  partial[ch][(Q + 2) * S] = {row q of the moments at q * S, the sums at Q * S, the sums of squares at
+// (Q + 1) * S}; k_group_combine adds the chunks in chunk order.  FIX: as in k_group_partial.
+constexpr int DESIGN_TJ = 32;
+template <bool FIX, int QB>
+__global__ void __launch_bounds__(256) k_design_partial(const double* __restrict__ x, int64_t ld, int32_t S, int64_t N,
+                                                        int nchunk, const double* __restrict__ B, int64_t ldb, int Q,
+                                                        double* __restrict__ partial,
+                                                        const double* __restrict__ med, double c, double alpha,
+                                                        const double* __restrict__ beta) {
+  __shared__ __align__(16) double Bs[DESIGN_TJ][QB + 2];
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  const int ch = blockIdx.y;
+  const int64_t j0 = (N * ch) / nchunk, j1 = (N * (ch + 1)) / nchunk;
+  const bool live = r < S;
+  const double b = (FIX && beta && live) ? beta[r] : 0.0;
+  double acc[QB];
+#pragma unroll
+  for (int q = 0; q < QB; ++q) acc[q] = 0.0;
+  double s = 0.0, t = 0.0;
+  for (int64_t jt = j0; jt < j1; jt += DESIGN_TJ) {
+    const int nj = (int)min((int64_t)DESIGN_TJ, j1 - jt);
+    __syncthreads();  // every thread is done with the previous tile
+    for (int i = threadIdx.x; i < DESIGN_TJ * QB; i += blockDim.x) {
+      const int jj = i % DESIGN_TJ, q = i / DESIGN_TJ;  // a warp reads 32 consecutive rows of one column of B
+      Bs[jj][q] = (jj < nj && q < Q) ? B[(jt + jj) + (int64_t)q * ldb] : 0.0;
+    }
+    __syncthreads();
+    if (!live) continue;
+#pragma unroll 4
+    for (int jj = 0; jj < nj; ++jj) {
+      const int64_t j = jt + jj;
+      double v = __ldcs(x + j * ld + r);
+      if (FIX) v = fixup_value(v, j, med, c, alpha, beta, b);
+      s += v;
+      t += v * v;
+#pragma unroll
+      for (int q = 0; q < QB; q += 2) {
+        const double2 w = *reinterpret_cast<const double2*>(&Bs[jj][q]);
+        acc[q] += v * w.x;
+        acc[q + 1] += v * w.y;
+      }
+    }
+  }
+  if (!live) return;
+  double* p = partial + (size_t)ch * (size_t)(Q + 2) * S;
+#pragma unroll
+  for (int q = 0; q < QB; ++q)
+    if (q < Q) p[(size_t)q * S + r] = acc[q];
+  p[(size_t)Q * S + r] = s;
+  p[(size_t)(Q + 1) * S + r] = t;
+}
+
+template <bool FIX>
+void design_partial(dim3 g, cudaStream_t st, int qb, const double* x, int64_t ld, int32_t S, int64_t N, int nchunk,
+                    const double* B, int64_t ldb, int Q, double* partial, const double* med, double c,
+                    double alpha, const double* beta) {
+#define PLAIDGPU_DESIGN_CASE(W)                                                                                   \
+  case W:                                                                                                         \
+    k_design_partial<FIX, W><<<g, 256, 0, st>>>(x, ld, S, N, nchunk, B, ldb, Q, partial, med, c, alpha, beta);     \
+    break;
+  switch (qb) {
+    PLAIDGPU_DESIGN_CASE(2)
+    PLAIDGPU_DESIGN_CASE(4)
+    PLAIDGPU_DESIGN_CASE(8)
+    PLAIDGPU_DESIGN_CASE(16)
+    PLAIDGPU_DESIGN_CASE(32)
+    PLAIDGPU_DESIGN_CASE(64)
+  }
+#undef PLAIDGPU_DESIGN_CASE
 }
 
 // device -> host-mapped memory by SM stores: small control values (minimum key, flags, medians) must not queue
@@ -1279,6 +1360,22 @@ cudaError_t launch_group_stats(const double* x, int64_t ld, int32_t S, int K, co
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
   const int64_t width = (int64_t)K * 2 * S;
+  k_group_combine<<<(unsigned)((width + 255) / 256), 256, 0, st>>>(partial, width, nchunk, out);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_design_stats(const double* x, int64_t ld, int32_t S, int64_t N, const double* B, int64_t ldb, int Q,
+                                int nchunk, double* partial, double* out, cudaStream_t st, bool fix, const double* med,
+                                double c, double alpha, const double* beta) {
+  if (S <= 0 || Q < 1 || Q > DESIGN_Q_MAX) return cudaErrorInvalidValue;
+  const dim3 g((unsigned)((S + 255) / 256), (unsigned)nchunk);
+  int qb = 2;  // the narrowest instantiation that holds Q: one pass over x for every Q
+  while (qb < Q) qb *= 2;
+  if (fix) design_partial<true>(g, st, qb, x, ld, S, N, nchunk, B, ldb, Q, partial, med, c, alpha, beta);
+  else design_partial<false>(g, st, qb, x, ld, S, N, nchunk, B, ldb, Q, partial, nullptr, 0.0, 1.0, nullptr);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  const int64_t width = (int64_t)(Q + 2) * S;
   k_group_combine<<<(unsigned)((width + 255) / 256), 256, 0, st>>>(partial, width, nchunk, out);
   return cudaGetLastError();
 }

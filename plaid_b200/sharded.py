@@ -268,6 +268,22 @@ def score_group_stats_shard(ctx, comm, M: L.Matrix, rowmap: np.ndarray, opts: L.
     return comm.allreduce_sum_vec(out.ravel()).reshape(out.shape)
 
 
+def score_design_stats_shard(ctx, comm, M: L.Matrix, rowmap: np.ndarray, opts: L.Opts, B_rows, n_cols: int):
+    """design_stats of this rank's scores, summed over all ranks (in rank order): score_shard into a device buffer,
+    plaidgpu_design_stats on it, then one all-reduce of (Q + 2) * S doubles.  B_rows: this rank's n_cols rows of the
+    global design basis U (N x Q).  `ctx` must hold the gene sets (Context.set_genesets).  Returns (Q + 2, S)."""
+    import torch
+    S = ctx.n_sets
+    b = np.asfortranarray(np.asarray(B_rows, dtype=np.float64).reshape(n_cols, -1))
+    buf = torch.empty(max(S * n_cols, 1), dtype=torch.float64, device=f"cuda:{ctx.device}")
+    opts.out_location = L.DEVICE
+    score_shard(ctx, comm, M, rowmap, opts, buf.data_ptr(), n_cols)
+    out = np.empty((b.shape[1] + 2, S), dtype=np.float64)
+    ctx.check(ctx.lib.plaidgpu_design_stats(ctx.h, buf.data_ptr(), S, n_cols, b.ctypes.data, b.shape[1], L.DEVICE,
+                                            out.ctypes.data))
+    return comm.allreduce_sum_vec(out.ravel()).reshape(out.shape)
+
+
 def score_topk_shard(ctx, comm, M: L.Matrix, rowmap: np.ndarray, opts: L.Opts, k: int, decreasing: bool, n_cols: int):
     """Each of this rank's cells' k best gene sets: score_shard into a device buffer, then plaidgpu_col_topk on it.
     The selection is column-local, so nothing is exchanged beyond what scoring needs.  `ctx` must hold the gene sets

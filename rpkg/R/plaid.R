@@ -37,7 +37,7 @@
   }
 }
 
-.score <- function(X, matG, opts, labels = NULL, K = NULL, topk = NULL, decreasing = TRUE) {
+.score <- function(X, matG, opts, labels = NULL, K = NULL, topk = NULL, decreasing = TRUE, design = NULL) {
   x <- .as_x(X)
   rn <- x$dimnames[[1]]
   gg <- intersect(rn, rownames(matG))                                 # R/plaid.R:65
@@ -54,6 +54,12 @@
   if (!is.null(labels)) {  # plaid.test("lm"): scores reduced per set and sample group on the device, S x 2K back
     out <- .Call(C_plaidgpu_score_group_stats, .ctxs(), x$kind, x$p, x$i, x$x, as.integer(x$dim),
                  G@p, G@i, G@x, as.integer(dim(G)), as.integer(rowmap), opts, as.integer(labels), as.integer(K))
+    rownames(out) <- colnames(matG)
+    return(out)
+  }
+  if (!is.null(design)) {  # plaid.lm: scores times the design basis, reduced per set on the device, S x (Q + 2) back
+    out <- .Call(C_plaidgpu_score_design_stats, .ctxs(), x$kind, x$p, x$i, x$x, as.integer(x$dim),
+                 G@p, G@i, G@x, as.integer(dim(G)), as.integer(rowmap), opts, design)
     rownames(out) <- colnames(matG)
     return(out)
   }
@@ -309,6 +315,63 @@ plaid.test.groups <- function(X, groups, G, gsetX, tests = c("one", "two", "lm")
     .test_table(pv, ff, G, metap.method, sort.by)
   })
   names(res) <- lev
+  res
+}
+
+## Ordinary least squares of every gene set's plaid scores on a design: lm(gsetX[s, ] ~ design - 1) for every set s,
+## or limma's lmFit + contrasts.fit without eBayes.  design: N x Q (one row per column of X), finite, of full column
+## rank, 1 <= Q <= 64; contrasts: NULL (one result per column of the design) or a Q x L matrix.  qr() of the design
+## runs in R; without gsetX, plaid() runs fused with the reduction U^T s, sum s, sum s^2 per set, so the S x N scores
+## never reach R (options(plaid.gpus) applies); with gsetX (the scores of any scorer, sets x cells) the reduction runs
+## on that matrix.  A named list (colnames of the design or the contrasts) of tables with rows = colnames(matG) and
+## columns logFC, SE, AveExpr, t, P.Value, adj.P.Val (BH over sets).  With N = Q or a perfect fit, SE, t and P.Value
+## are NA.  A NaN score makes that set's statistics NaN (lm would drop the sample instead).
+plaid.lm <- function(X, matG, design, contrasts = NULL, gsetX = NULL, sort.by = "none") {
+  design <- as.matrix(design)
+  storage.mode(design) <- "double"
+  if (nrow(design) != ncol(X)) stop("nrow(design) must equal ncol(X)")
+  if (anyNA(design) || any(!is.finite(design))) stop("the design must be finite (no NA)")
+  Q <- ncol(design); N <- nrow(design)
+  if (Q < 1 || Q > 64) stop("the design must have 1 to 64 columns")
+  qd <- qr(design)
+  if (qd$rank < Q || N < Q) stop("the design is not of full column rank")
+  U <- qr.Q(qd); R <- qr.R(qd)                             # full rank: no column was pivoted
+  cn <- colnames(design)
+  if (is.null(cn)) cn <- paste0("coef", seq_len(Q))
+  if (is.null(contrasts)) {
+    contrasts <- diag(Q); colnames(contrasts) <- cn
+  } else {
+    contrasts <- as.matrix(contrasts)
+    if (nrow(contrasts) != Q) stop("nrow(contrasts) must equal ncol(design)")
+    if (is.null(colnames(contrasts))) colnames(contrasts) <- paste0("contrast", seq_len(ncol(contrasts)))
+  }
+  if (is.null(gsetX)) {
+    mom <- .score(X, matG, list(scorer = 0L, stats_mean = 1L, normalize = 1L), design = U)
+    if (is.null(mom)) return(NULL)
+  } else {
+    gsetX <- as.matrix(gsetX)
+    storage.mode(gsetX) <- "double"
+    mom <- .Call(C_plaidgpu_design_stats, .ctx(), gsetX, U)
+  }
+  z <- t(mom[, seq_len(Q), drop = FALSE])
+  beta <- backsolve(R, z)
+  rss <- pmax(mom[, Q + 2L] - colSums(z^2), 0)
+  df <- N - Q
+  sigma <- if (df > 0) sqrt(rss / df) else rep(NA_real_, nrow(mom))
+  sigma[!is.na(sigma) & sigma == 0] <- NA_real_
+  sefac <- sqrt(colSums(backsolve(R, contrasts, transpose = TRUE)^2))
+  res <- lapply(seq_len(ncol(contrasts)), function(l) {
+    logFC <- drop(crossprod(contrasts[, l], beta))
+    SE <- sigma * sefac[l]
+    tt <- logFC / SE
+    p <- if (df > 0) 2 * stats::pt(-abs(tt), df) else rep(NA_real_, length(tt))
+    tab <- cbind(logFC = logFC, SE = SE, AveExpr = mom[, Q + 1L] / N, t = tt, P.Value = p,
+                 adj.P.Val = stats::p.adjust(p, method = "BH"))
+    rownames(tab) <- colnames(matG)
+    if (sort.by %in% colnames(tab)) tab <- tab[order(tab[, sort.by]), , drop = FALSE]
+    tab
+  })
+  names(res) <- colnames(contrasts)
   res
 }
 

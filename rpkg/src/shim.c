@@ -231,6 +231,64 @@ SEXP C_plaidgpu_score_group_stats(SEXP ctx, SEXP kind, SEXP Xp, SEXP Xi, SEXP Xx
   return out;
 }
 
+/* plaid.lm(gsetX = ): per set of gsetX (S x N) the products with the N x Q design basis B, the sum and the sum of
+ * squares as an S x (Q + 2) matrix */
+SEXP C_plaidgpu_design_stats(SEXP ctx, SEXP x, SEXP B) {
+  plaidgpu_ctx* c = get_ctx(ctx);
+  SEXP dim = Rf_getAttrib(x, R_DimSymbol), bdim = Rf_getAttrib(B, R_DimSymbol);
+  const int S = INTEGER(dim)[0], N = INTEGER(dim)[1];
+  if (bdim == R_NilValue || INTEGER(bdim)[0] != N) Rf_error("plaidgpu: nrow(design) must equal ncol(gsetX)");
+  const int Q = INTEGER(bdim)[1];
+  if (Q < 1 || Q > 64) Rf_error("plaidgpu: the design must have 1 to 64 columns");
+  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, S, Q + 2));
+  int rc = plaidgpu_design_stats(c, REAL(x), S, N, REAL(B), Q, PLAIDGPU_HOST, REAL(out));
+  if (rc != PLAIDGPU_OK) {
+    UNPROTECT(1);
+    Rf_error("plaidgpu_design_stats: %s", plaidgpu_last_error(c));
+  }
+  UNPROTECT(1);
+  return out;
+}
+
+/* plaid.lm(): plaid() fused with the per-set products with the design basis B (N x Q) — the S x N scores stay on the
+ * device, an S x (Q + 2) matrix comes back.  A list of contexts (options(plaid.gpus = n)) splits the columns over the
+ * devices (plaidgpu_score_design_stats_multi). */
+SEXP C_plaidgpu_score_design_stats(SEXP ctx, SEXP kind, SEXP Xp, SEXP Xi, SEXP Xx, SEXP Xdim, SEXP Gp, SEXP Gi,
+                                   SEXP Gx, SEXP Gdim, SEXP rowmap, SEXP opts, SEXP B) {
+  plaidgpu_ctx* cs[16];
+  int nctx = 1;
+  if (TYPEOF(ctx) == VECSXP) {
+    nctx = (int)XLENGTH(ctx);
+    if (nctx < 1 || nctx > 16) Rf_error("plaidgpu: between 1 and 16 contexts expected");
+    for (int j = 0; j < nctx; ++j) cs[j] = get_ctx(VECTOR_ELT(ctx, j));
+  } else {
+    cs[0] = get_ctx(ctx);
+  }
+  plaidgpu_ctx* c = cs[0];
+  const int PG = INTEGER(Gdim)[0], S = INTEGER(Gdim)[1];
+  for (int j = 0; j < nctx; ++j)
+    if (plaidgpu_set_genesets(cs[j], PG, S, INTEGER(Gp), INTEGER(Gi), REAL(Gx)) != PLAIDGPU_OK)
+      Rf_error("plaidgpu_set_genesets: %s", plaidgpu_last_error(cs[j]));
+  plaidgpu_matrix M;
+  fill_matrix(&M, Rf_asInteger(kind), Xp, Xi, Xx, Xdim);
+  SEXP bdim = Rf_getAttrib(B, R_DimSymbol);
+  if (bdim == R_NilValue || (int64_t)INTEGER(bdim)[0] != M.N) Rf_error("plaidgpu: nrow(design) must equal ncol(X)");
+  const int Q = INTEGER(bdim)[1];
+  if (Q < 1 || Q > 64) Rf_error("plaidgpu: the design must have 1 to 64 columns");
+  plaidgpu_opts o;
+  fill_opts(&o, opts);
+  R_CheckUserInterrupt();
+  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, S, Q + 2));
+  int rc = nctx > 1 ? plaidgpu_score_design_stats_multi(cs, nctx, &M, INTEGER(rowmap), &o, REAL(B), Q, REAL(out))
+                    : plaidgpu_score_design_stats(c, &M, INTEGER(rowmap), &o, REAL(B), Q, REAL(out));
+  if (rc != PLAIDGPU_OK) {
+    UNPROTECT(1);
+    Rf_error("plaidgpu_score_design_stats: %s", plaidgpu_last_error(c));
+  }
+  UNPROTECT(1);
+  return out;
+}
+
 /* per-column top k as one k x 2N matrix: columns 1..N the 1-based row indices (exact in a double), N+1..2N the values;
  * idx / val are what plaidgpu_col_topk / plaidgpu_score_topk wrote, val already in place */
 static void topk_indices_to_r(SEXP out, const int32_t* idx, int k, int N) {
@@ -306,6 +364,8 @@ static const R_CallMethodDef call_methods[] = {
     {"C_plaidgpu_colranks", (DL_FUNC)&C_plaidgpu_colranks, 9},
     {"C_plaidgpu_group_stats", (DL_FUNC)&C_plaidgpu_group_stats, 4},
     {"C_plaidgpu_score_group_stats", (DL_FUNC)&C_plaidgpu_score_group_stats, 14},
+    {"C_plaidgpu_design_stats", (DL_FUNC)&C_plaidgpu_design_stats, 3},
+    {"C_plaidgpu_score_design_stats", (DL_FUNC)&C_plaidgpu_score_design_stats, 13},
     {"C_plaidgpu_col_topk", (DL_FUNC)&C_plaidgpu_col_topk, 4},
     {"C_plaidgpu_score_topk", (DL_FUNC)&C_plaidgpu_score_topk, 14},
     {"C_plaidgpu_crossprod", (DL_FUNC)&C_plaidgpu_crossprod, 11},
