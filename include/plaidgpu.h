@@ -129,7 +129,10 @@ typedef struct plaidgpu_scalars {
   double score_min;    /* min(raw scores, na.rm)        (combine: min)  R/plaid.R:557 */
   double med_mean;     /* mean(medx): OUTPUT of the combine step, see plaidgpu_combine_medians */
   int32_t ignore_zero; /* resolved flag (0/1) after combine */
-  int32_t _pad;
+  int32_t fp64;        /* OUTPUT of plaidgpu_score_compute: 1 when the fixed-point route gave up on this context's
+                          data (a non-finite entry, a column exponent outside [-900, 900], or a non-zero entry that
+                          rounds to 0) and the fp64 passes produced its scores; 0 otherwise, also with exact_fp64
+                          (combine: max, see step 3b of the sharded protocol below) */
 } plaidgpu_scalars;
 
 /* ---- lifecycle ---------------------------------------------------------------- */
@@ -180,7 +183,10 @@ int plaidgpu_score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix
  *        context (plaidgpu_get_col_medians).  `out` is the buffer later given to
  *        plaidgpu_score_finish: with out_location == PLAIDGPU_DEVICE the raw scores are written
  *        straight into it (no second copy of the S x N matrix exists); with PLAIDGPU_HOST it
- *        may be NULL here;
+ *        may be NULL here.  It also reports fp64 (see plaidgpu_scalars);
+ *   3b. caller combines fp64 (max); when it is 1 and opts.exact_fp64 is 0, every shard that reported 0
+ *        repeats steps 1 and 3 with exact_fp64 = 1 (the scalars of step 2 stay), so that every column of the
+ *        call comes from the same route;
  *   4. if opts.normalize: caller combines score_min (min), gathers the medians of all shards
  *        in column order and calls plaidgpu_combine_medians() once to get med_mean /
  *        ignore_zero (bit-identical for any shard count);

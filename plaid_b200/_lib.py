@@ -39,7 +39,7 @@ class Opts(C.Structure):
 class Scalars(C.Structure):
     _fields_ = [("x_min", C.c_double), ("x_max", C.c_double), ("rank_max", C.c_double),
                 ("score_min", C.c_double), ("med_mean", C.c_double), ("ignore_zero", C.c_int32),
-                ("_pad", C.c_int32)]
+                ("fp64", C.c_int32)]
 
 
 # every symbol include/plaidgpu.h declares: name -> (restype, argtypes)

@@ -827,6 +827,14 @@ void ship_body(plaidgpu_ctx* c) {
     ++next;
   }
 }
+// forget the result blocks that left early: wait until their copies have landed, so that nothing overwrites the
+// raw scores under them, and let plaidgpu_score_finish ship every column
+int drop_early(plaidgpu_ctx* c) {
+  ship_join(c);
+  CK(cudaStreamSynchronize(c->copy_stream));
+  c->early_cols = 0;
+  return PLAIDGPU_OK;
+}
 // called by the scoring thread right after the kernels of a chunk were launched
 int ship_chunk(plaidgpu_ctx* c, int64_t j0, int64_t nj) {
   size_t k;
@@ -1356,6 +1364,11 @@ int plaidgpu_score_begin(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_
   if (!c->have_g) return fail(c, PLAIDGPU_ERR_STATE, "plaidgpu_set_genesets has not been called");
   trace("begin");
   CK(cudaSetDevice(c->device));
+  if (c->early_cols > 0) {  // the last call was computed but not finished (a shard or tile scored again in fp64 after
+    // another fell back): its early copies may still be reading the raw scores this call is about to overwrite
+    int rcd = drop_early(c);
+    if (rcd) return rcd;
+  }
   c->in_call = false;
   c->computed = false;
   c->opts = *opts;
@@ -1798,6 +1811,9 @@ int plaidgpu_score_compute(plaidgpu_ctx* c, plaidgpu_scalars* scal, double* out)
   scal->score_min = INFINITY;
   c->have_all = c->have_nz = false;
   c->raw_valid = true;
+  // did the fixed-point route give up (b_tcflag)?  Read with the score minimum when there is one, else in place of
+  // the stream synchronisation below.  b_tcflag is reserved with 8 bytes: the int flag sits in the low half.
+  unsigned long long flag = 0;
   if (c->need_norm) {
     // normalize_medians uses ONE of the two medians, chosen by min(x) == 0 over all shards (R/plaid.R:556-557).
     // The shard's own minimum (tracked by the score kernels) settles which: > 0 -> no zeros here, both medians
@@ -1805,8 +1821,8 @@ int plaidgpu_score_compute(plaidgpu_ctx* c, plaidgpu_scalars* scal, double* out)
     // median, unless another shard holds a negative score (then the plain one is computed on demand).
     unsigned long long key = ~0ull;
     {
-      const SmallRead it[1] = {{&key, c->b_smin.p, 1}};
-      int rcs = read_small(c, it, 1);
+      const SmallRead it[2] = {{&key, c->b_smin.p, 1}, {&flag, c->b_tcflag.p, use_tc ? 1 : 0}};
+      int rcs = read_small(c, it, 2);
       if (rcs) return rcs;
     }
     c->local_min = (key == ~0ull) ? INFINITY : host_value_of(key);
@@ -1826,20 +1842,17 @@ int plaidgpu_score_compute(plaidgpu_ctx* c, plaidgpu_scalars* scal, double* out)
     rc = fetch_medians(c);
     if (rc) return rc;
   }
-  CK(cudaStreamSynchronize(c->stream));
-  if (c->early_cols > 0) {
-    // a non-finite entry sent the call through the fp64 passes AFTER chunks had left: ship everything again
-    unsigned long long flag = 0;  // b_tcflag is reserved with 8 bytes: the int flag sits in the low half
-    {
-      const SmallRead it[1] = {{&flag, c->b_tcflag.p, 1}};
-      int rcs = read_small(c, it, 1);
-      if (rcs) return rcs;
-    }
-    if ((int)(flag & 0xFFFFFFFFull)) {
-      ship_join(c);
-      CK(cudaStreamSynchronize(c->copy_stream));
-      c->early_cols = 0;
-    }
+  if (use_tc && !c->need_norm) {
+    const SmallRead it[1] = {{&flag, c->b_tcflag.p, 1}};
+    int rcs = read_small(c, it, 1);
+    if (rcs) return rcs;
+  } else {
+    CK(cudaStreamSynchronize(c->stream));
+  }
+  scal->fp64 = (int32_t)(flag & 0xFFFFFFFFull) != 0;
+  if (scal->fp64) {  // the fp64 passes redid the scores AFTER chunks had left: ship everything again
+    int rcd = drop_early(c);
+    if (rcd) return rcd;
   }
   float ms = 0.f;
   cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]);
@@ -2093,8 +2106,9 @@ int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double*
 // The tile of columns [j0, j1) finishes into t.from(j0): its columns of the scores or of idx / val, or its group or
 // design moments, which are added to t.out (zeroed here) in tile order.  FILE_TILES stages every finished tile in a pinned
 // buffer and writes it to the file: tiled egress for results larger than host memory (scope row f4).
-static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
-                         const Target& t, int64_t chunk) {
+// One pass over the tiles; it stops with *fell_back set as soon as a tile leaves the fixed-point route.
+static int score_chunked_pass(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
+                              const Target& t, int64_t chunk, bool* fell_back) {
   const int64_t N = X->N;
   const int32_t S = c->S;
   std::vector<double> moments(t.moment_count(S));  // one tile's group or design moments
@@ -2142,6 +2156,10 @@ static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_
       plaidgpu_scalars s = g;
       rc = plaidgpu_score_compute(c, &s, nullptr);
       if (rc) return rc;
+      if (s.fp64) {
+        *fell_back = true;
+        return PLAIDGPU_OK;
+      }
       memcpy(ma.data() + j0, c->h_med_all.data(), (size_t)(j1 - j0) * sizeof(double));
       memcpy(mz.data() + j0, c->h_med_nz.data(), (size_t)(j1 - j0) * sizeof(double));
       smin = fmin(smin, s.score_min);
@@ -2169,6 +2187,10 @@ static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_
     plaidgpu_scalars s = g;
     rc = plaidgpu_score_compute(c, &s, nullptr);
     if (rc) return rc;
+    if (s.fp64) {
+      *fell_back = true;
+      return PLAIDGPU_OK;
+    }
     s.ignore_zero = g.ignore_zero;
     s.med_mean = g.med_mean;
     if (t.kind != Target::FILE_TILES) {
@@ -2192,6 +2214,21 @@ static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_
   if (writer.joinable()) writer.join();
   if (short_write) return fail(c, PLAIDGPU_ERR_ARG, "short write to the output file");
   return PLAIDGPU_OK;
+}
+
+// The tiles of one call all take the same route: when one of them falls back to the fp64 passes, the whole call is
+// scored again from tile 0 with exact_fp64 (a file is rewritten from its first tile), so the result does not depend
+// on the tiling.
+static int score_chunked(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
+                         const Target& t, int64_t chunk) {
+  const off_t start = t.file ? ftello(t.file) : 0;
+  bool fell_back = false;
+  int rc = score_chunked_pass(c, X, rowmap, opts, t, chunk, &fell_back);
+  if (rc || !fell_back) return rc;
+  plaidgpu_opts o = *opts;
+  o.exact_fp64 = 1;
+  if (t.file && fseeko(t.file, start, SEEK_SET) != 0) return fail(c, PLAIDGPU_ERR_ARG, "cannot rewind the output file");
+  return score_chunked_pass(c, X, rowmap, &o, t, chunk, &fell_back);
 }
 
 int plaidgpu_score_to_file(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
@@ -2471,10 +2508,26 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
         s.x_max = fmax(s.x_max, loc[k].x_max);
         s.rank_max = fmax(s.rank_max, loc[k].rank_max);
       }
+      const plaidgpu_scalars s_in = s;
       rc[r] = plaidgpu_score_compute(cr, &s, dst);
       loc[r].score_min = s.score_min;
+      loc[r].fp64 = s.fp64;
       bar.wait();
       if (failed()) return;
+      bool fell_back = false;
+      for (int k = 0; k < n; ++k) fell_back |= loc[k].fp64 != 0;
+      if (fell_back) {  // one shard left the fixed-point route: every shard scores in fp64, as one context would
+        if (!s.fp64) {
+          plaidgpu_scalars again;
+          o.exact_fp64 = 1;
+          rc[r] = plaidgpu_score_begin(cr, &M[r], rowmap, &o, &again);
+          s = s_in;
+          if (!rc[r]) rc[r] = plaidgpu_score_compute(cr, &s, dst);
+          loc[r].score_min = s.score_min;
+        }
+        bar.wait();
+        if (failed()) return;
+      }
       if (norm) {
         double smin = INFINITY;
         for (int k = 0; k < n; ++k) smin = fmin(smin, loc[k].score_min);

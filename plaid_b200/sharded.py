@@ -234,6 +234,25 @@ def combine_medians_of(ctx, comm, ignore_zero_opt: int, scal: L.Scalars, n_cols:
     return scal
 
 
+def compute_once_per_call(ctx, comm, M: L.Matrix, rowmap: np.ndarray, opts: L.Opts, scal: L.Scalars, out_ptr: int):
+    """step 3 (plaidgpu_score_compute) and 3b of the protocol: when any rank's fixed-point route gave up
+    (Scalars.fp64), the ranks that did not score their shard again with exact_fp64, so every column of the call
+    comes from the fp64 passes, as with one context.  Returns the scalars compute reported."""
+    lib = ctx.lib
+    s = L.Scalars()
+    C.memmove(C.byref(s), C.byref(scal), C.sizeof(L.Scalars))
+    ctx.check(lib.plaidgpu_score_compute(ctx.h, C.byref(s), out_ptr))
+    if opts.exact_fp64 or comm.allreduce_max(float(s.fp64)) == 0.0 or s.fp64:
+        return s
+    o = L.Opts()
+    C.memmove(C.byref(o), C.byref(opts), C.sizeof(L.Opts))
+    o.exact_fp64 = 1
+    ctx.check(lib.plaidgpu_score_begin(ctx.h, C.byref(M), rowmap.ctypes.data, C.byref(o), C.byref(L.Scalars())))
+    C.memmove(C.byref(s), C.byref(scal), C.sizeof(L.Scalars))
+    ctx.check(lib.plaidgpu_score_compute(ctx.h, C.byref(s), out_ptr))
+    return s
+
+
 def score_shard(ctx, comm, M: L.Matrix, rowmap: np.ndarray, opts: L.Opts, out_ptr: int, n_cols: int):
     """Run the begin / compute / finish protocol for this rank's column shard."""
     lib = ctx.lib
@@ -242,7 +261,7 @@ def score_shard(ctx, comm, M: L.Matrix, rowmap: np.ndarray, opts: L.Opts, out_pt
     # plaid() itself has no cross-shard scalar before the scores exist (x_min / x_max feed scse's removeLog2 switch,
     # rank_max the rank scorers): no collective, no host sync on its critical path
     scal = local if opts.scorer == L.PLAID else combine_scalars(comm, local)
-    ctx.check(lib.plaidgpu_score_compute(ctx.h, C.byref(scal), out_ptr))
+    scal = compute_once_per_call(ctx, comm, M, rowmap, opts, scal, out_ptr)
     needs_norm = (opts.scorer in (L.SSGSEA, L.UCELL, L.AUCELL, L.GSVA)) or (opts.scorer == L.PLAID and opts.normalize)
     if needs_norm:
         combine_medians_of(ctx, comm, opts.ignore_zero, scal, n_cols)
@@ -387,6 +406,16 @@ def score_multi(ctxs, mats, rowmap: np.ndarray, opts_list, out_ptrs, n_cols):
         C.memmove(C.byref(s), C.byref(g), C.sizeof(L.Scalars))
         c.check(lib.plaidgpu_score_compute(c.h, C.byref(s), outp))
         scal.append(s)
+    if any(s.fp64 for s in scal):  # step 3b: the shards still on the fixed-point route score again in fp64
+        for i, (c, M, o, outp) in enumerate(zip(ctxs, mats, opts_list, out_ptrs)):
+            if scal[i].fp64 or o.exact_fp64:
+                continue
+            o64 = L.Opts()
+            C.memmove(C.byref(o64), C.byref(o), C.sizeof(L.Opts))
+            o64.exact_fp64 = 1
+            c.check(lib.plaidgpu_score_begin(c.h, C.byref(M), rowmap.ctypes.data, C.byref(o64), C.byref(L.Scalars())))
+            C.memmove(C.byref(scal[i]), C.byref(g), C.sizeof(L.Scalars))
+            c.check(lib.plaidgpu_score_compute(c.h, C.byref(scal[i]), outp))
     o0 = opts_list[0]
     if (o0.scorer in (L.SSGSEA, L.UCELL, L.AUCELL, L.GSVA)) or (o0.scorer == L.PLAID and o0.normalize):
         smin = min(s.score_min for s in scal)

@@ -34,6 +34,7 @@ def test_struct_layouts_match_header():
     assert C.sizeof(L.Matrix) == 48
     assert C.sizeof(L.Opts) == 104
     assert C.sizeof(L.Scalars) == 48
+    assert L.Scalars.fp64.offset == 44 and L.Scalars.fp64.size == 4
     o = L.Opts()
     L.load().plaidgpu_default_opts(C.byref(o))
     assert (o.scorer, o.stats_mean, o.normalize, o.ignore_zero, o.remove_log2, o.rmax) == (0, 1, 1, -1, -1, 1500.0)
