@@ -353,6 +353,30 @@ int plaidgpu_score_topk(plaidgpu_ctx* ctx, const plaidgpu_matrix* X, const int32
 int plaidgpu_score_topk_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
                               const plaidgpu_opts* opts, int k, int decreasing, int32_t* idx, double* val);
 
+/* Per row of a dense S x N matrix at `location`: the k largest (decreasing = 1) or smallest values and their column
+ * indices, i.e. the first k entries of R's order(x[s, ], decreasing = decreasing): ties (fp64 ==, so -0 == +0) by
+ * ascending column, NaN last in both directions and by ascending column.  idx int64[k * S] (0-based columns) and
+ * val double[k * S] (val = x[s, idx] bit for bit), host, column-major: entry t of set s at t + k * s.
+ * 1 <= k <= min(N, 256), otherwise PLAIDGPU_ERR_ARG.  Kernel time: plaidgpu_last_kernel_ms(, 2). */
+int plaidgpu_row_topk(plaidgpu_ctx* ctx, const double* x, int32_t S, int64_t N, int k, int decreasing,
+                      int location, int64_t* idx, double* val);
+
+/* The same fused onto the scoring call, for any scorer and option plaidgpu_score accepts: the scores stay on the
+ * device as raw scores and are normalised in registers while selecting; k * S indices and values come back.  Equal,
+ * bit for bit, to plaidgpu_score followed by plaidgpu_row_topk, with 1 <= k <= min(N, 256) for the N columns of X.
+ * When X is in host memory and the S x N scores exceed the device, the columns are scored in tiles (two passes over X
+ * when normalised, like plaidgpu_score) and the tiles' lists are merged; a tile that falls back to the fp64 passes
+ * scores the call again from its first tile, and the lists gathered before are discarded. */
+int plaidgpu_score_row_topk(plaidgpu_ctx* ctx, const plaidgpu_matrix* X, const int32_t* rowmap,
+                            const plaidgpu_opts* opts, int k, int decreasing, int64_t* idx, double* val);
+
+/* plaidgpu_score_row_topk over n devices from ONE host process, split like plaidgpu_score_multi: every shard selects
+ * over its own columns and the shards' lists are merged on the host (the result does not depend on n).  Each
+ * shard's scores must fit its device.  The same context twice, or gsva rowtf = "ecdf" with n > 1, is
+ * PLAIDGPU_ERR_ARG. */
+int plaidgpu_score_row_topk_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
+                                  const plaidgpu_opts* opts, int k, int decreasing, int64_t* idx, double* val);
+
 /* ---- gene-set ingestion ("next" row f2): host-side, no GPU needed -------------------------- */
 
 /* read.gmt() + gmt2mat() with default arguments (reference R/gmt-utils.R:99-125, 19-66): a GMT text

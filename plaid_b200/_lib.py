@@ -71,6 +71,8 @@ SYMBOLS = {
                                                     C.c_void_p, C.c_int, C.c_void_p]),
     "plaidgpu_col_topk": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                     C.c_void_p]),
+    "plaidgpu_row_topk": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                    C.c_void_p]),
     "plaidgpu_normalize_medians": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
     "plaidgpu_gmt_read": (C.c_int, [C.c_char_p, C.POINTER(C.c_void_p)]),
     "plaidgpu_gmt_from_buffer": (C.c_int, [C.c_char_p, C.c_int64, C.POINTER(C.c_void_p)]),
@@ -109,6 +111,10 @@ SYMBOLS = {
                                        C.c_void_p]),
     "plaidgpu_score_topk_multi": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                              C.c_int, C.c_void_p, C.c_void_p]),
+    "plaidgpu_score_row_topk": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                          C.c_void_p, C.c_void_p]),
+    "plaidgpu_score_row_topk_multi": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "plaidgpu_score_multi": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "plaidgpu_tc_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "plaidgpu_tail_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),

@@ -613,6 +613,60 @@ def score_topk(X: NamedMatrix, matG: NamedMatrix, k=10, decreasing=True, *, ctx=
     return idx, val
 
 
+def row_topk(gsetX, k=10, decreasing=True, *, ctx=None):
+    """Per row of a dense S x N matrix: the first k entries of R's `order(x[s, ], decreasing = decreasing)`, i.e. the
+    k largest (or smallest) values with ties by ascending column and NaN last (`plaidgpu_row_topk`).  `gsetX` is a 2-D
+    array or a `DeviceDense` (S x N in device memory).  Returns (idx, val) of shape (k, S): 0-based column indices
+    (int64) and the values at those columns, bit for bit."""
+    ctx = ctx or default_context()
+    S, N, loc, ptr, keep = _dense_input(gsetX)
+    idx = np.empty((max(int(k), 0), S), dtype=np.int64, order="F")  # a bad k is the library's error
+    val = np.empty((max(int(k), 0), S), dtype=np.float64, order="F")
+    ctx.check(ctx.lib.plaidgpu_row_topk(ctx.h, ptr, S, N, int(k), 1 if decreasing else 0, loc, idx.ctypes.data,
+                                        val.ctypes.data))
+    del keep
+    return idx, val
+
+
+def score_row_topk(X: NamedMatrix, matG: NamedMatrix, k=10, decreasing=True, *, ctx=None, **opts_kw):
+    """plaid() (or another scorer through `opts_kw`) fused with row_topk (`plaidgpu_score_row_topk`): each gene set's
+    k best cells, while the S x N scores stay on the device.  Equal, bit for bit, to scoring followed by row_topk.
+    `ctx` may be a list of Contexts on different devices: the columns are then split over them and the lists merged
+    (`plaidgpu_score_row_topk_multi`).  Returns (idx, val) of shape (k, S), or None on no overlap."""
+    ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else None
+    ctx = (ctxs[0] if ctxs else ctx) or default_context()
+    if X.rownames is None or matG.rownames is None:
+        _message("[plaid] ERROR. No overlapping features.")
+        return None
+    rowmap = make_rowmap(X.rownames, matG.rownames)
+    if not (rowmap >= 0).any():
+        _message("[plaid] ERROR. No overlapping features.")
+        return None
+    for cx in (ctxs or [ctx]):
+        cx.set_genesets(matG.mat)
+    keep: list = []
+    M = _matrix_struct(X.mat, keep)
+    kw = dict(scorer=L.PLAID, stats_mean=1, normalize=1)
+    kw.update(opts_kw)
+    o = _opts(ctx.lib, **kw)
+    S = int(matG.mat.shape[1])
+    idx = np.empty((max(int(k), 0), S), dtype=np.int64, order="F")
+    val = np.empty((max(int(k), 0), S), dtype=np.float64, order="F")
+    dec = 1 if decreasing else 0
+    if ctxs and len(ctxs) > 1:
+        hs = (C.c_void_p * len(ctxs))(*[cx.h for cx in ctxs])
+        rc = ctx.lib.plaidgpu_score_row_topk_multi(hs, len(ctxs), C.byref(M), rowmap.ctypes.data, C.byref(o), int(k),
+                                                   dec, idx.ctypes.data, val.ctypes.data)
+    else:
+        rc = ctx.lib.plaidgpu_score_row_topk(ctx.h, C.byref(M), rowmap.ctypes.data, C.byref(o), int(k), dec,
+                                             idx.ctypes.data, val.ctypes.data)
+    if rc == L.ERR_NOOVERLAP:
+        _message("[plaid] ERROR. No overlapping features.")
+        return None
+    ctx.check(rc)
+    return idx, val
+
+
 def _design_basis(B, n):
     b = np.asarray(B, dtype=np.float64)
     if b.ndim == 1:

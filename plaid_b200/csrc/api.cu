@@ -1097,6 +1097,76 @@ int topk_device(plaidgpu_ctx* c, const double* dx, int32_t S, int64_t N, int k, 
   return PLAIDGPU_OK;
 }
 
+// ---- per-row top k (plaid.topcells) ---------------------------------------------------------
+// k over the N columns of the whole call
+int check_row_topk(plaidgpu_ctx* c, int64_t N, int k) {
+  if (k < 1 || k > TOPK_MAX || k > N)
+    return fail(c, PLAIDGPU_ERR_ARG, "k = " + std::to_string(k) + " is outside [1, min(N = " + std::to_string(N) +
+                                         ", " + std::to_string(TOPK_MAX) + ")]");
+  return PLAIDGPU_OK;
+}
+
+// Each row's top k of the S x N device matrix dx (ld = S) into host idx / val[k * S], idx = col0 + column (checked
+// k; when N < k the last entries are empty: idx -1, val NaN).  The column chunks follow reduce_nchunk with the
+// partial lists (16 bytes an entry) as the width.  Kernel time in ms[2].  fix / med / cc / alpha / beta: the fix-up
+// of plaidgpu_score_finish, applied in registers to raw scores.
+int row_topk_device(plaidgpu_ctx* c, const double* dx, int32_t S, int64_t N, int k, int decreasing, int64_t col0,
+                    int64_t* idx, double* val, bool fix = false, const double* med = nullptr, double cc = 0.0,
+                    double alpha = 1.0, const double* beta = nullptr) {
+  const size_t n = (size_t)k * (size_t)S;
+  const int nchunk = reduce_nchunk(N, 2 * (int64_t)n);
+  CK(c->b_rowa.reserve(2 * (size_t)nchunk * n * sizeof(uint64_t)));
+  CK(c->b_rowb.reserve(n * (sizeof(int64_t) + sizeof(double))));
+  int64_t* didx = c->b_rowb.as<int64_t>();
+  double* dval = reinterpret_cast<double*>(didx + n);
+  CK(cudaEventRecord(c->ev[4], c->stream));
+  CK(launch_row_topk(dx, S, S, N, k, decreasing, nchunk, c->b_rowa.as<uint64_t>(), col0, didx, dval, c->stream, fix,
+                     med, cc, alpha, beta));
+  c->launches += 2;
+  CK(cudaEventRecord(c->ev[5], c->stream));
+  CK(cudaMemcpyAsync(idx, didx, n * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(val, dval, n * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  float ms = 0.f;
+  cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]);
+  c->ms[2] = ms;
+  return PLAIDGPU_OK;
+}
+
+// The order of the device's selection key (topk_select.cuh) on final values: larger first (smaller when
+// !decreasing), -0 == +0, NaN after every number, equal values by ascending column.  An empty entry (column -1,
+// value NaN) compares as the largest column, after every NaN.
+uint64_t host_order_key(double v, bool decreasing) {
+  if (v != v) return 0;
+  uint64_t b = 0;
+  if (v != 0.0) memcpy(&b, &v, sizeof(b));
+  b = (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+  return decreasing ? b : ~b;
+}
+
+// Merges the row top-k lists b into a (k * S each, sorted, with distinct columns): a becomes each row's k best of
+// both.  The order is total, so merging tiles or shards in any grouping gives the same lists.
+void merge_row_topk(int32_t S, int k, bool decreasing, int64_t* ai, double* av, const int64_t* bi, const double* bv) {
+  std::vector<int64_t> ti((size_t)k);
+  std::vector<double> tv((size_t)k);
+  for (int32_t s = 0; s < S; ++s) {
+    int64_t* ri = ai + (size_t)k * s;
+    double* rv = av + (size_t)k * s;
+    const int64_t* qi = bi + (size_t)k * s;
+    const double* qv = bv + (size_t)k * s;
+    int x = 0, y = 0;
+    for (int t = 0; t < k; ++t) {
+      const uint64_t kx = host_order_key(rv[x], decreasing), ky = host_order_key(qv[y], decreasing);
+      const bool take_b = ky > kx || (ky == kx && (uint64_t)qi[y] < (uint64_t)ri[x]);
+      ti[t] = take_b ? qi[y] : ri[x];
+      tv[t] = take_b ? qv[y] : rv[x];
+      take_b ? ++y : ++x;
+    }
+    std::copy(ti.begin(), ti.end(), ri);
+    std::copy(tv.begin(), tv.end(), rv);
+  }
+}
+
 // Host X and host output larger than the device can hold: the column tile width score_chunked should use, or 0
 // when one pass fits (the raw scores get 45 % of the free memory; X, ranks and slack share the rest)
 int host_chunk_cols(plaidgpu_ctx* c, const plaidgpu_matrix* X, int64_t* chunk) {
@@ -1132,10 +1202,18 @@ plaidgpu_matrix column_slice(const plaidgpu_matrix* X, int64_t j0, int64_t j1, s
   return M;
 }
 
+// A column tile's or a shard's share of a result the whole call reduces: its group or design moments, or each row's
+// top-k list.  Target::from sizes it and Target::combine folds it into the call's result.
+struct Partial {
+  std::vector<double> moments;
+  std::vector<int64_t> cols;
+  std::vector<double> val;
+};
+
 // What the finish step of a scoring call makes of the raw S x N scores.  Every kind but SCORES keeps the raw scores
 // in the library's device buffer (out_location = PLAIDGPU_HOST) and applies the fix-up in registers.
 struct Target {
-  enum Kind { SCORES, GROUP_STATS, DESIGN_STATS, TOPK, FILE_TILES } kind = SCORES;
+  enum Kind { SCORES, GROUP_STATS, DESIGN_STATS, TOPK, ROW_TOPK, FILE_TILES } kind = SCORES;
   double* out = nullptr;            // SCORES: the S x N scores at opts.out_location; GROUP_STATS: K * 2 * S moments;
                                     // DESIGN_STATS: (Q + 2) * S moments
   const int32_t* labels = nullptr;  // GROUP_STATS: int32[N] in [-1, K)
@@ -1143,8 +1221,10 @@ struct Target {
   const double* B = nullptr;        // DESIGN_STATS: host, column-major N x Q, leading dimension ldb
   int64_t ldb = 0;
   int Q = 0;
-  int k = 0, decreasing = 0;        // TOPK: idx / val hold k * N entries
+  int k = 0, decreasing = 0;        // TOPK: idx / val hold k * N entries; ROW_TOPK: cols / val hold k * S entries
   int32_t* idx = nullptr;
+  int64_t* cols = nullptr;          // ROW_TOPK: columns of the call; this target's column 0 is column col0
+  int64_t col0 = 0;
   double* val = nullptr;
   FILE* file = nullptr;             // FILE_TILES (score_chunked): tile t is staged in stage[t & 1] (stage[0] when
   double* stage[2] = {};            // stage[1] is null) and written to `file` by a helper thread
@@ -1159,33 +1239,54 @@ struct Target {
   static Target topk(int k, int decreasing, int32_t* idx, double* val) {
     Target t; t.kind = TOPK; t.k = k; t.decreasing = decreasing != 0; t.idx = idx; t.val = val; return t;
   }
+  static Target row_topk(int k, int decreasing, int64_t* cols, double* val) {
+    Target t; t.kind = ROW_TOPK; t.k = k; t.decreasing = decreasing != 0; t.cols = cols; t.val = val; return t;
+  }
   static Target to_file(FILE* file, double* stage0, double* stage1) {
     Target t; t.kind = FILE_TILES; t.file = file; t.stage[0] = stage0; t.stage[1] = stage1; return t;
   }
-  // doubles of moments a GROUP_STATS / DESIGN_STATS target returns (0 for the other kinds)
-  size_t moment_count(int32_t S) const {
-    if (kind == GROUP_STATS) return (size_t)K * 2 * (size_t)S;
-    if (kind == DESIGN_STATS) return (size_t)(Q + 2) * (size_t)S;
-    return 0;
+  // the result before any tile or shard is combined into it: zero moments, empty row lists
+  void clear(int32_t S) const {
+    if (kind == GROUP_STATS) std::fill(out, out + (size_t)K * 2 * (size_t)S, 0.0);
+    if (kind == DESIGN_STATS) std::fill(out, out + (size_t)(Q + 2) * (size_t)S, 0.0);
+    if (kind == ROW_TOPK) {
+      std::fill(cols, cols + (size_t)k * (size_t)S, (int64_t)-1);
+      std::fill(val, val + (size_t)k * (size_t)S, NAN);
+    }
   }
-  // the same target for the columns from j0 on; group and design statistics write those columns' moments to
-  // `moments`
-  Target from(int64_t j0, int32_t S, double* moments) const {
+  // the same target for the columns from j0 on: their columns of the scores or of idx / val; the group or design
+  // moments or row lists of a reduced kind go to p, for combine
+  Target from(int64_t j0, int32_t S, Partial& p) const {
     Target t = *this;
     if (kind == SCORES) t.out = out + j0 * (int64_t)S;
     if (kind == GROUP_STATS) {
+      p.moments.resize((size_t)K * 2 * (size_t)S);
       t.labels = labels + j0;
-      t.out = moments;
+      t.out = p.moments.data();
     }
     if (kind == DESIGN_STATS) {
+      p.moments.resize((size_t)(Q + 2) * (size_t)S);
       t.B = B + j0;  // rows j0.. of B, same leading dimension
-      t.out = moments;
+      t.out = p.moments.data();
     }
     if (kind == TOPK) {
       t.idx = idx + j0 * k;
       t.val = val + j0 * k;
     }
+    if (kind == ROW_TOPK) {
+      p.cols.resize((size_t)k * (size_t)S);
+      p.val.resize((size_t)k * (size_t)S);
+      t.cols = p.cols.data();
+      t.val = p.val.data();
+      t.col0 = col0 + j0;
+    }
     return t;
+  }
+  // folds the partial result of a tile or shard into the call's result: moments are added (in the order of the
+  // calls), row lists merged by the selection order
+  void combine(const Partial& p, int32_t S) const {
+    for (size_t i = 0; i < p.moments.size(); ++i) out[i] += p.moments[i];
+    if (kind == ROW_TOPK) merge_row_topk(S, k, decreasing != 0, cols, val, p.cols.data(), p.val.data());
   }
 };
 
@@ -1918,7 +2019,7 @@ int plaidgpu_combine_medians(int ignore_zero_opt, double score_min, const double
   return PLAIDGPU_ERR_ARG;
 }
 
-// plaidgpu_score_finish into target t (SCORES, GROUP_STATS, DESIGN_STATS or TOPK)
+// plaidgpu_score_finish into target t (SCORES, GROUP_STATS, DESIGN_STATS, TOPK or ROW_TOPK)
 static int score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, const Target& t) try {
   if (t.kind == Target::SCORES && !t.out && c->N > 0) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
   if (!c->computed) return fail(c, PLAIDGPU_ERR_STATE, "plaidgpu_score_compute has not been called");
@@ -1952,11 +2053,13 @@ static int score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, const Tar
   }
 
   // the reductions read the raw scores with the fix-up applied in registers: the S x N matrix stays on the device
-  // and only K * 2 * S or (Q + 2) * S moments, or k * N indices and values, go back
+  // and only K * 2 * S or (Q + 2) * S moments, or k * N or k * S indices and values, go back
   if (t.kind == Target::GROUP_STATS) return group_stats_device(c, c->raw, S, N, t.labels, t.K, t.out, fix, med, cc, alpha, beta);
   if (t.kind == Target::DESIGN_STATS)
     return design_stats_device(c, c->raw, S, N, t.B, t.ldb, t.Q, t.out, fix, med, cc, alpha, beta);
   if (t.kind == Target::TOPK) return topk_device(c, c->raw, S, N, t.k, t.decreasing, t.idx, t.val, fix, med, cc, alpha, beta);
+  if (t.kind == Target::ROW_TOPK)
+    return row_topk_device(c, c->raw, S, N, t.k, t.decreasing, t.col0, t.cols, t.val, fix, med, cc, alpha, beta);
   double* out = t.out;
   c->raw_valid = false;  // the fix-up below rewrites the raw scores in place
   CK(cudaEventRecord(c->ev[4], c->stream));
@@ -2104,15 +2207,15 @@ int plaidgpu_score_finish(plaidgpu_ctx* c, const plaidgpu_scalars* scal, double*
 // pass 2 recomputes, fixes up and streams each chunk out (recomputing costs less than moving the raw
 // scores over PCIe twice).  Results are bit-identical to the un-chunked path.
 // The tile of columns [j0, j1) finishes into t.from(j0): its columns of the scores or of idx / val, or its group or
-// design moments, which are added to t.out (zeroed here) in tile order.  FILE_TILES stages every finished tile in a pinned
+// design moments or row top-k lists, which t.combine folds into the result (cleared here) in tile order.  FILE_TILES stages every finished tile in a pinned
 // buffer and writes it to the file: tiled egress for results larger than host memory (scope row f4).
 // One pass over the tiles; it stops with *fell_back set as soon as a tile leaves the fixed-point route.
 static int score_chunked_pass(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
                               const Target& t, int64_t chunk, bool* fell_back) {
   const int64_t N = X->N;
   const int32_t S = c->S;
-  std::vector<double> moments(t.moment_count(S));  // one tile's group or design moments
-  std::fill(t.out, t.out + moments.size(), 0.0);
+  Partial part;  // one tile's moments or row lists
+  t.clear(S);     // a pass scored again after a fallback starts over
   if (opts->scorer == PLAIDGPU_GSVA && opts->gsva_ecdf != PLAIDGPU_ROWTF_DONE &&
       (opts->gsva_ecdf || !(opts->row_mean && opts->row_sd)))
     return fail(c, PLAIDGPU_ERR_ARG, "replaid.gsva: matrix too large for one device pass (rowtf ecdf needs all samples; rowtf z needs row_mean / row_sd)");
@@ -2194,9 +2297,9 @@ static int score_chunked_pass(plaidgpu_ctx* c, const plaidgpu_matrix* X, const i
     s.ignore_zero = g.ignore_zero;
     s.med_mean = g.med_mean;
     if (t.kind != Target::FILE_TILES) {
-      rc = score_finish(c, &s, t.from(j0, S, moments.data()));
+      rc = score_finish(c, &s, t.from(j0, S, part));
       if (rc) return rc;
-      for (size_t i = 0; i < moments.size(); ++i) t.out[i] += moments[i];
+      t.combine(part, S);
       continue;
     }
     double* dst = (t.stage[1] && (tile & 1)) ? t.stage[1] : t.stage[0];
@@ -2384,6 +2487,24 @@ int plaidgpu_score_topk(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t
   return PLAIDGPU_ERR_ARG;
 }
 
+// score -> top cells fused: plaid() / a replaid.* scorer followed by each set's top k columns (plaid.topcells) without
+// the S x N matrix leaving the device or being written in its normalised form.  Bit-identical to plaidgpu_score +
+// plaidgpu_row_topk.  Host X whose S x N scores exceed the device is scored in column tiles whose lists are merged in
+// tile order.
+int plaidgpu_score_row_topk(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
+                            int k, int decreasing, int64_t* idx, double* val) try {
+  if (!c) return PLAIDGPU_ERR_ARG;
+  if (!X || !rowmap || !opts || !idx || !val) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  if (!c->have_g) return fail(c, PLAIDGPU_ERR_STATE, "plaidgpu_set_genesets has not been called");
+  int rc = check_row_topk(c, X->N, k);
+  if (rc) return rc;
+  return score_one(c, X, rowmap, opts, Target::row_topk(k, decreasing, idx, val));
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
 // two groups y != 0 / y == 0: the labels of plaidgpu_score_group_stats with K = 2
 int plaidgpu_score_group_moments(plaidgpu_ctx* c, const plaidgpu_matrix* X, const int32_t* rowmap, const plaidgpu_opts* opts,
                                  const int32_t* y, double* out) try {
@@ -2439,8 +2560,8 @@ static int check_shard_ctxs(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_opt
 }
 
 // Shard r (columns [lo_r, lo_{r+1})) finishes on ctxs[r] into t.from(lo_r): its block of the scores, its columns of
-// idx / val, or its own group or design moments, of which shard 0's are copied to t.out and shards 1 to n - 1 added
-// in shard order.
+// idx / val, or its own group or design moments or row top-k lists, which t.combine folds into the result in shard
+// order.  After a fallback only the lists of the fp64 route exist: finish runs once per shard, after the rerun.
 static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
                             const plaidgpu_opts* opts, const Target& t, const std::string& who) {
   plaidgpu_ctx* c = ctxs[0];
@@ -2456,8 +2577,7 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
     for (int r = 0; r < n; ++r) M[r] = column_slice(X, lo[r], lo[r + 1], pbuf[r]);
     std::vector<plaidgpu_scalars> loc((size_t)n);
     std::vector<int> rc((size_t)n, PLAIDGPU_OK);
-    const size_t width = t.moment_count(S);
-    std::vector<std::vector<double>> moments((size_t)n, std::vector<double>(width));
+    std::vector<Partial> parts((size_t)n);
     std::vector<double> med((size_t)std::max<int64_t>(N, 1));
     std::vector<std::vector<double>> part(gsva_z ? (size_t)n : 0, std::vector<double>((size_t)P));
     std::vector<double> rmean(gsva_z ? (size_t)P : 0), rsd(gsva_z ? (size_t)P : 0);
@@ -2473,7 +2593,7 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
       plaidgpu_ctx* cr = ctxs[r];
       plaidgpu_opts o = *opts;
       if (t.kind != Target::SCORES) o.out_location = PLAIDGPU_HOST;  // raw scores stay in the context's device buffer
-      const Target tr = t.from(lo[r], S, moments[r].data());
+      const Target tr = t.from(lo[r], S, parts[r]);
       double* dst = t.kind == Target::SCORES ? tr.out : nullptr;
       if (gsva_z) {  // rowMeans / rowSds over ALL shards, summed in shard order (R/plaid.R:343)
         rc[r] = plaidgpu_row_moments(cr, &M[r], nullptr, part[r].data());
@@ -2553,11 +2673,8 @@ static int score_multi_impl(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_mat
         if (r > 0) c->err = "shard " + std::to_string(r) + ": " + ctxs[r]->err;
         return rc[r];
       }
-    if (width) {
-      std::copy(moments[0].begin(), moments[0].end(), t.out);
-      for (int r = 1; r < n; ++r)
-        for (size_t i = 0; i < width; ++i) t.out[i] += moments[r][i];
-    }
+    t.clear(S);
+    for (int r = 0; r < n; ++r) t.combine(parts[r], S);
     return PLAIDGPU_OK;
   } catch (const std::bad_alloc&) {
     return fail(c, PLAIDGPU_ERR_NOMEM, "out of host memory");
@@ -2581,11 +2698,13 @@ static int score_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* 
     if (t.kind == Target::GROUP_STATS) return plaidgpu_score_group_stats(c, X, rowmap, opts, t.labels, t.K, t.out);
     if (t.kind == Target::DESIGN_STATS) return plaidgpu_score_design_stats(c, X, rowmap, opts, t.B, t.Q, t.out);
     if (t.kind == Target::TOPK) return plaidgpu_score_topk(c, X, rowmap, opts, t.k, t.decreasing, t.idx, t.val);
+    if (t.kind == Target::ROW_TOPK) return plaidgpu_score_row_topk(c, X, rowmap, opts, t.k, t.decreasing, t.cols, t.val);
     return plaidgpu_score(c, X, rowmap, opts, t.out);
   }
   if (t.kind == Target::GROUP_STATS) rc = check_groups(c, t.labels, X->N, t.K);
   if (t.kind == Target::DESIGN_STATS) rc = check_design(c, t.B, X->N, t.ldb, t.Q);
   if (t.kind == Target::TOPK) rc = check_topk(c, c->S, t.k);
+  if (t.kind == Target::ROW_TOPK) rc = check_row_topk(c, X->N, t.k);
   if (rc) return rc;
   return score_multi_impl(ctxs, n, X, rowmap, opts, t, who);
 }
@@ -2628,6 +2747,17 @@ int plaidgpu_score_topk_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_m
   if (!ctxs || n <= 0 || !ctxs[0]) return PLAIDGPU_ERR_ARG;
   if (!X || !rowmap || !opts || !idx || !val) return fail(ctxs[0], PLAIDGPU_ERR_ARG, "null argument");
   return score_multi(ctxs, n, X, rowmap, opts, Target::topk(k, decreasing, idx, val), "plaidgpu_score_topk_multi");
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
+int plaidgpu_score_row_topk_multi(plaidgpu_ctx* const* ctxs, int n, const plaidgpu_matrix* X, const int32_t* rowmap,
+                                  const plaidgpu_opts* opts, int k, int decreasing, int64_t* idx, double* val) try {
+  if (!ctxs || n <= 0 || !ctxs[0]) return PLAIDGPU_ERR_ARG;
+  if (!X || !rowmap || !opts || !idx || !val) return fail(ctxs[0], PLAIDGPU_ERR_ARG, "null argument");
+  return score_multi(ctxs, n, X, rowmap, opts, Target::row_topk(k, decreasing, idx, val), "plaidgpu_score_row_topk_multi");
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {
@@ -2866,6 +2996,29 @@ int plaidgpu_col_topk(plaidgpu_ctx* c, const double* x, int32_t S, int64_t N, in
     dx = c->b_raw.as<double>();
   }
   return topk_device(c, dx, S, N, k, decreasing != 0, idx, val);
+} catch (const std::bad_alloc&) {
+  return PLAIDGPU_ERR_NOMEM;
+} catch (...) {
+  return PLAIDGPU_ERR_ARG;
+}
+
+int plaidgpu_row_topk(plaidgpu_ctx* c, const double* x, int32_t S, int64_t N, int k, int decreasing, int location,
+                      int64_t* idx, double* val) try {
+  if (!c) return PLAIDGPU_ERR_ARG;
+  if (S <= 0 || N < 0) return fail(c, PLAIDGPU_ERR_ARG, "bad argument");
+  if (!x || !idx || !val) return fail(c, PLAIDGPU_ERR_ARG, "null argument");
+  if (location != PLAIDGPU_HOST && location != PLAIDGPU_DEVICE) return fail(c, PLAIDGPU_ERR_ARG, "unknown location");
+  int rc = check_row_topk(c, N, k);
+  if (rc) return rc;
+  CK(cudaSetDevice(c->device));
+  const double* dx = x;
+  if (location == PLAIDGPU_HOST) {
+    const size_t total = (size_t)S * (size_t)N;
+    CK(c->b_raw.reserve(total * sizeof(double)));
+    CK(cudaMemcpyAsync(c->b_raw.p, x, total * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    dx = c->b_raw.as<double>();
+  }
+  return row_topk_device(c, dx, S, N, k, decreasing != 0, 0, idx, val);
 } catch (const std::bad_alloc&) {
   return PLAIDGPU_ERR_NOMEM;
 } catch (...) {

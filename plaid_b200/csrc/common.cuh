@@ -206,6 +206,15 @@ constexpr int TOPK_MAX = 256;
 cudaError_t launch_col_topk(const double* x, int64_t ld, int32_t S, int64_t N, int k, int decreasing, int32_t* idx,
                             double* val, cudaStream_t st, bool fix = false, const double* med = nullptr, double c = 0.0,
                             double alpha = 1.0, const double* beta = nullptr);
+// per row of a column-major S x N matrix: the k (1 <= k <= TOPK_MAX) columns first in R's order(x[s, ], decreasing =
+// decreasing) (ties by ascending column, NaN last) into idx / val[k * S] (device, column-major: entry t of row s at
+// t + k * s; idx = col0 + column).  When N < k the last k - N entries are "no entry": idx -1, val NaN.
+// The columns are split into nchunk chunks (the N * c / nchunk split); partial = 2 * nchunk * S * k words of scratch
+// for the chunks' lists, merged by a second launch.  fix: as for launch_col_topk
+cudaError_t launch_row_topk(const double* x, int64_t ld, int32_t S, int64_t N, int k, int decreasing, int nchunk,
+                            uint64_t* partial, int64_t col0, int64_t* idx, double* val, cudaStream_t st, bool fix = false,
+                            const double* med = nullptr, double c = 0.0, double alpha = 1.0,
+                            const double* beta = nullptr);
 // nwords 8-byte words device -> host-mapped (cudaHostAllocMapped) memory by a kernel, bypassing the copy engine
 cudaError_t launch_copy_words(const void* src, void* dst_mapped, int64_t nwords, cudaStream_t st);
 // global min / max of a device array of n doubles, NaN ignored (na.rm = TRUE); res[0]=min res[1]=max
@@ -273,6 +282,15 @@ __device__ __forceinline__ double score_epilogue(double v, int s, int64_t j, dou
   if (mode >= XF_SING) v += fb * ns[s];
   v *= inv[s];
   if (colscale) v *= colscale[j];
+  return v;
+}
+
+// k_fixup's operations, in its order, on one raw score v of column j (b = beta[row], read once by the caller)
+__device__ __forceinline__ double fixup_value(double v, int64_t j, const double* __restrict__ med, double c, double alpha,
+                                              const double* __restrict__ beta, double b) {
+  const double shift = (med ? -med[j] : 0.0) + c;
+  v = __dmul_rn(alpha, __dadd_rn(v, shift));
+  if (beta) v = __dadd_rn(v, b);
   return v;
 }
 

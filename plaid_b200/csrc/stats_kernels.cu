@@ -1100,15 +1100,6 @@ __global__ void __launch_bounds__(256) k_minmax(const double* __restrict__ x, in
   }
 }
 
-// k_fixup's operations, in its order, on one raw score v of column j (b = beta[row], read once by the caller)
-__device__ __forceinline__ double fixup_value(double v, int64_t j, const double* __restrict__ med, double c, double alpha,
-                                              const double* __restrict__ beta, double b) {
-  const double shift = (med ? -med[j] : 0.0) + c;
-  v = __dmul_rn(alpha, __dadd_rn(v, shift));
-  if (beta) v = __dadd_rn(v, b);
-  return v;
-}
-
 // row sums / sums of squares of a column-major S x N matrix by column group (labels in [0, K); unlabelled columns
 // take no part).  The host sorts the labelled columns by (chunk, group), ascending inside each group, into `cols`;
 // segment g = chunk * K + group is cols[seg[g] .. seg[g + 1]).  grid = (segments, row blocks): each thread owns one

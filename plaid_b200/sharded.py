@@ -319,6 +319,53 @@ def score_topk_shard(ctx, comm, M: L.Matrix, rowmap: np.ndarray, opts: L.Opts, k
     return idx, val
 
 
+def merge_row_topk(lists, k: int, decreasing: bool):
+    """Each row's k best of several (idx, val) row top-k lists of shape (k, S) over disjoint columns, in the order of
+    plaidgpu_row_topk: larger values first (smaller when not decreasing), -0 == +0, NaN after every number, equal values
+    by ascending column; an empty entry (column -1) after everything."""
+    idx = np.concatenate([np.asarray(i, dtype=np.int64) for i, _ in lists], axis=0)
+    val = np.concatenate([np.asarray(v, dtype=np.float64) for _, v in lists], axis=0)
+    nan = np.isnan(val)
+    v = np.where(nan, 0.0, val) + 0.0  # -0 -> +0
+    col = idx.astype(np.uint64)         # -1 (empty) -> the largest column
+    out_i = np.empty((k, idx.shape[1]), dtype=np.int64, order="F")
+    out_v = np.empty((k, idx.shape[1]), dtype=np.float64, order="F")
+    for s in range(idx.shape[1]):
+        o = np.lexsort((col[:, s], -v[:, s] if decreasing else v[:, s], nan[:, s]))[:k]
+        out_i[:, s] = idx[o, s]
+        out_v[:, s] = val[o, s]
+    return out_i, out_v
+
+
+def score_row_topk_shard(ctx, comm, M: L.Matrix, rowmap: np.ndarray, opts: L.Opts, k: int, decreasing: bool, n_cols: int,
+                         col0: int):
+    """Each gene set's k best cells over all ranks: score_shard into a device buffer, plaidgpu_row_topk on it, the
+    indices shifted by this shard's first global column col0, then one all-gather of the lists, merged in rank order
+    with the selection's order (merge_row_topk).  k may exceed n_cols (the shard's lists then end in empty entries)
+    but not the total column count.  `ctx` must hold the gene sets (Context.set_genesets).  Every rank returns the same
+    (idx, val) of shape (k, S)."""
+    import torch
+    S = ctx.n_sets
+    buf = torch.empty(max(S * n_cols, 1), dtype=torch.float64, device=f"cuda:{ctx.device}")
+    opts.out_location = L.DEVICE
+    score_shard(ctx, comm, M, rowmap, opts, buf.data_ptr(), n_cols)
+    kk = min(int(k), n_cols)
+    idx = np.full((int(k), S), -1, dtype=np.int64, order="F")
+    val = np.full((int(k), S), np.nan, order="F")
+    if kk > 0:
+        i = np.empty((kk, S), dtype=np.int64, order="F")
+        v = np.empty((kk, S), dtype=np.float64, order="F")
+        ctx.check(ctx.lib.plaidgpu_row_topk(ctx.h, buf.data_ptr(), S, n_cols, kk, 1 if decreasing else 0, L.DEVICE,
+                                            i.ctypes.data, v.ctypes.data))
+        idx[:kk] = i + int(col0)
+        val[:kk] = v
+    gi, gv = comm.allgather_vecs([idx.ravel(order="F").astype(np.float64), val.ravel(order="F")])
+    world = comm.world
+    gi = np.asarray(gi).reshape(world, S, int(k)).astype(np.int64)
+    gv = np.asarray(gv).reshape(world, S, int(k))
+    return merge_row_topk([(gi[r].T, gv[r].T) for r in range(world)], int(k), decreasing)
+
+
 def shard_columns(n_total: int, world: int, rank: int):
     """contiguous, equal-count column ranges (equal output bytes, the dominant cost)"""
     base, rem = divmod(n_total, world)

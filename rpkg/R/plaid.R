@@ -37,7 +37,8 @@
   }
 }
 
-.score <- function(X, matG, opts, labels = NULL, K = NULL, topk = NULL, decreasing = TRUE, design = NULL) {
+.score <- function(X, matG, opts, labels = NULL, K = NULL, topk = NULL, decreasing = TRUE, design = NULL,
+                   topcells = NULL) {
   x <- .as_x(X)
   rn <- x$dimnames[[1]]
   gg <- intersect(rn, rownames(matG))                                 # R/plaid.R:65
@@ -69,13 +70,20 @@
                  as.integer(isTRUE(decreasing)))
     return(.topsets(out, topk, x$dimnames[[2]]))
   }
+  if (!is.null(topcells)) {  # plaid.topcells: each set's top k cells selected on the device, k x 2S back
+    out <- .Call(C_plaidgpu_score_row_topk, .ctxs(), x$kind, x$p, x$i, x$x, as.integer(x$dim),
+                 G@p, G@i, G@x, as.integer(dim(G)), as.integer(rowmap), opts, as.integer(topcells),
+                 as.integer(isTRUE(decreasing)))
+    return(.topsets(out, topcells, colnames(matG)))
+  }
   out <- .Call(C_plaidgpu_score, .ctxs(), x$kind, x$p, x$i, x$x, as.integer(x$dim),
                G@p, G@i, G@x, as.integer(dim(G)), as.integer(rowmap), opts)
   dimnames(out) <- list(colnames(matG), x$dimnames[[2]])
   out
 }
 
-## the k x 2N matrix of the top-k shim entries (1-based indices, then scores) -> list(index, score)
+## the k x 2N matrix of the top-k shim entries (1-based indices, then scores) -> list(index, score); the row top-k
+## entries return k x 2S the same way
 .topsets <- function(out, k, cn) {
   N <- ncol(out) %/% 2L
   index <- matrix(as.integer(out[, seq_len(N)]), k, N)
@@ -100,6 +108,23 @@ plaid.topsets <- function(X, matG, k = 10, decreasing = TRUE, gsetX = NULL) {
   cn <- colnames(X)
   if (is.null(cn)) cn <- colnames(gsetX)
   .topsets(out, k, cn)
+}
+
+## Each gene set's k best cells: the first k entries of order(x, decreasing = decreasing) for every row x of
+## plaid(X, matG) (ties by cell order, NA last), i.e. apply(plaid(X, matG), 1, order, decreasing = TRUE)[1:k, ] and
+## the scores at those cells, without the S x N score matrix ever reaching R: plaid() and the selection run as one
+## device call (options(plaid.gpus) applies).  With gsetX (the scores of any scorer, sets x cells) the selection
+## runs on that matrix instead.  1 <= k <= min(ncol(X), 256).  Returns list(index = integer k x S (columns of X,
+## 1-based), score = double k x S), both with colnames(matG); colnames(X)[index] names the cells.
+plaid.topcells <- function(X, matG, k = 10, decreasing = TRUE, gsetX = NULL) {
+  if (is.null(gsetX))
+    return(.score(X, matG, list(scorer = 0L, stats_mean = 1L, normalize = 1L), topcells = k, decreasing = decreasing))
+  gsetX <- as.matrix(gsetX)
+  storage.mode(gsetX) <- "double"
+  out <- .Call(C_plaidgpu_row_topk, .ctx(), gsetX, as.integer(k), as.integer(isTRUE(decreasing)))
+  rn <- colnames(matG)
+  if (is.null(rn)) rn <- rownames(gsetX)
+  .topsets(out, k, rn)
 }
 
 plaid <- function(X, matG, stats = c("mean", "sum"), chunk = NULL, normalize = TRUE) {

@@ -357,6 +357,73 @@ SEXP C_plaidgpu_score_topk(SEXP ctx, SEXP kind, SEXP Xp, SEXP Xi, SEXP Xx, SEXP 
   return out;
 }
 
+/* per-row top k as one k x 2S matrix: columns 1..S the 1-based column indices (exact in a double), S+1..2S the
+ * values; idx / val are what plaidgpu_row_topk / plaidgpu_score_row_topk wrote, val already in place */
+static void row_topk_indices_to_r(SEXP out, const int64_t* idx, int k, int S) {
+  double* o = REAL(out);
+  for (R_xlen_t t = 0, n = (R_xlen_t)k * S; t < n; ++t) o[t] = (double)idx[t] + 1.0;
+}
+
+/* plaid.topcells(gsetX = ): each row's k first columns of order(x[s, ], decreasing = decreasing) */
+SEXP C_plaidgpu_row_topk(SEXP ctx, SEXP x, SEXP k, SEXP decreasing) {
+  plaidgpu_ctx* c = get_ctx(ctx);
+  SEXP dim = Rf_getAttrib(x, R_DimSymbol);
+  const int S = INTEGER(dim)[0], N = INTEGER(dim)[1], kk = Rf_asInteger(k);
+  if (kk < 1 || kk > 256 || kk > N) Rf_error("plaidgpu: k must be in [1, min(ncol(x), 256)]");
+  int64_t* idx = (int64_t*)R_alloc((size_t)kk * (size_t)S + 1, sizeof(int64_t));
+  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, kk, 2 * S));
+  int rc = plaidgpu_row_topk(c, REAL(x), S, N, kk, Rf_asInteger(decreasing), PLAIDGPU_HOST, idx,
+                             REAL(out) + (R_xlen_t)kk * S);
+  if (rc != PLAIDGPU_OK) {
+    UNPROTECT(1);
+    Rf_error("plaidgpu_row_topk: %s", plaidgpu_last_error(c));
+  }
+  row_topk_indices_to_r(out, idx, kk, S);
+  UNPROTECT(1);
+  return out;
+}
+
+/* plaid.topcells(): plaid() fused with each gene set's top k cells — the S x N scores stay on the device, a k x 2S
+ * matrix (indices, then scores) comes back.  A list of contexts (options(plaid.gpus = n)) splits the columns over the
+ * devices (plaidgpu_score_row_topk_multi). */
+SEXP C_plaidgpu_score_row_topk(SEXP ctx, SEXP kind, SEXP Xp, SEXP Xi, SEXP Xx, SEXP Xdim, SEXP Gp, SEXP Gi, SEXP Gx,
+                               SEXP Gdim, SEXP rowmap, SEXP opts, SEXP k, SEXP decreasing) {
+  plaidgpu_ctx* cs[16];
+  int nctx = 1;
+  if (TYPEOF(ctx) == VECSXP) {
+    nctx = (int)XLENGTH(ctx);
+    if (nctx < 1 || nctx > 16) Rf_error("plaidgpu: between 1 and 16 contexts expected");
+    for (int j = 0; j < nctx; ++j) cs[j] = get_ctx(VECTOR_ELT(ctx, j));
+  } else {
+    cs[0] = get_ctx(ctx);
+  }
+  plaidgpu_ctx* c = cs[0];
+  const int PG = INTEGER(Gdim)[0], S = INTEGER(Gdim)[1], kk = Rf_asInteger(k);
+  plaidgpu_matrix M;
+  fill_matrix(&M, Rf_asInteger(kind), Xp, Xi, Xx, Xdim);
+  if (kk < 1 || kk > 256 || kk > M.N) Rf_error("plaidgpu: k must be in [1, min(ncol(X), 256)]");
+  if (S > INT_MAX / 2) Rf_error("plaidgpu: too many gene sets for one k x 2S result");
+  for (int j = 0; j < nctx; ++j)
+    if (plaidgpu_set_genesets(cs[j], PG, S, INTEGER(Gp), INTEGER(Gi), REAL(Gx)) != PLAIDGPU_OK)
+      Rf_error("plaidgpu_set_genesets: %s", plaidgpu_last_error(cs[j]));
+  plaidgpu_opts o;
+  fill_opts(&o, opts);
+  R_CheckUserInterrupt();
+  int64_t* idx = (int64_t*)R_alloc((size_t)kk * (size_t)S + 1, sizeof(int64_t));
+  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, kk, 2 * S));
+  double* val = REAL(out) + (R_xlen_t)kk * S;
+  const int dec = Rf_asInteger(decreasing);
+  int rc = nctx > 1 ? plaidgpu_score_row_topk_multi(cs, nctx, &M, INTEGER(rowmap), &o, kk, dec, idx, val)
+                    : plaidgpu_score_row_topk(c, &M, INTEGER(rowmap), &o, kk, dec, idx, val);
+  if (rc != PLAIDGPU_OK) {
+    UNPROTECT(1);
+    Rf_error("plaidgpu_score_row_topk: %s", plaidgpu_last_error(c));
+  }
+  row_topk_indices_to_r(out, idx, kk, S);
+  UNPROTECT(1);
+  return out;
+}
+
 static const R_CallMethodDef call_methods[] = {
     {"C_plaidgpu_ctx", (DL_FUNC)&C_plaidgpu_ctx, 1},
     {"C_plaidgpu_score", (DL_FUNC)&C_plaidgpu_score, 12},
@@ -368,6 +435,8 @@ static const R_CallMethodDef call_methods[] = {
     {"C_plaidgpu_score_design_stats", (DL_FUNC)&C_plaidgpu_score_design_stats, 13},
     {"C_plaidgpu_col_topk", (DL_FUNC)&C_plaidgpu_col_topk, 4},
     {"C_plaidgpu_score_topk", (DL_FUNC)&C_plaidgpu_score_topk, 14},
+    {"C_plaidgpu_row_topk", (DL_FUNC)&C_plaidgpu_row_topk, 4},
+    {"C_plaidgpu_score_row_topk", (DL_FUNC)&C_plaidgpu_score_row_topk, 14},
     {"C_plaidgpu_crossprod", (DL_FUNC)&C_plaidgpu_crossprod, 11},
     {NULL, NULL, 0}};
 
