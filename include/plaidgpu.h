@@ -196,7 +196,7 @@ int plaidgpu_score_begin(plaidgpu_ctx* ctx, const plaidgpu_matrix* X, const int3
                          const plaidgpu_opts* opts, plaidgpu_scalars* local);
 int plaidgpu_score_compute(plaidgpu_ctx* ctx, plaidgpu_scalars* scal, double* out);
 /* per-column medians of the raw scores of this shard: med_all (NaN dropped) and med_nz
- * (NaN and zeros dropped, all-dropped -> 0); each double[N_shard] (host). */
+ * (NaN and zeros dropped; all-dropped, or middles -inf and +inf -> 0); each double[N_shard] (host). */
 int plaidgpu_get_col_medians(plaidgpu_ctx* ctx, double* med_all, double* med_nz);
 /* The one median vector normalize_medians will use once the global flag is known: ignore_zero != 0 ->
  * medians over the non-zero scores, else over all scores; med: host double[N of this shard].  The library

@@ -1937,7 +1937,7 @@ int plaidgpu_score_compute(plaidgpu_ctx* c, plaidgpu_scalars* scal, double* out)
     if (rc) return rc;
     CK(cudaEventRecord(c->ev[3], c->stream));
     if (which == COLSTATS_ALL && c->local_min > 0.0 && c->N) {  // no zeros: the two medians are the same numbers
-      CK(launch_copy_words(c->b_med_all.p, c->b_med_nz.p, c->N, c->stream));  // by a kernel: copy engines may be busy with result blocks
+      CK(launch_med_nz_from_all(c->b_med_all.as<double>(), c->b_med_nz.as<double>(), c->N, c->stream));
       c->have_nz = true;
     }
     rc = fetch_medians(c);

@@ -217,6 +217,8 @@ cudaError_t launch_row_topk(const double* x, int64_t ld, int32_t S, int64_t N, i
                             const double* beta = nullptr);
 // nwords 8-byte words device -> host-mapped (cudaHostAllocMapped) memory by a kernel, bypassing the copy engine
 cudaError_t launch_copy_words(const void* src, void* dst_mapped, int64_t nwords, cudaStream_t st);
+// med_nz = med_all of scores without zeros or negatives, except that a column with no valid score gets 0, not NaN
+cudaError_t launch_med_nz_from_all(const double* med_all, double* med_nz, int64_t n, cudaStream_t st);
 // global min / max of a device array of n doubles, NaN ignored (na.rm = TRUE); res[0]=min res[1]=max
 cudaError_t launch_minmax(const double* x, int64_t n, double* res2, cudaStream_t st);
 

@@ -290,6 +290,7 @@ __global__ void __launch_bounds__(NT) k_colstats(const double* __restrict__ x, i
       if (m2 > 0) {
         const double a = value_of(s.result[2]), b = value_of(s.result[3]);
         mz = (m2 & 1u) ? a : (a + b) / 2.0;
+        if (mz != mz) mz = 0.0;  // middles -inf and +inf: NA -> 0 like an empty column (R/plaid.R:561-566)
       }
       med_all[j] = ma;
       med_nz[j] = mz;
@@ -650,6 +651,7 @@ __global__ void __launch_bounds__(NT) k_colstats_fast(const double* __restrict__
         if (DO1 && cnt[1] > 0) {
           const double a = value_of(s.res[1][0]), b = value_of(s.res[1][1]);
           mz = (cnt[1] & 1u) ? a : (a + b) / 2.0;
+          if (mz != mz) mz = 0.0;  // middles -inf and +inf (see k_colstats)
         }
         if (DO0) med_all[j] = ma;
         if (DO1) med_nz[j] = mz;
@@ -994,6 +996,7 @@ __global__ void __launch_bounds__(NT) k_colstats_one(const double* __restrict__ 
         if (count > 0) {
           const double a = value_of(A), b = value_of(B);
           m = (count & 1u) ? a : (a + b) / 2.0;
+          if (NZ && m != m) m = 0.0;  // middles -inf and +inf (see k_colstats)
         }
         med[j] = m;
         colmin[j] = s.minkey != ~0ull ? value_of(s.minkey) : INFINITY;
@@ -1224,6 +1227,16 @@ __global__ void __launch_bounds__(256) k_copy_words(const unsigned long long* __
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) dst[i] = src[i];
 }
 
+// by a kernel, not a copy engine: those may be busy with result blocks.  A NaN median of a column without zeros or
+// -inf comes from a column without any valid value, whose non-zero median is 0 (R/plaid.R:561-566)
+__global__ void __launch_bounds__(256) k_med_nz_from_all(const double* __restrict__ med_all, double* __restrict__ med_nz,
+                                                         int64_t n) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const double m = med_all[i];
+    med_nz[i] = m == m ? m : 0.0;
+  }
+}
+
 __global__ void k_minmax_init(unsigned long long* res) {
   res[0] = ~0ull;
   res[1] = 0ull;
@@ -1376,6 +1389,14 @@ cudaError_t launch_copy_words(const void* src, void* dst_mapped, int64_t nwords,
   int64_t grid = (nwords + 255) / 256;
   if (grid > 148 * 4) grid = 148 * 4;
   k_copy_words<<<(unsigned)grid, 256, 0, st>>>(static_cast<const unsigned long long*>(src), static_cast<unsigned long long*>(dst_mapped), nwords);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_med_nz_from_all(const double* med_all, double* med_nz, int64_t n, cudaStream_t st) {
+  if (n <= 0) return cudaSuccess;
+  int64_t grid = (n + 255) / 256;
+  if (grid > 148 * 4) grid = 148 * 4;
+  k_med_nz_from_all<<<(unsigned)grid, 256, 0, st>>>(med_all, med_nz, n);
   return cudaGetLastError();
 }
 
